@@ -29,6 +29,8 @@ import numpy as np  # noqa: E402
 N_PER_GPU = 100000
 DIM = 100
 SETUP_GENS = 60
+DUMP_ROWS = 8192        # chains whose rows --dump-outputs writes: all 10^5 would be 80 MB per generation
+DUMP_GENS = 4           # ... and how many of the last timed generations of their history (64 MB cap in all)
 METRIC = "DREAM chain-steps/s, 100-D Gaussian"
 UNIT = "chain-steps/s"
 
@@ -121,8 +123,8 @@ def cpu_port_spec(n_chains):
 
 
 def cpu_arm(n_chains, procs, gens, gens_warm):
-    """Time the reference's DREAM on `procs` host processes: the UNMODIFIED reference from baseline/_ref
-    (oracle/ref_runner.py: shared-memory stand-in for mpirun) when it travelled with the tree, else the
+    """Time the reference's DREAM on `procs` host processes: the UNMODIFIED reference from oracle/_ref
+    (oracle/ref_runner.py: shared-memory stand-in for mpirun) when it is installed there, else the
     oracle port (oracle/mp_port.py).  Returns (seconds, chain_steps, kind)."""
     from oracle import ref_runner
     if ref_runner.reference_dir() is not None:
@@ -137,7 +139,7 @@ def cpu_arm(n_chains, procs, gens, gens_warm):
 
 def run_reference(args):
     """The reference's own CPU implementation of the path on the host cores: wgurecky/bipymc DreamMpi,
-    unmodified (baseline/_ref), one rank per core over a shared-memory communicator."""
+    unmodified (oracle/_ref), one rank per core over a shared-memory communicator."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
@@ -147,7 +149,7 @@ def run_reference(args):
     # a step = one generation of the sample population; warm-up generations are untimed
     dt, steps, kind = cpu_arm(n_chains, procs, gens=args.steps, gens_warm=max(args.warmup, 1))
     v = steps / dt
-    what = "unmodified reference DreamMpi (baseline/_ref)" if kind == "reference" else "oracle port of DreamMpi"
+    what = "unmodified reference DreamMpi (oracle/_ref)" if kind == "reference" else "oracle port of DreamMpi"
     sample = "%s, %d ranks, 100-D Gaussian, %d chains (200 per rank), %d timed generations, %.1f s" % (
         what, procs, n_chains, args.steps, dt)
     line = {"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus,
@@ -167,7 +169,7 @@ def cpu_baseline_leg():
     n_chains = 40 * procs
     gens = 400            # ~10-20 s of host work: np.std over the growing history is O(T) per step (dream.py:128)
     dt, steps, kind = cpu_arm(n_chains, procs, gens=gens, gens_warm=2)
-    what = "unmodified reference DreamMpi (baseline/_ref), shared-memory ranks" if kind == "reference" else \
+    what = "unmodified reference DreamMpi (oracle/_ref), shared-memory ranks" if kind == "reference" else \
         "oracle port of DreamMpi (shared-memory ranks)"
     out = {"value": steps / dt, "unit": UNIT, "cores": procs, "kind": kind,
            "sample": "%s, 100-D Gaussian, %d chains, %d generations, %.1f s" % (what, n_chains, gens, dt)}
@@ -234,6 +236,28 @@ def selfcheck_sharded(world, rank, local_rank):
     return out
 
 
+def dump_outputs(out_dir, s, k_timed):
+    """Write what a caller of run_mcmc holds after the last timed generation, as float64 .npy files:
+    for a fixed, seeded sample of chains their indices, current states and (history kept) their history rows of
+    the last timed generations; every chain's cached ln-likelihood, DREAM's crossover state and the accepted /
+    rejected counts of the timed generations."""
+    import torch
+    rows = np.sort(np.random.RandomState(0).choice(s.n_chains, min(DUMP_ROWS, s.n_chains), replace=False))
+    idx = torch.from_numpy(rows).to(s._X.device)
+    out = {"state_sample": s._X[idx, :s.dim].cpu().numpy(),
+           "state_sample_rows": rows,
+           "lnl": s._lnl.cpu().numpy(),
+           "p_cr": s.p_cr,
+           "delta_m": s.delta_m,
+           "accepted_rejected": [s.n_accepted, s.n_rejected]}
+    if s._hist.policy == "full":
+        # tensor() first writes the newest row, which the fused kernel leaves pending, into the history
+        out["history_sample"] = s._hist.tensor()[-min(k_timed, DUMP_GENS):, idx, :s.dim].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -293,6 +317,8 @@ def run_ours(args):
     e1.record()
     sync_all()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, s, K)
     # pass 2 -- the next K generations of the same run with CUDA events around every launch
     # (bpm_profile): per-kernel durations for the roofline.  Two event records per launch cost a few
     # microseconds per generation, so they are kept out of `value`; the pass's own time is reported.
@@ -520,7 +546,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-buffer end-to-end leg (profiling runs)")
     ap.add_argument("--no-stationary", action="store_true", help="skip the second (stationary-population) point")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed generations, write their results to DIR/<name>.npy (1 GPU only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.gpus != 1):
+        ap.error("--dump-outputs needs --impl ours and --gpus 1")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args)

@@ -1,5 +1,5 @@
 """Times the UNMODIFIED reference (wgurecky/bipymc, installed by __graft_entry__.build() into
-baseline/_ref with `pip install --target`) on the host cores: the `kind: "reference"` CPU baseline of
+oracle/_ref with `pip install --target`) on the host cores: the `kind: "reference"` CPU baseline of
 bench.py (BASELINE.md section 5 items 1-2).
 
 TEST / BENCH INFRASTRUCTURE ONLY.  The reference imports mpi4py / h5py / matplotlib / corner at module
@@ -18,7 +18,7 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-REF_DIRS = [os.path.join(ROOT, "baseline", "_ref")]     # travels with the tree; /root/reference does not
+REF_DIRS = [os.path.join(ROOT, "oracle", "_ref")]
 
 
 def reference_dir():
@@ -31,7 +31,7 @@ def reference_dir():
 def _import_reference():
     d = reference_dir()
     if d is None:
-        raise ImportError("unmodified reference not found (baseline/_ref is written by __graft_entry__.build())")
+        raise ImportError("unmodified reference not found (oracle/_ref is written by __graft_entry__.build())")
     shims = os.path.join(HERE, "shims")
     for p in (d, shims):
         if p in sys.path:

@@ -1,10 +1,12 @@
-"""bench.py's reference arm (the unmodified reference from baseline/_ref on the host cores; the oracle port
+"""bench.py's reference arm (the unmodified reference from oracle/_ref on the host cores; the oracle port
 when that install is absent) keeps the JSON contract the driver reads:
 one line, the same metric / unit as our arm, a cpu_baseline describing the run and a zero-copy e2e object."""
 import json
 import os
 import subprocess
 import sys
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -24,12 +26,22 @@ def test_reference_arm_prints_one_contract_line():
     assert j["value"] > 0 and j["ms_per_step"] > 0
     assert "workload" in j["config"] and "model" not in j["config"]
     cb = j["cpu_baseline"]
-    have_ref = os.path.exists(os.path.join(ROOT, "baseline", "_ref", "bipymc", "dream.py"))
+    sys.path.insert(0, ROOT)
+    from oracle import ref_runner
+    have_ref = ref_runner.reference_dir() is not None
     assert cb["kind"] == ("reference" if have_ref else "port")
     assert cb["cores"] >= 1 and cb["value"] == j["value"] and cb["sample"]
     e = j["e2e"]
     assert e["value"] == j["value"] and e["unit"] == j["unit"]
     assert e["h2d_bytes_per_step"] == 0 and e["d2h_bytes_per_step"] == 0
+
+
+@pytest.mark.parametrize("args", [["--steps", "0"], ["--gpus", "2", "--dump-outputs", "x"],
+                                  ["--impl", "reference", "--dump-outputs", "x"]])
+def test_bench_refuses_bad_arguments(args):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + args, stdout=subprocess.PIPE,
+                       stderr=subprocess.PIPE, text=True, timeout=600, cwd=ROOT)
+    assert r.returncode == 2 and "error:" in r.stderr
 
 
 def test_reference_runner_shared_memory_ranks():
@@ -39,7 +51,7 @@ def test_reference_runner_shared_memory_ranks():
     sys.path.insert(0, ROOT)
     from oracle import ref_runner
     if ref_runner.reference_dir() is None:
-        pytest.skip("baseline/_ref not installed (built by __graft_entry__.build() where /root/reference exists)")
+        pytest.skip("the unmodified reference is not installed in oracle/_ref")
     spec = dict(n_chains=8, dim=100, algo="dream", seed=42, ctor_kwargs=dict(n_cr_gen=2, burnin_gen=100))
     dt, steps = ref_runner.time_reference(spec, 2, gens=3, gens_warm=1)
     assert steps == 8 * 3 and dt > 0

@@ -1,6 +1,6 @@
 """Checkpoint files travel between the UNMODIFIED reference and bipymc_b200 (chain.py:59-93, demc.py:198-233).
 
-The reference runs from baseline/_ref (pip-installed by __graft_entry__.build(); it travels to the GPU box) with
+The reference runs from oracle/_ref (pip-installed by __graft_entry__.build() where its source is present) with
 oracle/shims on the path: a single-rank mpi4py, and an `h5py` that is the package's HDF5 implementation
 (bipymc_b200/h5lite.py) -- so the reference's own write_chain_h5 / read_chain_h5 / save_state / load_state code
 executes, calling exactly the h5py API it was written against.  What this pins: the API slice h5lite offers is the
@@ -13,11 +13,11 @@ import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, "baseline", "_ref")
+REF = os.path.join(ROOT, "oracle", "_ref")
 SHIMS = os.path.join(ROOT, "oracle", "shims")
 
 pytestmark = pytest.mark.skipif(not os.path.exists(os.path.join(REF, "bipymc", "chain.py")),
-                                reason="baseline/_ref (the pip-installed reference) is not present")
+                                reason="oracle/_ref (the pip-installed reference) is not present")
 
 
 @pytest.fixture(scope="module")
