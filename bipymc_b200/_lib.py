@@ -13,7 +13,8 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("BIPYMC_B200_LIB") or os.path.join(_HERE, "lib", "libbipymc_b200.so")
 
 BPM_ALGO_DEMC, BPM_ALGO_DREAM, BPM_ALGO_DEMC_SERIAL = 0, 1, 2
-TARGET_EXTERNAL, TARGET_BANANA, TARGET_BIMODAL, TARGET_GAUSS, TARGET_LINEFIT, TARGET_EXPFIT = 0, 1, 2, 3, 4, 5
+TARGET_EXTERNAL, TARGET_BANANA, TARGET_BIMODAL, TARGET_GAUSS, TARGET_LINEFIT, TARGET_EXPFIT, TARGET_JIT = \
+    0, 1, 2, 3, 4, 5, 6
 BPM_MAX_PAIRS, BPM_MAX_CR, BPM_MAX_PEERS = 8, 16, 15
 
 
@@ -58,6 +59,10 @@ SIGNATURES = {
     "bpm_set_fused": (C.c_int, [C.c_void_p, C.c_int32]),
     "bpm_set_target": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(C.c_double), C.c_int64]),
     "bpm_set_batched_lnl": (C.c_int, [C.c_void_p, LNL_FN, C.c_void_p]),
+    "bpm_jit_compile": (C.c_int, [C.c_char_p, C.c_int32, C.c_int64, C.c_int32, C.POINTER(C.c_int32), C.c_char_p,
+                                  C.c_int64]),
+    "bpm_set_jit_target": (C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(C.c_double), C.c_int64, C.c_int32,
+                                     C.POINTER(C.c_int32), C.c_char_p, C.c_int64]),
     "bpm_eval_lnl": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),
     "bpm_set_cr_state": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_double),
                                    C.POINTER(C.c_double)]),
@@ -121,11 +126,35 @@ class BpmError(RuntimeError):
     pass
 
 
+def _nvrtc_default():
+    """NVRTC for the run-time compiled likelihoods (bpm_jit_compile): the library looks at
+    $BIPYMC_B200_NVRTC, then next to nvcc, then on the loader path.  Without a toolkit, point it at
+    the copy torch ships (nvidia/cuda_nvrtc), when there is one."""
+    if os.environ.get("BIPYMC_B200_NVRTC"):
+        return
+    for b in os.environ.get("PATH", "").split(os.pathsep) + ["/usr/local/cuda/bin"]:
+        if b and os.access(os.path.join(b, "nvcc"), os.X_OK):
+            if os.path.exists(os.path.join(b, "..", "lib64", "libnvrtc.so.12")):
+                return
+            break
+    try:
+        import importlib.util
+        spec = importlib.util.find_spec("nvidia.cuda_nvrtc")
+    except (ImportError, ValueError):
+        return
+    for d in (spec.submodule_search_locations or []) if spec else []:
+        p = os.path.join(d, "lib", "libnvrtc.so.12")
+        if os.path.exists(p):
+            os.environ["BIPYMC_B200_NVRTC"] = p
+            return
+
+
 def load():
     """Load the CUDA library or fail loudly (no fallback of any kind)."""
     global _lib
     if _lib is not None:
         return _lib
+    _nvrtc_default()
     if not os.path.exists(LIB_PATH):
         raise ImportError(
             "bipymc_b200: CUDA library %s is missing. Build it with "

@@ -16,6 +16,14 @@ attribute surface as the reference.  What changed underneath:
 Likelihood plug-ins, fastest first:
   1. ``ln_like_fn`` is ``obj.ln_like`` of a built-in target (bipymc_b200.targets): the
      likelihood is evaluated inside the generation kernels;
+  1b. ``ln_like_cuda=targets.CudaLikelihood(source, dim, data)``: the user's own
+     ``__device__ double ln_like(const double* theta, const double* data)`` (``theta[BPM_DIM]``,
+     ``data[BPM_NDATA]``), compiled at run time with NVRTC into the same kernels -- the fused
+     d <= 4 half-phase kernel, or a batched row kernel between propose and accept above that.
+     ``-INFINITY`` = outside the prior; NaN raises ``ValueError("probabilities contain NaN")``;
+     ``fmad=False`` rounds like numpy.  The first compile takes up to about 2 s, later samplers with the
+     same source reuse the cubin.  Takes precedence over a built-in target and over
+     ``ln_like_batched``; ``ln_like_fn`` stays the drop-in positional argument and is not called;
   2. ``ln_like_batched=f``: ``f(theta)`` takes a CUDA float64 tensor ``[n, dim]`` and
      returns ``[n]`` log-likelihoods (torch ops on the current stream);
   3. any scalar ``ln_like_fn(theta, **ln_kwargs) -> float`` exactly as in the reference
@@ -347,6 +355,7 @@ class DeMcMpi(object):
         self._seed = kwargs.get("seed", None)
         self._history_policy = kwargs.get("history", "full")
         self._ln_like_batched = kwargs.get("ln_like_batched", None)
+        self._ln_like_cuda = kwargs.get("ln_like_cuda", None)
         self._device_index = kwargs.get("device", None)
         self._fused = kwargs.get("fused", True)
         self._chunk_bytes = int(kwargs.get("history_chunk_bytes", 1 << 30))
@@ -420,6 +429,12 @@ class DeMcMpi(object):
 
     def _create_handle(self):
         d = self.dim
+        if self._ln_like_cuda is not None:
+            from .targets import CudaLikelihood
+            if not isinstance(self._ln_like_cuda, CudaLikelihood):
+                raise TypeError("ln_like_cuda must be a targets.CudaLikelihood")
+            if self._ln_like_cuda.dim != d:
+                raise ValueError("ln_like_cuda dimension %d != theta_0 dimension %d" % (self._ln_like_cuda.dim, d))
         self._ld = d if d <= 4 else ((d + 3) // 4) * 4
         ids = np.array_split(np.arange(self.n_chains), self.comm.size)[self.comm.rank]
         self.rank_chain_ids = ids                                   # demc.py:39-40
@@ -446,6 +461,10 @@ class DeMcMpi(object):
         _lib.check(self._libh.bpm_create(C.byref(cfg), C.byref(h)))
         self._handle = h
         _lib.check(self._libh.bpm_set_fused(h, int(self._fused)))   # 0 split, 1 fused, 2 fused (two-halves variant)
+        if self._ln_like_cuda is not None:
+            self._target = self._ln_like_cuda
+            self._jit_from_cache = self._target._attach(self._libh, h)     # True: the cubin came from the cache
+            return
         self._target = resolve_device_target(self.log_like_fn, self._ln_kwargs)
         if self._target is not None:
             if self._target.dim != d:

@@ -42,6 +42,7 @@ class DeMc(DeMcMpi):
         self._seed = proposal_kwargs.get("seed", None)
         self._history_policy = proposal_kwargs.get("history", "full")
         self._ln_like_batched = proposal_kwargs.get("ln_like_batched", None)
+        self._ln_like_cuda = proposal_kwargs.get("ln_like_cuda", None)
         self._device_index = proposal_kwargs.get("device", None)
         self._fused = False                                         # the sweep uses the split launches
         self._chunk_bytes = int(proposal_kwargs.get("history_chunk_bytes", 1 << 30))

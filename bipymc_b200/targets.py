@@ -9,6 +9,9 @@ Mirrors the reference's test-target classes (same constructor arguments, same ``
   LineFit         examples/ex_para_fit.py:26-55 (lnprob of the second example)
   ExpFit          examples/ex_exp_fit.py:38-121 (5-parameter relaxation fit)
 
+and ``CudaLikelihood``: any other model as CUDA C++ source, compiled at run time into the same
+kernels (``ln_like_cuda=`` of the samplers).
+
 ``ln_like`` stays a scalar host function, so the objects remain valid ``ln_like_fn``
 arguments everywhere; when a sampler of this package receives ``obj.ln_like`` it
 recognises the owner through ``device_target()`` and evaluates the likelihood inside the
@@ -19,6 +22,8 @@ reference calls): symmetric eigendecomposition, ``U = V / sqrt(lambda)``,
 ``maha = |(x - mu) U|^2``, ``logpdf = -0.5 (rank log 2pi + log pdet + maha)``
 (scipy/stats/_multivariate.py ``_PSD`` and ``_logpdf``).
 """
+import ctypes as C
+
 import numpy as np
 
 from . import _lib
@@ -273,3 +278,76 @@ def resolve_device_target(ln_like_fn, ln_kwargs):
     if isinstance(ln_like_fn, DeviceTarget):
         return ln_like_fn
     return None
+
+
+class CudaCompileError(_lib.BpmError):
+    """NVRTC rejected a CudaLikelihood source; ``log`` is the compiler's log, whose line numbers
+    refer to the user's source (``ln_like.cu(line)``)."""
+    def __init__(self, msg, log=""):
+        super(CudaCompileError, self).__init__(msg + ("\n" + log if log else ""))
+        self.log = log
+
+
+class CudaLikelihood(object):
+    """A user likelihood in CUDA C++, compiled at run time (NVRTC, sm_100a) into the sampler's
+    own generation kernels -- the fast path of the built-in targets, for any model.
+
+    ``source`` defines ONE device function::
+
+        __device__ double ln_like(const double* theta, const double* data)
+
+    with ``theta[BPM_DIM]`` (the parameters) and ``data[BPM_NDATA]`` (``data`` below, read-only,
+    copied to the device once); ``BPM_DIM`` / ``BPM_NDATA`` are macros, and the CUDA math functions
+    and the ``bpm::`` helpers of the package's csrc/targets.cuh are in scope.  Return ``-INFINITY``
+    outside the prior; a NaN makes ``run_mcmc`` raise ``ValueError("probabilities contain NaN")``
+    as the reference does.  ``fmad=False`` rounds every ``+ - * /`` on its own (numpy's results);
+    ``fmad=True`` lets the compiler fuse multiply-adds.  The first compile of a source takes up to
+    about 2 s; later samplers with the same source, dim, data size and fmad reuse the cubin for the rest
+    of the process.
+
+    At d <= 4 the likelihood runs inside the fused one-thread-per-chain half-phase kernel, above that
+    in a batched row kernel between the proposal and accept kernels.  Pass it as ``ln_like_cuda=``."""
+
+    _LOG_BYTES = 1 << 16
+
+    def __init__(self, source, dim, data=None, fmad=True):
+        if not isinstance(source, str):
+            raise ValueError("source must be a str of CUDA C++")
+        if isinstance(dim, bool) or int(dim) != dim or int(dim) < 1:
+            raise ValueError("dim must be an integer >= 1")
+        data = np.zeros(0) if data is None else np.asarray(data, dtype=np.float64)
+        if data.ndim != 1:
+            raise ValueError("data must be 1-D (concatenate the arrays the source reads)")
+        if not np.all(np.isfinite(data)):
+            raise ValueError("data must be finite")
+        self.source = source
+        self.dim = int(dim)
+        self.data = np.ascontiguousarray(data)
+        self.fmad = bool(fmad)
+
+    @property
+    def _flags(self):
+        return 1 if self.fmad else 0
+
+    def _call(self, fn, *head):
+        log = C.create_string_buffer(self._LOG_BYTES)
+        cached = C.c_int32(0)
+        rc = fn(*(head + (C.byref(cached), log, self._LOG_BYTES)))
+        if rc != 0:
+            msg = _lib.load().bpm_last_error().decode()
+            text = log.value.decode(errors="replace")
+            if text:
+                raise CudaCompileError(msg, text)
+            raise _lib.BpmError(msg)
+        return bool(cached.value)
+
+    def compile(self):
+        """Compile for sm_100a (no device needed).  Returns True when the cubin came from the
+        process cache; raises CudaCompileError with the NVRTC log."""
+        lib = _lib.load()
+        return self._call(lib.bpm_jit_compile, self.source.encode(), self.dim, self.data.size, self._flags)
+
+    def _attach(self, lib, handle):
+        """Compile (or take the cached cubin), load it on the handle's device and copy the data."""
+        return self._call(lib.bpm_set_jit_target, handle, self.source.encode(), _lib.dptr(self.data),
+                          self.data.size, self._flags)

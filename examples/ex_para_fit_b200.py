@@ -1,11 +1,13 @@
 #!/usr/bin/env python
 """Line fit with a nuisance scatter parameter -- the workload of the reference's
-examples/ex_para_fit.py (theta = (m, b, ln f), 50 synthetic points, box prior), run three ways
+examples/ex_para_fit.py (theta = (m, b, ln f), 50 synthetic points, box prior), run four ways
 on the device sampler:
 
   1. the built-in device likelihood (whole generations inside the CUDA kernels),
-  2. a batched torch likelihood  f(theta[n, 3]) -> lnL[n]  (device tensors, same stream),
-  3. the reference's scalar ln_like_fn(theta, x, y, yerr) with ln_kwargs (host round trip).
+  2. the reference's per-term likelihood as CUDA source (targets.CudaLikelihood, compiled at run
+     time into the same kernels; fmad=False rounds every operation like numpy),
+  3. a batched torch likelihood  f(theta[n, 3]) -> lnL[n]  (device tensors, same stream),
+  4. the reference's scalar ln_like_fn(theta, x, y, yerr) with ln_kwargs (host round trip).
 
 Usage:  python examples/ex_para_fit_b200.py            (one GPU)
         torchrun --nproc-per-node 2 examples/ex_para_fit_b200.py   (chains sharded over 2 GPUs)
@@ -18,6 +20,41 @@ import numpy as np
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 
+# ex_para_fit.py:39-55, one data point at a time; data = x[M], y[M], yerr[M]
+LNPROB_CUDA = r'''
+__device__ double ln_like(const double* theta, const double* data) {
+  const int M = BPM_NDATA / 3;
+  const double* x = data;
+  const double* y = data + M;
+  const double* yerr = data + 2 * M;
+  const double m = theta[0], b = theta[1], lnf = theta[2];
+  if (!(-5.0 < m && m < 0.5 && 0.0 < b && b < 10.0 && -10.0 < lnf && lnf < 1.0)) return -INFINITY;
+  const double e2 = exp(2.0 * lnf);
+  double s = 0.0;
+  for (int i = 0; i < M; ++i) {
+    const double model = m * x[i] + b;
+    const double inv_sigma2 = 1.0 / (yerr[i] * yerr[i] + model * model * e2);
+    s += (y[i] - model) * (y[i] - model) * inv_sigma2 - log(inv_sigma2);
+  }
+  return 0.0 + -0.5 * s;
+}
+'''
+
+
+def make_lnprob_batched(x, y, yerr):
+    """The same likelihood as torch ops on [n, 3] CUDA float64 tensors (x, y, yerr: CUDA tensors)."""
+    import torch
+
+    def lnprob_batched(theta):
+        m, b, lnf = theta[:, 0:1], theta[:, 1:2], theta[:, 2:3]
+        model = m * x[None, :] + b
+        inv_sigma2 = 1.0 / (yerr[None, :] ** 2 + model ** 2 * torch.exp(2 * lnf))
+        ll = -0.5 * ((y[None, :] - model) ** 2 * inv_sigma2 - torch.log(inv_sigma2)).sum(dim=1)
+        ok = (theta[:, 0] > -5.0) & (theta[:, 0] < 0.5) & (theta[:, 1] > 0.0) & (theta[:, 1] < 10.0) & \
+             (theta[:, 2] > -10.0) & (theta[:, 2] < 1.0)
+        return torch.where(ok, ll, torch.full_like(ll, -float("inf")))
+    return lnprob_batched
+
 
 def main():
     import torch
@@ -29,21 +66,15 @@ def main():
     rank = int(os.environ.get("RANK", 0))
     fit = targets.LineFit()                         # x, y, yerr generated like ex_para_fit.py:17,26-35
     theta_0 = np.array([-0.8, 4.5, 0.2])
-    x, y, yerr = (torch.from_numpy(v).cuda() for v in (fit.x, fit.y, fit.yerr))
-
-    def lnprob_batched(theta):                      # theta: [n, 3] float64 CUDA tensor
-        m, b, lnf = theta[:, 0:1], theta[:, 1:2], theta[:, 2:3]
-        model = m * x[None, :] + b
-        inv_sigma2 = 1.0 / (yerr[None, :] ** 2 + model ** 2 * torch.exp(2 * lnf))
-        ll = -0.5 * ((y[None, :] - model) ** 2 * inv_sigma2 - torch.log(inv_sigma2)).sum(dim=1)
-        ok = (theta[:, 0] > -5.0) & (theta[:, 0] < 0.5) & (theta[:, 1] > 0.0) & (theta[:, 1] < 10.0) & \
-             (theta[:, 2] > -10.0) & (theta[:, 2] < 1.0)
-        return torch.where(ok, ll, torch.full_like(ll, -float("inf")))
+    lnprob_batched = make_lnprob_batched(*(torch.from_numpy(v).cuda() for v in (fit.x, fit.y, fit.yerr)))
+    lik = targets.CudaLikelihood(LNPROB_CUDA, 3, np.concatenate([fit.x, fit.y, fit.yerr]), fmad=False)
 
     def lnprob_scalar(theta, x, y, yerr):           # the reference's plug-in signature (samplers.py:36-43)
         return targets.LineFit(x, y, yerr).ln_like(theta)
 
     runs = [("device target", dict(ln=fit.ln_like), 20000, 300),
+            ("CUDA source plug-in", dict(ln=lnprob_scalar, ln_like_cuda=lik,
+                                         ln_kwargs=dict(x=fit.x, y=fit.y, yerr=fit.yerr)), 20000, 300),
             ("batched torch plug-in", dict(ln=lnprob_scalar, ln_like_batched=lnprob_batched,
                                            ln_kwargs=dict(x=fit.x, y=fit.y, yerr=fit.yerr)), 20000, 300),
             ("scalar host plug-in", dict(ln=lnprob_scalar, ln_kwargs=dict(x=fit.x, y=fit.y, yerr=fit.yerr)), 64, 300)]

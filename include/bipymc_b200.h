@@ -42,6 +42,7 @@ extern "C" {
 #define BPM_TARGET_GAUSS 3    /* bipymc/utils/d100_gauss.py:14-35  params: mu[d], W[d][r], c0      */
 #define BPM_TARGET_LINEFIT 4  /* examples/ex_para_fit.py:39-55     params: x[M], y[M], yerr[M]     */
 #define BPM_TARGET_EXPFIT 5   /* examples/ex_exp_fit.py:38-121     params: t[M], y[M]; dim = 5     */
+#define BPM_TARGET_JIT 6      /* user CUDA source compiled at run time: bpm_set_jit_target only   */
 
 typedef struct bpm_engine* bpm_handle;
 typedef void* bpm_stream; /* cudaStream_t */
@@ -141,6 +142,24 @@ int bpm_set_run_params(bpm_handle h, double flip, int32_t shuffle, double epsilo
  * samplers.py:43).  `params` is a HOST array; layout per target in DESIGN.md. */
 int bpm_set_target(bpm_handle h, int32_t target, const double* params, int64_t n_params);
 int bpm_set_batched_lnl(bpm_handle h, bpm_lnl_fn fn, void* user);
+
+/* Run-time compiled likelihood (BPM_TARGET_JIT).  `source` is CUDA C++ defining
+ *   __device__ double ln_like(const double* theta, const double* data)
+ * with theta[BPM_DIM] and data[BPM_NDATA] (both defined as macros; the bpm:: helpers of the
+ * library's targets.cuh and the CUDA math functions are in scope).  -inf = outside the prior.
+ * The library compiles it with NVRTC for sm_100a together with its own d <= 4 chain-step kernel
+ * and a batched row kernel, so the likelihood runs inside the generation kernels.  NVRTC is
+ * loaded on first use from $BIPYMC_B200_NVRTC, else the toolkit holding nvcc, else the default
+ * loader path.  Compiled cubins are cached for the life of the process (key: translation unit
+ * + options); *from_cache (may be NULL) is set to 1 when the cubin came from there.
+ * flags: bit 0 = fmad (contract multiply-adds; 0 gives IEEE + - * / rounding of every operation).
+ * On a compile error the NVRTC log (line numbers of `source` as "ln_like.cu(line)") goes into
+ * log[log_cap].  bpm_jit_compile needs no device.  bpm_set_jit_target compiles (or takes the
+ * cached cubin), loads it on the handle's device and copies data[n_data] (HOST) there. */
+int bpm_jit_compile(const char* source, int32_t dim, int64_t n_data, int32_t flags, int32_t* from_cache,
+                    char* log, int64_t log_cap);
+int bpm_set_jit_target(bpm_handle h, const char* source, const double* data, int64_t n_data, int32_t flags,
+                       int32_t* from_cache, char* log, int64_t log_cap);
 
 /* ln_like for n rows (device in, device out) with the current target. */
 int bpm_eval_lnl(bpm_handle h, const double* X, int32_t n, double* lnl, bpm_stream stream);

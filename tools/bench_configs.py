@@ -3,6 +3,11 @@
 (bench.py measures configs[1]).  Prints one JSON line per configuration:
   c3  DREAM, bimodal 2-D Gaussian, 10^6 chains, CR adaptation + outlier reset on, no history
   c4  DREAM, line fit (3 parameters, 50 data points), 10^5 chains
+  c4_cuda_same / c4_cuda / c4_torch  the same run with the likelihood as a run-time compiled CUDA
+      source calling the built-in's bpm::linefit_lnl / in the reference's per-term form (fmad=False) /
+      as examples/ex_para_fit_b200.py's batched torch function
+  expfit / expfit_cuda / expfit_torch  DREAM on the 5-parameter exp fit (60 points), 10^5 chains:
+      built-in split path / the reference's form as CUDA source (fmad=False) / torch ops
   demc100  DE-MC on the 100-D Gaussian, 10^5 chains (32 d + 16 bytes per chain-step)
 Device-resident timing with CUDA events, same rules as bench.py."""
 import json
@@ -15,7 +20,7 @@ import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 
-def run(name, make, N, d, bytes_per_step, gens=100, warm=20):
+def run(name, make, N, d, bytes_per_step, gens=100, warm=20, extra=None):
     from bipymc_b200 import _lib
     np.random.seed(1)
     s = make()
@@ -43,15 +48,89 @@ def run(name, make, N, d, bytes_per_step, gens=100, warm=20):
     _lib.check(s._libh.bpm_profile(s._handle, 0))
     kinds = ["split", "propose", "likelihood", "accept", "fused_phase", "cr_reduce", "other6", "other7"]
     kms = dict((kinds[i], {"avg_ms": ms_k[i] / n_k[i], "per_generation": n_k[i] / pg}) for i in range(8) if n_k[i])
-    print(json.dumps({"config": name, "n_chains": N, "dim": d, "chain_steps_per_s": v, "ms_per_generation": ms / gens,
+    print(json.dumps(dict({"config": name, "n_chains": N, "dim": d, "chain_steps_per_s": v, "ms_per_generation": ms / gens,
                       "algorithmic_bytes_per_chain_step": bytes_per_step,
                       "algorithmic_GBps": v * bytes_per_step / 1e9, "frac_of_hbm_peak": v * bytes_per_step / 1e9 / peak,
-                      "acceptance_fraction": s.acceptance_fraction, "launches_event_pass": kms}))
+                      "acceptance_fraction": s.acceptance_fraction, "launches_event_pass": kms}, **(extra or {}))))
+    s.close()
+
+
+LINEFIT_SAME = r'''
+__device__ double ln_like(const double* theta, const double* data) {
+  const int M = BPM_NDATA / 3;
+  return bpm::linefit_lnl(data, data + M, data + 2 * M, M, theta[0], theta[1], theta[2]);
+}
+'''
+
+# ex_exp_fit.py:73-121 as written there (one data point at a time); data = t[M], y[M]
+EXPFIT_CUDA = r'''
+__device__ double ln_like(const double* th, const double* data) {
+  const int M = BPM_NDATA / 2;
+  const double tau = th[0], c_inf = th[1], c_0 = th[2], leak = th[3], sigma = th[4];
+  if (!(-5.0 < c_inf && c_inf < 5.0 && 1.0 < tau && tau < 50.0 && -1.0 < c_0 && c_0 < 1.0 &&
+        -5.0 < leak && leak < 5.0 && 0.0 < sigma && sigma < 1.0)) return -INFINITY;
+  double s = 0.0;
+  for (int i = 0; i < M; ++i) {
+    const double t = data[i];
+    const double m = c_inf + c_0 * -1.0 * exp(-t / tau) - leak * t;
+    s += (m - data[M + i]) * (m - data[M + i]) / sigma - log(1.0 / sigma);
+  }
+  return 0.0 + -0.5 * s;
+}
+'''
+
+
+def _expfit_torch(t, y):
+    def lnprob(th):
+        tau, c_inf, c_0, leak, sigma = (th[:, i:i + 1] for i in range(5))
+        m = c_inf + c_0 * -1.0 * torch.exp(-t[None, :] / tau) - leak * t[None, :]
+        ll = 0.0 + -0.5 * ((m - y[None, :]) ** 2 / sigma - torch.log(1.0 / sigma)).sum(dim=1)
+        ok = (th[:, 1] > -5) & (th[:, 1] < 5) & (th[:, 0] > 1) & (th[:, 0] < 50) & (th[:, 2] > -1) & (th[:, 2] < 1) & \
+             (th[:, 3] > -5) & (th[:, 3] < 5) & (th[:, 4] > 0) & (th[:, 4] < 1)
+        return torch.where(ok, ll, torch.full_like(ll, -float("inf")))
+    return lnprob
+
+
+def _plain(target):
+    """The target's scalar ln_like hidden behind a lambda: a built-in target's own method would select the
+    built-in device likelihood, which takes precedence over ln_like_batched."""
+    return lambda theta: target.ln_like(theta)
+
+
+def _nvrtc_loaded():
+    """Path (symlinks resolved: the file name carries the version) of the NVRTC this process loaded."""
+    with open("/proc/self/maps") as f:
+        for line in f:
+            if "libnvrtc.so" in line:
+                return os.path.realpath(line.split()[-1])
+    return None
+
+
+def _cuda_lik(src, dim, data, fmad):
+    """CudaLikelihood plus its compile time: first compile of the source in this process, then the cached one."""
+    import time
+    from bipymc_b200 import targets
+    lik = targets.CudaLikelihood(src, dim, data, fmad=fmad)
+    t0 = time.perf_counter()
+    first_cached = lik.compile()
+    t1 = time.perf_counter()
+    assert lik.compile()
+    t2 = time.perf_counter()
+    return lik, {"compile_s": t1 - t0, "compile_was_cached": first_cached, "compile_cached_s": t2 - t1,
+                 "nvrtc": _nvrtc_loaded()}
 
 
 def main():
     from bipymc_b200 import DreamMpi, DeMcMpi, targets
     which = sys.argv[1:] or ["c3", "c4", "demc100", "c5shape"]
+    c4_kw = dict(n_chains=100000, seed=3, varepsilon=1e-2, history="none", burnin_gen=10 ** 6, n_cr_gen=10)
+    c4_bytes = 64 * 3 + 16 + 32 * 3 + 8 * 3
+    ex_kw = dict(n_chains=100000, seed=3, varepsilon=np.asarray([1e-2, 1e-2, 1e-3, 1e-8, 1e-9]) * 1e-2,
+                 history="none", burnin_gen=10 ** 6, n_cr_gen=10)                   # ex_exp_fit.py:135
+    ex_bytes = 64 * 5 + 16 + 32 * 5 + 8 * 5
+    ex_th0 = [12.0, 1.5, 0.6, 1e-3, 2e-3]
+    lf, ef = targets.LineFit(), targets.ExpFit()
+    lf_data, ef_data = np.concatenate([lf.x, lf.y, lf.yerr]), np.concatenate([ef.t, ef.y])
     if "c3" in which:
         N = 1000000
         t = targets.BimodeGauss_2D(log_of_pdf=False)
@@ -65,6 +144,34 @@ def main():
         run("c4 linefit DREAM 1e5 chains", lambda: DreamMpi(t.ln_like, [-0.8, 4.5, 0.2], n_chains=N, seed=3,
                                                               varepsilon=1e-2, history="none", burnin_gen=10 ** 6,
                                                               n_cr_gen=10), N, 3, 64 * 3 + 16 + 32 * 3 + 8 * 3)
+    if "c4_cuda_same" in which:
+        lik, info = _cuda_lik(LINEFIT_SAME, 3, lf_data, True)
+        run("c4_cuda_same linefit (bpm::linefit_lnl as CUDA source) DREAM 1e5 chains",
+            lambda: DreamMpi(lf.ln_like, [-0.8, 4.5, 0.2], ln_like_cuda=lik, **c4_kw), 100000, 3, c4_bytes, extra=info)
+    if "c4_cuda" in which:
+        sys.path.insert(0, os.path.join(ROOT, "examples"))
+        from ex_para_fit_b200 import LNPROB_CUDA
+        lik, info = _cuda_lik(LNPROB_CUDA, 3, lf_data, False)
+        run("c4_cuda linefit (reference per-term form as CUDA source, fmad=False) DREAM 1e5 chains",
+            lambda: DreamMpi(lf.ln_like, [-0.8, 4.5, 0.2], ln_like_cuda=lik, **c4_kw), 100000, 3, c4_bytes, extra=info)
+    if "c4_torch" in which:
+        sys.path.insert(0, os.path.join(ROOT, "examples"))
+        from ex_para_fit_b200 import make_lnprob_batched
+        fb = make_lnprob_batched(*(torch.from_numpy(v).cuda() for v in (lf.x, lf.y, lf.yerr)))
+        assert DreamMpi(_plain(lf), [-0.8, 4.5, 0.2], ln_like_batched=fb, n_chains=8)._mode() == "batched"
+        run("c4_torch linefit (batched torch plug-in) DREAM 1e5 chains",
+            lambda: DreamMpi(_plain(lf), [-0.8, 4.5, 0.2], ln_like_batched=fb, **c4_kw), 100000, 3, c4_bytes,
+            gens=50, warm=10)
+    if "expfit" in which:
+        run("expfit DREAM d=5 1e5 chains (built-in)", lambda: DreamMpi(ef.ln_like, ex_th0, **ex_kw), 100000, 5, ex_bytes)
+    if "expfit_cuda" in which:
+        lik, info = _cuda_lik(EXPFIT_CUDA, 5, ef_data, False)
+        run("expfit_cuda DREAM d=5 1e5 chains (reference form as CUDA source, fmad=False)",
+            lambda: DreamMpi(ef.ln_like, ex_th0, ln_like_cuda=lik, **ex_kw), 100000, 5, ex_bytes, extra=info)
+    if "expfit_torch" in which:
+        fe = _expfit_torch(*(torch.from_numpy(v).cuda() for v in (ef.t, ef.y)))
+        run("expfit_torch DREAM d=5 1e5 chains (batched torch plug-in)",
+            lambda: DreamMpi(_plain(ef), ex_th0, ln_like_batched=fe, **ex_kw), 100000, 5, ex_bytes, gens=50, warm=10)
     if "demc100" in which:
         N = 100000
         t = targets.Gauss_100D()

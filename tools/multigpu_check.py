@@ -14,6 +14,13 @@ import torch.distributed as dist
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
+LINEFIT_CUDA = r'''
+__device__ double ln_like(const double* theta, const double* data) {
+  const int M = BPM_NDATA / 3;
+  return bpm::linefit_lnl(data, data + M, data + 2 * M, M, theta[0], theta[1], theta[2]);
+}
+'''
+
 
 def main():
     rank = int(os.environ["RANK"])
@@ -24,6 +31,7 @@ def main():
     from bipymc_b200 import DreamMpi, DeMcMpi, targets
     from bipymc_b200.demc import _SingleComm
     world = dist.get_world_size()
+    lf = targets.LineFit()
     cases = [
         ("dream-gauss100", DreamMpi, targets.Gauss_100D(), np.zeros(100), 4096 + 2 * world, dict(burnin_gen=0), 1.0),
         ("dream-gauss100-adapt", DreamMpi, targets.Gauss_100D(), np.zeros(100), 2048, dict(burnin_gen=1000, n_cr_gen=2), 1.0),
@@ -32,6 +40,10 @@ def main():
         ("dream-gauss128", DreamMpi, targets.Gauss_100D(dim=128), np.zeros(128), 640 + 2 * world, dict(burnin_gen=0), 1.0),
         ("dream-linefit-outlier", DreamMpi, targets.LineFit(), [-0.8, 4.5, 0.2], 512 * world,
          dict(burnin_gen=1000, n_cr_gen=3, outlier_gen=5), 1e-2),
+        # user likelihood compiled at run time (BPM_TARGET_JIT): the fused d <= 4 kernel with in-kernel peer stores
+        ("dream-linefit-cuda", DreamMpi, lf, [-0.8, 4.5, 0.2], 512 * world,
+         dict(burnin_gen=0, ln_like_cuda=targets.CudaLikelihood(LINEFIT_CUDA, 3, np.concatenate([lf.x, lf.y, lf.yerr]))),
+         1e-2),
     ]
     G = 12
     runs = [(c, ex) for c in cases for ex in ("p2p", "allgather")]
