@@ -13,8 +13,8 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("BIPYMC_B200_LIB") or os.path.join(_HERE, "lib", "libbipymc_b200.so")
 
 BPM_ALGO_DEMC, BPM_ALGO_DREAM, BPM_ALGO_DEMC_SERIAL = 0, 1, 2
-TARGET_EXTERNAL, TARGET_BANANA, TARGET_BIMODAL, TARGET_GAUSS, TARGET_LINEFIT, TARGET_EXPFIT, TARGET_JIT = \
-    0, 1, 2, 3, 4, 5, 6
+TARGET_EXTERNAL, TARGET_BANANA, TARGET_BIMODAL, TARGET_GAUSS, TARGET_LINEFIT, TARGET_EXPFIT, TARGET_JIT, \
+    TARGET_JIT_SUM = 0, 1, 2, 3, 4, 5, 6, 7
 BPM_MAX_PAIRS, BPM_MAX_CR, BPM_MAX_PEERS = 8, 16, 15
 
 
@@ -63,6 +63,10 @@ SIGNATURES = {
                                   C.c_int64]),
     "bpm_set_jit_target": (C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(C.c_double), C.c_int64, C.c_int32,
                                      C.POINTER(C.c_int32), C.c_char_p, C.c_int64]),
+    "bpm_jit_compile_sum": (C.c_int, [C.c_char_p, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.POINTER(C.c_int32),
+                                      C.c_char_p, C.c_int64]),
+    "bpm_set_jit_sum_target": (C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(C.c_double), C.c_int64, C.c_int32,
+                                         C.c_int32, C.POINTER(C.c_int32), C.c_char_p, C.c_int64]),
     "bpm_eval_lnl": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),
     "bpm_set_cr_state": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_double),
                                    C.POINTER(C.c_double)]),

@@ -24,6 +24,10 @@ Likelihood plug-ins, fastest first:
      ``fmad=False`` rounds like numpy.  The first compile takes up to about 2 s, later samplers with the
      same source reuse the cubin.  Takes precedence over a built-in target and over
      ``ln_like_batched``; ``ln_like_fn`` stays the drop-in positional argument and is not called;
+  1c. ``ln_like_cuda=targets.CudaSumLikelihood(source, dim, data, prior)``: a likelihood that is a sum
+     of ``__device__ double ln_like_term(const double* theta, const double* row)`` over the rows of
+     ``data[M][k]`` (plus an optional ``ln_prior``), each chain's sum split over the whole GPU between
+     the proposal and accept kernels, in an order fixed by M alone;
   2. ``ln_like_batched=f``: ``f(theta)`` takes a CUDA float64 tensor ``[n, dim]`` and
      returns ``[n]`` log-likelihoods (torch ops on the current stream);
   3. any scalar ``ln_like_fn(theta, **ln_kwargs) -> float`` exactly as in the reference
@@ -432,7 +436,7 @@ class DeMcMpi(object):
         if self._ln_like_cuda is not None:
             from .targets import CudaLikelihood
             if not isinstance(self._ln_like_cuda, CudaLikelihood):
-                raise TypeError("ln_like_cuda must be a targets.CudaLikelihood")
+                raise TypeError("ln_like_cuda must be a targets.CudaLikelihood or targets.CudaSumLikelihood")
             if self._ln_like_cuda.dim != d:
                 raise ValueError("ln_like_cuda dimension %d != theta_0 dimension %d" % (self._ln_like_cuda.dim, d))
         self._ld = d if d <= 4 else ((d + 3) // 4) * 4

@@ -10,7 +10,8 @@ Mirrors the reference's test-target classes (same constructor arguments, same ``
   ExpFit          examples/ex_exp_fit.py:38-121 (5-parameter relaxation fit)
 
 and ``CudaLikelihood``: any other model as CUDA C++ source, compiled at run time into the same
-kernels (``ln_like_cuda=`` of the samplers).
+kernels (``ln_like_cuda=`` of the samplers); ``CudaSumLikelihood``: a model that is a sum over
+observations, one CUDA C++ term per observation, summed across the whole GPU.
 
 ``ln_like`` stays a scalar host function, so the objects remain valid ``ln_like_fn``
 arguments everywhere; when a sampler of this package receives ``obj.ln_like`` it
@@ -351,3 +352,75 @@ class CudaLikelihood(object):
         """Compile (or take the cached cubin), load it on the handle's device and copy the data."""
         return self._call(lib.bpm_set_jit_target, handle, self.source.encode(), _lib.dptr(self.data),
                           self.data.size, self._flags)
+
+
+class CudaSumLikelihood(CudaLikelihood):
+    """A likelihood that is a sum over independent observations, in CUDA C++: the library splits the
+    sum across the whole GPU.  ``source`` defines::
+
+        __device__ double ln_like_term(const double* theta, const double* row);   // one observation
+        __device__ double ln_prior(const double* theta);                          // only when prior=True
+
+    ``data`` is a finite float64 array of shape ``(M, k)`` (a 1-D array is ``(M, 1)``), ``row`` points at
+    the k values of one observation.  ``BPM_DIM``, ``BPM_NROWS`` (M) and ``BPM_ROWLEN`` (k) are macros;
+    the scope, ``fmad``, the NaN rule, the compile cache and ``CudaCompileError`` are those of
+    ``CudaLikelihood`` (M, k and ``prior`` are part of the cache key).  The value is::
+
+        ln L(theta) = ln_prior(theta) + sum_{i < M} ln_like_term(theta, row_i)
+
+    and ``-inf``, with no term of that chain evaluated, when ``ln_prior`` is ``-inf``.
+
+    The order of the additions depends on M alone, never on the number of chains, the batch size, the
+    launch shape or the number of GPUs, so a given theta always gets the same bits: rows are cut into
+    chunks of 256 consecutive rows (the last padded with 0.0 terms); inside a chunk a halving pairwise
+    tree adds ``a[i] + a[i + w/2]`` for w = 256, 128, ..., 2; the chunk partials, padded with 0.0 to the
+    next power of two, are added by an adjacent-pair tree ``p[2i] + p[2i+1]``, level by level; the prior
+    is added last.  In numpy::
+
+        a = np.zeros((nc, 256)); a.flat[:M] = terms
+        while a.shape[1] > 1: a = a[:, :a.shape[1] // 2] + a[:, a.shape[1] // 2:]
+        p = np.zeros(P2); p[:nc] = a[:, 0]
+        while p.size > 1: p = p[0::2] + p[1::2]
+        lnl = prior + p[0]
+
+    Which form to use: ``CudaLikelihood`` (one ``ln_like`` per chain) for a model that is not a sum over
+    observations, or for small data at d <= 4, where it runs fused into the one-thread-per-chain step
+    kernel.  ``CudaSumLikelihood`` for many observations or few chains: every chain's sum is spread over
+    all SMs, between the proposal and accept kernels at every d.  Pass it as ``ln_like_cuda=``."""
+
+    def __init__(self, source, dim, data, prior=False, fmad=True):
+        if not isinstance(source, str):
+            raise ValueError("source must be a str of CUDA C++")
+        if isinstance(dim, bool) or int(dim) != dim or int(dim) < 1:
+            raise ValueError("dim must be an integer >= 1")
+        data = np.asarray(data, dtype=np.float64)
+        if data.ndim == 1:
+            data = data.reshape(-1, 1)
+        if data.ndim != 2 or data.shape[0] < 1 or data.shape[1] < 1:
+            raise ValueError("data must have shape (M, k) with M >= 1 and k >= 1 (or be 1-D with M >= 1)")
+        if data.shape[0] >= 2 ** 31:
+            raise ValueError("data must have fewer than 2^31 rows")
+        if not np.all(np.isfinite(data)):
+            raise ValueError("data must be finite")
+        self.source = source
+        self.dim = int(dim)
+        self.data = np.ascontiguousarray(data)
+        self.prior = bool(prior)
+        self.fmad = bool(fmad)
+
+    @property
+    def _flags(self):
+        return (1 if self.fmad else 0) | (2 if self.prior else 0)
+
+    def compile(self):
+        """Compile for sm_100a (no device needed).  Returns True when the cubin came from the
+        process cache; raises CudaCompileError with the NVRTC log."""
+        lib = _lib.load()
+        M, k = self.data.shape
+        return self._call(lib.bpm_jit_compile_sum, self.source.encode(), self.dim, M, k, self._flags)
+
+    def _attach(self, lib, handle):
+        """Compile (or take the cached cubin), load it on the handle's device and copy the data."""
+        M, k = self.data.shape
+        return self._call(lib.bpm_set_jit_sum_target, handle, self.source.encode(), _lib.dptr(self.data), M, k,
+                          self._flags)

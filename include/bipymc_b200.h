@@ -43,6 +43,7 @@ extern "C" {
 #define BPM_TARGET_LINEFIT 4  /* examples/ex_para_fit.py:39-55     params: x[M], y[M], yerr[M]     */
 #define BPM_TARGET_EXPFIT 5   /* examples/ex_exp_fit.py:38-121     params: t[M], y[M]; dim = 5     */
 #define BPM_TARGET_JIT 6      /* user CUDA source compiled at run time: bpm_set_jit_target only   */
+#define BPM_TARGET_JIT_SUM 7  /* per-observation CUDA source, summed: bpm_set_jit_sum_target only */
 
 typedef struct bpm_engine* bpm_handle;
 typedef void* bpm_stream; /* cudaStream_t */
@@ -160,6 +161,26 @@ int bpm_jit_compile(const char* source, int32_t dim, int64_t n_data, int32_t fla
                     char* log, int64_t log_cap);
 int bpm_set_jit_target(bpm_handle h, const char* source, const double* data, int64_t n_data, int32_t flags,
                        int32_t* from_cache, char* log, int64_t log_cap);
+
+/* Run-time compiled per-observation likelihood (BPM_TARGET_JIT_SUM).  `source` is CUDA C++ defining
+ *   __device__ double ln_like_term(const double* theta, const double* row)   -- one observation
+ *   __device__ double ln_prior(const double* theta)                          -- only with flags bit 1
+ * with theta[BPM_DIM] and row[BPM_ROWLEN]; BPM_NROWS (M) is defined too, and the scope is that of
+ * bpm_jit_compile.  data is the row-major [n_rows][row_len] array (HOST), 1 <= n_rows < 2^31.
+ *   ln L = ln_prior(theta) + sum over the M rows of ln_like_term(theta, row)
+ * (-inf, with no term evaluated, when ln_prior is -inf).  The terms are added in an order fixed by M
+ * alone -- chunks of 256 rows, a pairwise tree inside each chunk, an adjacent-pair tree over the chunk
+ * partials padded to a power of two, the prior last (bipymc_b200/csrc/kernels_sum.cuh) -- so a given
+ * theta gets the same bits whatever the number of chains, the batch size of bpm_eval_lnl, the launch
+ * shape or the number of GPUs.  The sum is split over the whole GPU (tiles of chains x groups of
+ * chunks); the group partials take at most 2^22 doubles of workspace.  The likelihood runs between
+ * the propose and accept kernels at every dim (never in the fused d <= 4 kernel), in serial DE-MC and
+ * in bpm_eval_lnl.  flags: bit 0 = fmad, bit 1 = the source defines ln_prior.  Cache, log and
+ * from_cache as for bpm_jit_compile; M and row_len are part of the cache key. */
+int bpm_jit_compile_sum(const char* source, int32_t dim, int64_t n_rows, int32_t row_len, int32_t flags,
+                        int32_t* from_cache, char* log, int64_t log_cap);
+int bpm_set_jit_sum_target(bpm_handle h, const char* source, const double* data, int64_t n_rows, int32_t row_len,
+                           int32_t flags, int32_t* from_cache, char* log, int64_t log_cap);
 
 /* ln_like for n rows (device in, device out) with the current target. */
 int bpm_eval_lnl(bpm_handle h, const double* X, int32_t n, double* lnl, bpm_stream stream);

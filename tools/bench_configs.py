@@ -8,6 +8,10 @@
       as examples/ex_para_fit_b200.py's batched torch function
   expfit / expfit_cuda / expfit_torch  DREAM on the 5-parameter exp fit (60 points), 10^5 chains:
       built-in split path / the reference's form as CUDA source (fmad=False) / torch ops
+  expfit_sum_N<N>_M<M> / expfit_cuda_N<N>_M<M>  the exp fit on targets.expfit_data(n=M) with N chains, as a
+      per-observation CudaSumLikelihood / as a whole-function CudaLikelihood (both fmad=False, the reference's
+      arithmetic): N1024_M1e5, N1e5_M1e4, N1024_M1e6 (sum only)
+  c4_sum  c4 with the reference's per-term line fit as a CudaSumLikelihood (fmad=False), against c4_cuda
   demc100  DE-MC on the 100-D Gaussian, 10^5 chains (32 d + 16 bytes per chain-step)
 Device-resident timing with CUDA events, same rules as bench.py."""
 import json
@@ -20,7 +24,7 @@ import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 
-def run(name, make, N, d, bytes_per_step, gens=100, warm=20, extra=None):
+def run(name, make, N, d, bytes_per_step, gens=100, warm=20, extra=None, terms_per_gen=None):
     from bipymc_b200 import _lib
     np.random.seed(1)
     s = make()
@@ -48,6 +52,8 @@ def run(name, make, N, d, bytes_per_step, gens=100, warm=20, extra=None):
     _lib.check(s._libh.bpm_profile(s._handle, 0))
     kinds = ["split", "propose", "likelihood", "accept", "fused_phase", "cr_reduce", "other6", "other7"]
     kms = dict((kinds[i], {"avg_ms": ms_k[i] / n_k[i], "per_generation": n_k[i] / pg}) for i in range(8) if n_k[i])
+    if terms_per_gen:       # likelihood terms (chains x observations) per generation over likelihood time per generation
+        extra = dict(extra or {}, terms_per_s=terms_per_gen / (ms_k[2] / pg * 1e-3), likelihood_avg_ms=ms_k[2] / n_k[2])
     print(json.dumps(dict({"config": name, "n_chains": N, "dim": d, "chain_steps_per_s": v, "ms_per_generation": ms / gens,
                       "algorithmic_bytes_per_chain_step": bytes_per_step,
                       "algorithmic_GBps": v * bytes_per_step / 1e9, "frac_of_hbm_peak": v * bytes_per_step / 1e9 / peak,
@@ -80,6 +86,35 @@ __device__ double ln_like(const double* th, const double* data) {
 '''
 
 
+# the same two models per observation (targets.CudaSumLikelihood); rows = (t, y) / (x, y, yerr)
+EXPFIT_TERM = r'''
+__device__ double ln_like_term(const double* th, const double* row) {
+  const double m = th[1] + th[2] * -1.0 * exp(-row[0] / th[0]) - th[3] * row[0];
+  return -0.5 * ((m - row[1]) * (m - row[1]) / th[4] - log(1.0 / th[4]));
+}
+'''
+EXPFIT_PRIOR = r'''
+__device__ double ln_prior(const double* th) {
+  const double tau = th[0], c_inf = th[1], c_0 = th[2], leak = th[3], sigma = th[4];
+  return (-5.0 < c_inf && c_inf < 5.0 && 1.0 < tau && tau < 50.0 && -1.0 < c_0 && c_0 < 1.0 &&
+          -5.0 < leak && leak < 5.0 && 0.0 < sigma && sigma < 1.0) ? 0.0 : -INFINITY;
+}
+'''
+LINEFIT_TERM = r'''
+__device__ double ln_like_term(const double* theta, const double* row) {
+  const double model = theta[0] * row[0] + theta[1];
+  const double inv = 1.0 / (row[2] * row[2] + model * model * exp(2.0 * theta[2]));
+  return -0.5 * ((row[1] - model) * (row[1] - model) * inv - log(inv));
+}
+'''
+LINEFIT_PRIOR = r'''
+__device__ double ln_prior(const double* theta) {
+  const double m = theta[0], b = theta[1], lnf = theta[2];
+  return (-5.0 < m && m < 0.5 && 0.0 < b && b < 10.0 && -10.0 < lnf && lnf < 1.0) ? 0.0 : -INFINITY;
+}
+'''
+
+
 def _expfit_torch(t, y):
     def lnprob(th):
         tau, c_inf, c_0, leak, sigma = (th[:, i:i + 1] for i in range(5))
@@ -106,11 +141,12 @@ def _nvrtc_loaded():
     return None
 
 
-def _cuda_lik(src, dim, data, fmad):
-    """CudaLikelihood plus its compile time: first compile of the source in this process, then the cached one."""
+def _cuda_lik(src, dim, data, fmad, cls=None, **kw):
+    """CudaLikelihood (or cls) plus its compile time: first compile of the source in this process, then the cached
+    one."""
     import time
     from bipymc_b200 import targets
-    lik = targets.CudaLikelihood(src, dim, data, fmad=fmad)
+    lik = (cls or targets.CudaLikelihood)(src, dim, data, fmad=fmad, **kw)
     t0 = time.perf_counter()
     first_cached = lik.compile()
     t1 = time.perf_counter()
@@ -172,6 +208,27 @@ def main():
         fe = _expfit_torch(*(torch.from_numpy(v).cuda() for v in (ef.t, ef.y)))
         run("expfit_torch DREAM d=5 1e5 chains (batched torch plug-in)",
             lambda: DreamMpi(_plain(ef), ex_th0, ln_like_batched=fe, **ex_kw), 100000, 5, ex_bytes, gens=50, warm=10)
+    sum_runs = {"expfit_sum_N1024_M1e5": (1024, 100000), "expfit_cuda_N1024_M1e5": (1024, 100000),
+                "expfit_sum_N1e5_M1e4": (100000, 10000), "expfit_cuda_N1e5_M1e4": (100000, 10000),
+                "expfit_sum_N1024_M1e6": (1024, 1000000)}
+    for name in [w for w in which if w in sum_runs]:
+        N, M = sum_runs[name]
+        t, y = targets.expfit_data(n=M)
+        if "_sum_" in name:
+            lik, info = _cuda_lik(EXPFIT_TERM + EXPFIT_PRIOR, 5, np.stack([t, y], 1), False, targets.CudaSumLikelihood,
+                                  prior=True)
+        else:
+            lik, info = _cuda_lik(EXPFIT_CUDA, 5, np.concatenate([t, y]), False)
+        slow = N * M >= 10 ** 9
+        run(name + " DREAM d=5 exp fit", lambda: DreamMpi(ef.ln_like, ex_th0, ln_like_cuda=lik, **dict(ex_kw, n_chains=N)),
+            N, 5, ex_bytes, gens=10 if slow else 50, warm=3 if slow else 10, extra=dict(info, n_obs=M),
+            terms_per_gen=N * M)
+    if "c4_sum" in which:
+        lik, info = _cuda_lik(LINEFIT_TERM + LINEFIT_PRIOR, 3, np.stack([lf.x, lf.y, lf.yerr], 1), False,
+                              targets.CudaSumLikelihood, prior=True)
+        run("c4_sum linefit (reference per-term form as CudaSumLikelihood, fmad=False) DREAM 1e5 chains",
+            lambda: DreamMpi(lf.ln_like, [-0.8, 4.5, 0.2], ln_like_cuda=lik, **c4_kw), 100000, 3, c4_bytes,
+            extra=dict(info, n_obs=lf.x.size), terms_per_gen=100000 * lf.x.size)
     if "demc100" in which:
         N = 100000
         t = targets.Gauss_100D()

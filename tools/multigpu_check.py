@@ -20,6 +20,14 @@ __device__ double ln_like(const double* theta, const double* data) {
   return bpm::linefit_lnl(data, data + M, data + 2 * M, M, theta[0], theta[1], theta[2]);
 }
 '''
+LINEFIT_TERM = r'''
+__device__ double ln_like_term(const double* theta, const double* row) {
+  const double model = theta[0] * row[0] + theta[1];
+  const double inv = 1.0 / (row[2] * row[2] + model * model * exp(2.0 * theta[2]));
+  const double r = row[1] - model;
+  return -0.5 * (r * r * inv - log(inv));
+}
+'''
 
 
 def main():
@@ -43,6 +51,10 @@ def main():
         # user likelihood compiled at run time (BPM_TARGET_JIT): the fused d <= 4 kernel with in-kernel peer stores
         ("dream-linefit-cuda", DreamMpi, lf, [-0.8, 4.5, 0.2], 512 * world,
          dict(burnin_gen=0, ln_like_cuda=targets.CudaLikelihood(LINEFIT_CUDA, 3, np.concatenate([lf.x, lf.y, lf.yerr]))),
+         1e-2),
+        # per-observation source summed across the GPU (BPM_TARGET_JIT_SUM): the split path with device-counted lists
+        ("dream-linefit-cuda-sum", DreamMpi, lf, [-0.8, 4.5, 0.2], 512 * world,
+         dict(burnin_gen=0, ln_like_cuda=targets.CudaSumLikelihood(LINEFIT_TERM, 3, np.stack([lf.x, lf.y, lf.yerr], 1))),
          1e-2),
     ]
     G = 12
