@@ -2,21 +2,22 @@
 // state / moments / history update in ONE launch (demc.py:153-196, dream.py:32-107 for a
 // whole half of the population).
 //
-//  * fused_gauss_kernel  -- correlated-Gaussian target, d <= 112 (the 100-D headline
-//    case).  One persistent 512-thread CTA per SM; its two 256-thread halves work on
-//    different 64-chain tiles with their own named barrier, sharing one copy of the
-//    whitening matrix W (d x 112 doubles) in shared memory, so the HBM gather stage of
-//    one half overlaps the FP64 quadratic-form stage of the other.
-//      stage A  warp-per-chain: Philox draws, 7 coalesced row gathers, proposal -> smem tile
-//      stage B  Y = (P - mu) W as a register-tiled DFMA GEMM straight from smem
-//               (lanes = rows, warps = 14-column strips), folded into row sums of squares.
-//               B200 measures the same 36.5 TFLOP/s through DFMA and through DMMA
-//               (mma.sync m8n8k4 f64; tcgen05 has no FP64 kind), so the plain pipe is used.
-//      stage C  accept / reject, state + lnL + Welford moments + history row written once
-//  * fused_small_kernel  -- d <= 4 analytic targets (banana, bimodal, line fit),
-//    thread-per-chain (kernels_small.cuh, which the run-time compiled likelihoods share).
-// Both share every draw / arithmetic helper with the generic split path (step.cuh), so
-// the chains they produce are bit-identical to it.
+// Correlated-Gaussian target, 5 <= d <= 108 (the 100-D headline case), one persistent
+// warp-specialised CTA per SM: producer warps draw, gather and build the proposals of a
+// 64-chain tile, consumer warps run the quadratic form and the Metropolis decision.
+// gauss_fused_kernel (end of this file) picks the kernel from the shape:
+//  * fused_gauss_v4_kernel (kernels_fused_v4.cuh) -- the default: partner rows staged in
+//    shared memory by TMA, quadratic form on the FP64 tensor pipe (DMMA), lazy history /
+//    moments protocol (PhaseArgs::pending).  Needs d % 4 == 0, ld == d and its landing
+//    slots to fit shared memory.
+//  * fused_gauss_v3_kernel -- the same pipeline with register gathers, where v4's landing
+//    slots do not fit (larger d or more pairs), and on request (BPM_FUSED_GAUSS_V3).
+//  * fused_gauss_ws_kernel -- 12 producer / 8 DFMA consumer warps, eager write-back, where
+//    v3 / v4 cannot run (d % 4 != 0 or ld != d), and on request (BPM_FUSED_GAUSS_WS).
+// d <= 4 analytic targets (banana, bimodal, line fit): fused_small_kernel, thread per
+// chain (kernels_small.cuh, which the run-time compiled likelihoods share).
+// All of them share every draw / arithmetic helper with the generic split path (step.cuh),
+// so the chains they produce are bit-identical to it.
 #pragma once
 #include <cuda_runtime.h>
 #include "step.cuh"
@@ -29,10 +30,6 @@ constexpr int kTileRows = 64;    // chains per tile
 constexpr int kColStrip = 14;    // columns per warp in the quadratic form
 constexpr int kWld = 8 * kColStrip;  // padded row length of W in shared memory (112)
 constexpr int kHalfThreads = 256;
-
-__device__ __forceinline__ void half_barrier(int half) {
-  asm volatile("bar.sync %0, %1;" ::"r"(half + 1), "r"(kHalfThreads) : "memory");
-}
 
 // Row sums of squares of (P - mu) . W for a 64-row tile held in shared memory.
 //   P     [64][pld]   row-major, pld odd (conflict-free column walks)
@@ -545,51 +542,12 @@ __device__ __forceinline__ void tile_stage_writeback(const PhaseArgs& a, const T
   }
 }
 
-// Variant 1: two symmetric 256-thread halves per CTA, each running D -> A -> B -> C on its
-// own tile with its own named barrier (kept for A/B measurements: bpm_set_fused(h, 2)).
-template <bool REPLAY, bool CENTER>
-__global__ void __launch_bounds__(2 * kHalfThreads, 1)
-fused_gauss_kernel(const PhaseArgs a, const GaussArgs g) {
-  extern __shared__ __align__(16) double smem[];
-  const int d = a.d, pld = d | 1;
-  const GaussTables tb = carve_tables(smem, d);
-  const int half = threadIdx.x >> 8;
-  const int tid = threadIdx.x & (kHalfThreads - 1);
-  const int warp = tid >> 5, lane = tid & 31;
-  double* P = smem + gauss_table_doubles(d) + half * gauss_ptile_doubles(d);
-  double* part = P + (((size_t)kTileRows * pld + 1) & ~(size_t)1);
-  TileScratch& T = *reinterpret_cast<TileScratch*>(smem + gauss_table_doubles(d) +
-                                                   2 * gauss_ptile_doubles(d) +
-                                                   half * gauss_scratch_doubles());
-  fill_tables(a, g, tb, threadIdx.x, 2 * kHalfThreads);
-  __syncthreads();
-  const PhaseLists L = phase_lists(a);
-  const int n_tiles = (L.n_self + kTileRows - 1) / kTileRows;
-  unsigned n_acc = 0, n_rej = 0;
-  for (int tile = blockIdx.x * 2 + half; tile < n_tiles; tile += 2 * gridDim.x) {
-    tile_stage_draws<REPLAY>(a, L, tb, T, tile, tid, kHalfThreads);
-    half_barrier(half);
-    tile_stage_propose<REPLAY>(a, tb, T, P, pld, warp, 8, lane);
-    half_barrier(half);
-    gauss_tile_rowsums<CENTER>(P, pld, tb.Ws, tb.mus, d, part, warp, lane);
-    half_barrier(half);
-    if (tid < kTileRows) tile_stage_decide(a, g, T, part, tid, n_acc, n_rej);
-    half_barrier(half);
-    tile_stage_writeback(a, T, P, pld, warp, 8, lane);
-    half_barrier(half);   // the tile buffers are reused by the next iteration
-  }
-  if (lane == 0) {
-    if (n_acc) atomicAdd(a.n_acc, (unsigned long long)n_acc);
-    if (n_rej) atomicAdd(a.n_rej, (unsigned long long)n_rej);
-  }
-}
-
-// shared memory of both fused variants: tables, 2 proposal tiles, 3 scratch blocks
+// shared memory of fused_gauss_ws_kernel: tables, 2 proposal tiles, 3 scratch blocks
 inline size_t fused_gauss_smem(int d) {
   return sizeof(double) * (gauss_table_doubles(d) + 2 * gauss_ptile_doubles(d) + 3 * gauss_scratch_doubles());
 }
 
-// Variant 2 (default): warp-specialised producer / consumer pipeline.
+// fused_gauss_ws_kernel: warp-specialised producer / consumer pipeline.
 //   8 consumer warps (128 registers each) run nothing but the FP64 tile GEMM + the
 //   Metropolis decision; 12 producer warps (72 registers each) run the latency-bound
 //   stages -- draws, row gathers, proposal, write-back.  Two tile buffers rotate between
@@ -799,8 +757,8 @@ __device__ __forceinline__ int tile_stage_decide_reg(const PhaseArgs& a, const G
 }
 
 // =====================================================================================
-// Variant 3 (default): the same producer / consumer pipeline re-balanced after profiling
-// variant 2 (profiles/r1_v2_*): its 8 consumer warps sat at the FULL barrier 76 % of the
+// fused_gauss_v3_kernel: the same producer / consumer pipeline re-balanced after profiling
+// fused_gauss_ws_kernel (profiles/r1_v2_*): its 8 consumer warps sat at the FULL barrier 76 % of the
 // time while each of the 12 producer warps walked its chains serially at ~0.2 IPC.  Here
 //   * 8 consumer warps (64 registers) each own 8 rows of the tile product and run it on the FP64
 //     tensor pipe (mma.sync.m8n8k4.f64, W pre-arranged in fragment order in shared memory), decide
@@ -1268,189 +1226,43 @@ inline int launch_fused_v3(const PhaseArgs& a, const GaussArgs& g, int grid, siz
   return 0;
 }
 
-// d <= 4 in fly mode (unsharded, native RNG): thread = chain, in CHAIN order (16-byte rows share sectors, moments
-// and history stream) -- the chain finds its half from the inverse Feistel image of its own id, its partners from
-// the forward image of the pool positions it drew.  No split kernel, no list-packing kernels: a generation is two
-// of these launches plus the CR reduction (C4, 10^5 line-fit chains: 93 -> ~50 us per generation).
-template <int TARGET>
-__global__ void __launch_bounds__(128) fused_small_fly_kernel(const PhaseArgs a, const TargetView tv) {
-  extern __shared__ __align__(16) double sdata[];
-  if (TARGET == BPM_TARGET_LINEFIT) {
-    for (int i = threadIdx.x; i < 3 * tv.linefit_M; i += blockDim.x) sdata[i] = tv.linefit[i];
-    __syncthreads();
-  }
-  const int c = blockIdx.x * blockDim.x + threadIdx.x;
-  const bool self_first = (a.phase ^ a.flip_val) == 0;                 // this phase updates list positions [0, nA)
-  bool valid = c < a.N;
-  if (valid) {
-    const int pos = a.fly_shuffle ? (int)feistel_inv(a.fk, (uint32_t)c) : c;
-    valid = (pos < a.nA) == self_first;
-  }
-  int acc = 0;
-  if (valid) {
-    const int n_pool = self_first ? a.N - a.nA : a.nA, off = self_first ? a.nA : 0;
-    acc = small_chain_step<false, TARGET>(a, tv, sdata, c, n_pool, [&](int r) {
-      return a.fly_shuffle ? (int)feistel_perm(a.fk, (uint32_t)(off + r)) : off + r;
-    });
-  }
-  const unsigned am = __ballot_sync(0xFFFFFFFFu, valid && acc);
-  const unsigned rm = __ballot_sync(0xFFFFFFFFu, valid && !acc);
-  if ((threadIdx.x & 31) == 0) {
-    if (am) atomicAdd(a.n_acc, (unsigned long long)__popc(am));
-    if (rm) atomicAdd(a.n_rej, (unsigned long long)__popc(rm));
-  }
-}
-
-// ---- d <= 4: a whole run of generations in ONE persistent cooperative launch -----------------------------
-// (EXPERIMENTAL, bpm_set_fused(h, 6): measured slower than the per-phase launches -- 152 vs 91 us per generation at
-// 10^5 line-fit chains; every warp runs the chain-step twice with half its lanes, at 80 registers with spills.)
-// A generation of 10^5 three-parameter chains is ~10 us of work; launched as split + list packing + two
-// half-phases + CR reduction it costs 93 us (profiles/r1b_secondary_configs.txt: launch-bound).  Here one
-// cooperative grid keeps every generation of a bpm_step_generations call on the device (demc.py:79-135,
-// the whole while-loop):
-//   * no shuffle is materialised: a chain finds its half from the INVERSE Feistel permutation of its own id
-//     and its partners from the forward permutation of the pool positions it drew;
-//   * thread <-> chain is fixed, ONE chain per thread (chain order: 16-byte rows share sectors, moments /
-//     history stream).  A chain-step is a long dependent instruction sequence (the 50-point line-fit
-//     likelihood is ~25 us of latency), so the kernel only pays while every chain has its own resident thread:
-//     the engine uses it up to 148 x 3 x 256 chains and keeps the per-phase launches (which are throughput-bound
-//     there: C3, 10^6 chains) beyond;
-//   * three grid-wide barriers per generation: after phase a (its updates are phase b's partner states),
-//     after phase b, after the CR reduction (block partials in the per-phase kernels' own order -- bit-identical
-//     p_cr -- then block 0 applies dream.py:132-140).
-// Native RNG, unsharded handles; draws are addressed by chain id, so the chains are those of the per-phase path.
-struct SmallGens {
-  int64_t k_gen0;
-  int32_t n_gen, burnin_gen, n_cr_gen, jump_mod, shuffle;
-  double flip_p;
-  uint64_t seed;
-  double* hist0;           // row 0 of the flat history (or nullptr)
-  double* omega_sum;       // per-chain running sum of ln_like (outlier tracking) or nullptr
-  double* cr_block;        // [<= kCrBlocks][2 BPM_MAX_CR]
-  double* cr_part;
-  double* cr_dm;
-  double* cr_cnt;
-  double* p_cr;
-  int32_t cr_blocks;
-};
-
-}  // namespace bpm
-#include <cooperative_groups.h>
-namespace bpm {
-
-template <int TARGET>
-__global__ void __launch_bounds__(256, 3) small_generations_kernel(const PhaseArgs a0, const TargetView tv, const SmallGens q) {
-  namespace cg = cooperative_groups;
-  cg::grid_group grid = cg::this_grid();
-  extern __shared__ __align__(16) double sdata[];
-  __shared__ FeistelKey fkey;
-  __shared__ int flip_s;
-  if (TARGET == BPM_TARGET_LINEFIT) {
-    for (int i = threadIdx.x; i < 3 * tv.linefit_M; i += blockDim.x) sdata[i] = tv.linefit[i];
-  }
-  PhaseArgs a = a0;
-  const int N = a.N, nA = a.nA;
-  const int gtid = blockIdx.x * blockDim.x + threadIdx.x, nthreads = gridDim.x * blockDim.x;
-  const size_t hstride = (size_t)N * a.ld;
-  unsigned n_acc = 0, n_rej = 0;
-  for (int g = 0; g < q.n_gen; ++g) {
-    const int64_t k_gen = q.k_gen0 + g, hist_len = a0.hist_len + g, mom_len = a0.mom_len + g;
-    a.gamma_jump = (k_gen % q.jump_mod) == 0;                       // dream.py:77 / demc.py:174
-    a.adapt = a.algo == BPM_ALGO_DREAM && q.burnin_gen > k_gen && hist_len > q.n_cr_gen && a.m2 != nullptr;
-    a.hist_len = hist_len; a.mom_len = mom_len;
-    a.inv_mom = 1.0 / (double)mom_len;
-    a.inv_n1 = 1.0 / (double)(mom_len + 1);
-    a.rng = make_rng(q.seed, (uint64_t)hist_len);
-    a.hist_row = q.hist0 ? q.hist0 + (size_t)hist_len * hstride : nullptr;
-    if (threadIdx.x == 0) {                                          // demc.py:81-86, keyed by (seed, generation) only
-      const Philox4 f = draw4(a.rng, 0xFFFFFFFFu, RNG_GEN, 0);
-      const double thr = __ddiv_rn(q.flip_p, __dadd_rn(q.flip_p, __dsub_rn(1.0, q.flip_p)));
-      flip_s = u53(f.x, f.y) < thr ? 1 : 0;
-      if (q.shuffle) fkey = make_feistel(a.rng, (uint32_t)N);
-    }
-    __syncthreads();
-    const int flip = flip_s;
-    for (int ph = 0; ph < 2; ++ph) {
-      const bool self_first = (ph ^ flip) == 0;                      // this phase updates perm[0 : nA)
-      const int n_pool = self_first ? N - nA : nA, off = self_first ? nA : 0;
-      for (int c = gtid; c < N; c += nthreads) {
-        const int pos = q.shuffle ? (int)feistel_inv(fkey, (uint32_t)c) : c;
-        if ((pos < nA) != self_first) continue;
-        const int acc = small_chain_step<false, TARGET>(a, tv, sdata, c, n_pool, [&](int r) {
-          return q.shuffle ? (int)feistel_perm(fkey, (uint32_t)(off + r)) : off + r;
-        });
-        n_acc += acc; n_rej += 1 - acc;
-      }
-      grid.sync();
-    }
-    if (q.omega_sum)
-      for (int c = gtid; c < N; c += nthreads) q.omega_sum[c] += a.lnl[c];
-    if (a.algo == BPM_ALGO_DREAM) {
-      if ((int)blockIdx.x < q.cr_blocks)
-        cr_block_partials(a.cr_delta, a.cr_pick, 0, N, a.n_cr, (int)blockIdx.x, q.cr_blocks, q.cr_block);
-      grid.sync();
-      if (blockIdx.x == 0) cr_finish(q.cr_block, q.cr_blocks, a.n_cr, q.cr_part, 1, q.cr_dm, q.cr_cnt, q.p_cr);
-      grid.sync();                                                   // the next generation draws CR from the new p_cr
-    }
-  }
-  // accept / reject tallies: one atomic pair per warp
-  n_acc = __reduce_add_sync(0xFFFFFFFFu, n_acc);
-  n_rej = __reduce_add_sync(0xFFFFFFFFu, n_rej);
-  if ((threadIdx.x & 31) == 0) {
-    if (n_acc) atomicAdd(a.n_acc, (unsigned long long)n_acc);
-    if (n_rej) atomicAdd(a.n_rej, (unsigned long long)n_rej);
-  }
-}
-
 }  // namespace bpm
 #include "kernels_fused_v4.cuh"     // fused_gauss_v4_kernel: v3 with TMA-staged partner gathers (uses the helpers above)
 namespace bpm {
 
-// Will try_fused_phase run a lazy-protocol kernel (fused_gauss_v4_kernel / _v3_kernel) for this configuration?
-// The engine asks BEFORE building the phase arguments, because that kernel leaves the generation's new
-// history row / moment sample pending (PhaseArgs::lazy) and the others do not.
-inline bool fused_plan_is_v3(int target, int d, int ld, int r, int variant) {
-  if (!(target == BPM_TARGET_GAUSS && gauss_rows_supported(d, r) && (ld % 2) == 0)) return false;
+// The fused Gaussian half-phase kernel of a configuration, decided here and nowhere else: the engine plans the
+// lazy protocol from it before it builds the phase arguments (v3 and v4 leave the generation's new history row /
+// moment sample pending, PhaseArgs::lazy; ws writes them eagerly), and try_fused_phase launches it.  Shared memory
+// (227 KB per CTA) decides which kernels exist for a d: d = 108 fits v3 only, d = 112 none.
+//   1. none, unless the target is the Gaussian, gauss_rows_supported(d, r) holds and ld is even;
+//   2. ws, if fused_gauss_smem(d) fits and either mode is BPM_FUSED_GAUSS_WS or the v3 conditions below fail;
+//   3. if the v3 conditions hold (d % 4 == 0, ld == d, fused_v3_smem(d) fits): v4 when mode is not
+//      BPM_FUSED_GAUSS_V3 and fused_v4_fits(d, ld, r, npair) holds, otherwise v3;
+//   4. none otherwise (d = 112): the engine runs the split path.
+// npair: del_pairs for DREAM, 1 for DE-MC.  mode: bpm_set_fused's value (not BPM_FUSED_OFF).
+enum class GaussKernel { none, ws, v3, v4 };
+inline GaussKernel gauss_fused_kernel(int target, int d, int ld, int r, int npair, int mode) {
+  if (!(target == BPM_TARGET_GAUSS && gauss_rows_supported(d, r) && (ld % 2) == 0)) return GaussKernel::none;
   const bool v3_ok = (d % 4) == 0 && ld == d && fused_v3_smem(d) <= kMaxDynSmem;
-  const bool v12_ok = fused_gauss_smem(d) <= kMaxDynSmem;
-  if (!v3_ok) return false;
-  if (variant == 2 && v12_ok) return false;
-  if (variant == 3 && v12_ok) return false;
-  return true;
+  if (fused_gauss_smem(d) <= kMaxDynSmem && (mode == BPM_FUSED_GAUSS_WS || !v3_ok)) return GaussKernel::ws;
+  if (v3_ok)
+    return mode != BPM_FUSED_GAUSS_V3 && fused_v4_fits(d, ld, r, npair) ? GaussKernel::v4 : GaussKernel::v3;
+  return GaussKernel::none;
 }
 
+// One fused half-phase: the Gaussian kernel gk names (gauss_fused_kernel), or fused_small_kernel for the d <= 4
+// analytic targets.  *done = 0: nothing was launched, the caller runs the split path.
 template <bool REPLAY>
-inline int try_fused_phase(const TargetView& tv, const PhaseArgs& a, cudaStream_t s, int variant,
-                           int* done) {
+inline int try_fused_phase(const TargetView& tv, const PhaseArgs& a, cudaStream_t s, GaussKernel gk, int* done) {
   *done = 0;
-  if (tv.target == BPM_TARGET_GAUSS && gauss_rows_supported(a.d, tv.r) && (a.ld % 2) == 0) {
+  if (gk != GaussKernel::none) {
     GaussArgs g;
     g.mu = tv.mu; g.W = tv.W; g.Wf = tv.Wf; g.r = tv.r; g.c0 = tv.c0; g.log_of_pdf = tv.log_of_pdf;
-    const size_t sm = fused_gauss_smem(a.d);
     const int n_tiles = (a.nA + kTileRows - 1) / kTileRows;
-    cudaError_t e;
-    // shared memory decides which variants exist for this d (227 KB per CTA): d = 108 fits variant 3
-    // only, d = 112 none -- the caller then runs the split path
-    const bool v3_ok = (a.d % 4) == 0 && a.ld == a.d && fused_v3_smem(a.d) <= kMaxDynSmem;
-    const bool v12_ok = sm <= kMaxDynSmem;
-    if (!v3_ok && !v12_ok) return 0;
-    if (variant == 2 && !v12_ok) variant = 1;
-    if (variant == 2) {
-      int grid = (n_tiles + 1) / 2;
-      grid = grid > 148 ? 148 : (grid < 1 ? 1 : grid);
-      if (tv.mu_is_zero) {
-        e = cudaFuncSetAttribute(fused_gauss_kernel<REPLAY, false>,
-                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-        if (e != cudaSuccess) return 1;
-        fused_gauss_kernel<REPLAY, false><<<grid, 2 * kHalfThreads, sm, s>>>(a, g);
-      } else {
-        e = cudaFuncSetAttribute(fused_gauss_kernel<REPLAY, true>,
-                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-        if (e != cudaSuccess) return 1;
-        fused_gauss_kernel<REPLAY, true><<<grid, 2 * kHalfThreads, sm, s>>>(a, g);
-      }
-    } else if (v12_ok && (variant == 3 || !v3_ok)) {
-      const int grid = n_tiles > 148 ? 148 : (n_tiles < 1 ? 1 : n_tiles);
+    const int grid = n_tiles > 148 ? 148 : (n_tiles < 1 ? 1 : n_tiles);
+    if (gk == GaussKernel::ws) {
+      const size_t sm = fused_gauss_smem(a.d);
+      cudaError_t e;
       if (tv.mu_is_zero) {
         e = cudaFuncSetAttribute(fused_gauss_ws_kernel<REPLAY, false>,
                                  cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
@@ -1463,13 +1275,10 @@ inline int try_fused_phase(const TargetView& tv, const PhaseArgs& a, cudaStream_
         fused_gauss_ws_kernel<REPLAY, true><<<grid, kWsThreads, sm, s>>>(a, g);
       }
     } else {
-      if (!a.lazy) return 1;       // the engine must have planned the lazy protocol (fused_plan_is_v3)
-      const int grid = n_tiles > 148 ? 148 : (n_tiles < 1 ? 1 : n_tiles);
       const bool d3 = a.algo == BPM_ALGO_DREAM && a.del_pairs == 3;
-      const int npair = a.algo == BPM_ALGO_DREAM ? a.del_pairs : 1;
       int rc;
-      // default: TMA-staged gathers (v4) whenever its shared-memory layout fits; variant 5 = v3 (register gathers)
-      if (variant != 5 && fused_v4_fits(a.d, a.ld, tv.r, npair)) {
+      if (gk == GaussKernel::v4) {        // TMA-staged gathers
+        const int npair = a.algo == BPM_ALGO_DREAM ? a.del_pairs : 1;
         const size_t sm4 = v4_layout(a.d, tv.r, npair).total;
         const bool d1 = a.algo == BPM_ALGO_DEMC;
         if (tv.mu_is_zero)
@@ -1480,33 +1289,17 @@ inline int try_fused_phase(const TargetView& tv, const PhaseArgs& a, cudaStream_
           rc = d3 ? launch_fused_v4<REPLAY, true, 3>(a, g, grid, sm4, s)
              : d1 ? launch_fused_v4<REPLAY, true, 1>(a, g, grid, sm4, s)
                   : launch_fused_v4<REPLAY, true, 0>(a, g, grid, sm4, s);
-        if (rc) return 1;
-        if (cudaGetLastError() != cudaSuccess) return 1;
-        *done = 1;
-        return 0;
+      } else {                            // v3: register gathers
+        const size_t sm = fused_v3_smem(a.d);
+        if (tv.mu_is_zero)
+          rc = d3 ? launch_fused_v3<REPLAY, false, 3>(a, g, grid, sm, s)
+                  : launch_fused_v3<REPLAY, false, 0>(a, g, grid, sm, s);
+        else
+          rc = d3 ? launch_fused_v3<REPLAY, true, 3>(a, g, grid, sm, s)
+                  : launch_fused_v3<REPLAY, true, 0>(a, g, grid, sm, s);
       }
-      const size_t sm = fused_v3_smem(a.d);
-      if (tv.mu_is_zero)
-        rc = d3 ? launch_fused_v3<REPLAY, false, 3>(a, g, grid, sm, s)
-                : launch_fused_v3<REPLAY, false, 0>(a, g, grid, sm, s);
-      else
-        rc = d3 ? launch_fused_v3<REPLAY, true, 3>(a, g, grid, sm, s)
-                : launch_fused_v3<REPLAY, true, 0>(a, g, grid, sm, s);
       if (rc) return 1;
     }
-    if (cudaGetLastError() != cudaSuccess) return 1;
-    *done = 1;
-    return 0;
-  }
-  if (a.d <= 4 && a.fly && !REPLAY && (tv.target == BPM_TARGET_BANANA || tv.target == BPM_TARGET_BIMODAL ||
-                                       tv.target == BPM_TARGET_LINEFIT)) {
-    const int grid = (a.N + 127) / 128;
-    if (tv.target == BPM_TARGET_BANANA)
-      fused_small_fly_kernel<BPM_TARGET_BANANA><<<grid, 128, 0, s>>>(a, tv);
-    else if (tv.target == BPM_TARGET_BIMODAL)
-      fused_small_fly_kernel<BPM_TARGET_BIMODAL><<<grid, 128, 0, s>>>(a, tv);
-    else
-      fused_small_fly_kernel<BPM_TARGET_LINEFIT><<<grid, 128, sizeof(double) * 3 * tv.linefit_M, s>>>(a, tv);
     if (cudaGetLastError() != cudaSuccess) return 1;
     *done = 1;
     return 0;

@@ -97,28 +97,19 @@ __device__ __forceinline__ void block_excl_scan2(int xa, int xb, int& ea, int& e
   tota = wa[NT / 32 - 1];
   totb = wb[NT / 32 - 1];
 }
-// where chain c sits in the shuffled list: looked up (inv) or, in fly mode, the inverse Feistel image
-struct ListPos {
-  const int32_t* inv;
-  int32_t fly, shuffle;
-  FeistelKey fk;
-  __device__ __forceinline__ int operator()(int c) const {
-    if (!fly) return inv[c];
-    return shuffle ? (int)feistel_inv(fk, (uint32_t)c) : c;
-  }
-};
-__device__ __forceinline__ void compact_flags(const ListPos& pos, int nA, int hi, int c0, int& cA,
+// inv[c]: where chain c sits in the shuffled list
+__device__ __forceinline__ void compact_flags(const int32_t* inv, int nA, int hi, int c0, int& cA,
                                               int& cB, unsigned& mA, unsigned& mB) {
   cA = cB = 0; mA = mB = 0u;
 #pragma unroll
   for (int k = 0; k < kCompactPer; ++k) {
     const int c = c0 + k;
     if (c < hi) {
-      if (pos(c) < nA) { ++cA; mA |= 1u << k; } else { ++cB; mB |= 1u << k; }
+      if (inv[c] < nA) { ++cA; mA |= 1u << k; } else { ++cB; mB |= 1u << k; }
     }
   }
 }
-__global__ void __launch_bounds__(kCompactThreads) compact_count_kernel(const ListPos inv,
+__global__ void __launch_bounds__(kCompactThreads) compact_count_kernel(const int32_t* inv,
                                                                         int nA, int lo, int hi,
                                                                         int32_t* __restrict__ blk_cnt) {
   __shared__ int sa[kCompactThreads / 32], sb[kCompactThreads / 32];
@@ -151,7 +142,7 @@ __global__ void __launch_bounds__(1024) compact_scan_kernel(const int32_t* __res
     ra += blk_cnt[2 * b]; rb += blk_cnt[2 * b + 1];
   }
 }
-__global__ void __launch_bounds__(kCompactThreads) compact_write_kernel(const ListPos inv,
+__global__ void __launch_bounds__(kCompactThreads) compact_write_kernel(const int32_t* inv,
                                                                         int nA, int lo, int hi,
                                                                         const int32_t* __restrict__ blk_off,
                                                                         int32_t* __restrict__ loc_list) {

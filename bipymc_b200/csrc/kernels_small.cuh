@@ -1,6 +1,6 @@
-// d <= 4 targets, one thread per chain: the chain-step shared by every d <= 4 kernel and the per-phase
-// fused_small_kernel.  Device code only: besides the engine build, the run-time compiled likelihoods
-// (BPM_TARGET_JIT, engine.cu: bpm_jit_compile) compile this header with NVRTC, which has no host runtime.
+// d <= 4 targets, one thread per chain: the chain-step and the per-phase fused_small_kernel.  Device code
+// only: besides the engine build, the run-time compiled likelihoods (BPM_TARGET_JIT, engine.cu:
+// bpm_jit_compile) compile this header with NVRTC, which has no host runtime.
 //
 // BPM_JIT_LIKELIHOOD is defined only by that NVRTC translation unit, which places the user's
 //   __device__ double ln_like(const double* theta, const double* data)
@@ -34,12 +34,11 @@ constexpr int64_t kJitSmemDoubles = 4096;
 
 // ---- d <= 4 analytic targets: one thread per chain ------------------------------------
 // One chain-step of a d <= 4 target, start to finish (draws, proposal, likelihood, Metropolis decision,
-// state / moments / history update).  pool_id(r) maps a pool position to a global chain id: a lookup in the
-// materialised shuffle for the per-phase kernel, the Feistel permutation evaluated on the fly for the
-// persistent multi-generation kernel.  Returns 1 when the proposal was accepted.
-template <bool REPLAY, int TARGET, typename PoolFn>
+// state / moments / history update).  pool[r] is the global chain id of pool position r (the other half of the
+// materialised shuffle).  Returns 1 when the proposal was accepted.
+template <bool REPLAY, int TARGET>
 __device__ __forceinline__ int small_chain_step(const PhaseArgs& a, const TargetView& tv, const double* sdata,
-                                                int c, int n_pool, PoolFn pool_id) {
+                                                int c, int n_pool, const int32_t* pool) {
   const int d = a.d;
   const bool dream = a.algo == BPM_ALGO_DREAM;
   const int npair = dream ? a.del_pairs : 1;
@@ -49,8 +48,8 @@ __device__ __forceinline__ int small_chain_step(const PhaseArgs& a, const Target
   for (int p = 0; p < npair; ++p) {
     BPM_CHECK(D.r1[p] >= 0 && D.r1[p] < n_pool && D.r2[p] >= 0 && D.r2[p] < n_pool && D.r1[p] != D.r2[p],
               "pair draw", D.r1[p] * 100000LL + D.r2[p]);
-    BPM_CHECK(pool_id(D.r1[p]) >= 0 && pool_id(D.r1[p]) < a.N && pool_id(D.r2[p]) >= 0 && pool_id(D.r2[p]) < a.N,
-              "partner chain id", pool_id(D.r1[p]));
+    BPM_CHECK(pool[D.r1[p]] >= 0 && pool[D.r1[p]] < a.N && pool[D.r2[p]] >= 0 && pool[D.r2[p]] < a.N,
+              "partner chain id", pool[D.r1[p]]);
   }
   uint32_t mbits = 0xFu;
   double gamma;
@@ -103,8 +102,8 @@ __device__ __forceinline__ int small_chain_step(const PhaseArgs& a, const Target
 #pragma unroll
   for (int p = 0; p < BPM_MAX_PAIRS; ++p)
     if (p < npair) {
-      const double* pa = a.X + (size_t)pool_id(D.r1[p]) * a.ld;
-      const double* pb = a.X + (size_t)pool_id(D.r2[p]) * a.ld;
+      const double* pa = a.X + (size_t)pool[D.r1[p]] * a.ld;
+      const double* pb = a.X + (size_t)pool[D.r2[p]] * a.ld;
 #pragma unroll
       for (int q = 0; q < 4; ++q)
         if (q < d) {
@@ -207,7 +206,7 @@ __global__ void __launch_bounds__(128) fused_small_kernel(const PhaseArgs a, con
   const int c = valid ? L.self[gid] : 0;
   valid = valid && c >= a.chain_lo && c < a.chain_hi;
   int acc = 0;
-  if (valid) acc = small_chain_step<REPLAY, TARGET>(a, tv, sdata, c, L.n_pool, [&](int r) { return L.pool[r]; });
+  if (valid) acc = small_chain_step<REPLAY, TARGET>(a, tv, sdata, c, L.n_pool, L.pool);
   const unsigned am = __ballot_sync(0xFFFFFFFFu, valid && acc);
   const unsigned rm = __ballot_sync(0xFFFFFFFFu, valid && !acc);
   if ((threadIdx.x & 31) == 0) {

@@ -154,22 +154,6 @@ __host__ __device__ __forceinline__ uint32_t feistel_perm(const FeistelKey& f, u
   return v;
 }
 
-// position of element v in the permutation: feistel_inv(f, feistel_perm(f, i)) == i
-__host__ __device__ __forceinline__ uint32_t feistel_inv(const FeistelKey& f, uint32_t v) {
-  const uint32_t h = f.half_bits, mask = (1u << h) - 1u;
-  do {
-    uint32_t l = v >> h, r = v & mask;
-#pragma unroll
-    for (int t = 5; t >= 0; --t) {
-      uint32_t pr = l;                                   // forward: (l, r) -> (r, l ^ F(r ^ k))
-      l = r ^ (mix32(pr ^ f.k[t]) & mask);
-      r = pr;
-    }
-    v = (l << h) | r;
-  } while (v >= f.n);
-  return v;
-}
-
 __host__ __device__ __forceinline__ FeistelKey make_feistel(const RngCtx& r, uint32_t n) {
   FeistelKey f;
   Philox4 a = draw4(r, 0xFFFFFFFFu, RNG_GEN, 1), b = draw4(r, 0xFFFFFFFFu, RNG_GEN, 2);

@@ -87,15 +87,7 @@ struct PhaseArgs {
   unsigned long long* n_acc;
   unsigned long long* n_rej;
   int32_t* nan_flag;
-  // "fly" mode (EXPERIMENT, fused_small_fly_kernel / small_generations_kernel only): the shuffle of
-  // demc.py:84-86 is never materialised.  flip and the Feistel key are functions of (seed, generation) only, so
-  // the HOST evaluates them per generation and passes them by value; kernels turn list positions into chain
-  // ids (feistel_perm) and chain ids into positions (feistel_inv) on the fly.  Measured slower than a table
-  // lookup in the materialised shuffle (DESIGN.md section 9), hence opt-in.
-  int32_t fly;
-  int32_t flip_val;
-  int32_t fly_shuffle;     // 0: identity permutation (run_mcmc(shuffle=False))
-  FeistelKey fk;
+  int32_t flip_val;     // the flip flag's value (host_flip or the replayed coin), valid when flip_known
   // native RNG
   RngCtx rng;
   // replay buffers (REPLAY kernels only)

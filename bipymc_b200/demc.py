@@ -464,7 +464,8 @@ class DeMcMpi(object):
         h = C.c_void_p()
         _lib.check(self._libh.bpm_create(C.byref(cfg), C.byref(h)))
         self._handle = h
-        _lib.check(self._libh.bpm_set_fused(h, int(self._fused)))   # 0 split, 1 fused, 2 fused (two-halves variant)
+        # 0 split path, 1 fused (default), 3 / 5 the Gaussian's 12-producer / v3 kernel (include/bipymc_b200.h)
+        _lib.check(self._libh.bpm_set_fused(h, int(self._fused)))
         if self._ln_like_cuda is not None:
             self._target = self._ln_like_cuda
             self._jit_from_cache = self._target._attach(self._libh, h)     # True: the cubin came from the cache

@@ -185,10 +185,22 @@ int bpm_set_jit_sum_target(bpm_handle h, const char* source, const double* data,
 /* ln_like for n rows (device in, device out) with the current target. */
 int bpm_eval_lnl(bpm_handle h, const double* X, int32_t n, double* lnl, bpm_stream stream);
 
-/* DreamMpi._init_cr / CR state (dream.py:109-117): host arrays of n_cr doubles. */
-/* Switch the fused single-kernel fast paths off / on (testing: both must agree). */
-int bpm_set_fused(bpm_handle h, int32_t on);
+/* Which kernels run a half-phase.  Every mode computes the same chains (the Gaussian kernels
+ * that sum the quadratic form on the tensor pipe agree with the others' ln_like to rounding);
+ * BPM_FUSED_OFF and the two Gaussian modes exist so that the kernels can be compared with each other.
+ * Any other value is refused. */
+#define BPM_FUSED_OFF 0      /* split path: propose, likelihood and accept kernels                  */
+#define BPM_FUSED_DEFAULT 1  /* one fused kernel per half-phase where the target and shape have one:
+                                the Gaussian at 5 <= d <= 108 (v4, else v3, else the 12-producer
+                                kernel), banana / bimodal / line fit / BPM_TARGET_JIT at d <= 4;
+                                the split path elsewhere                                            */
+#define BPM_FUSED_GAUSS_WS 3 /* as DEFAULT, but the Gaussian runs the 12-producer kernel
+                                (fused_gauss_ws_kernel) wherever its shared memory fits             */
+#define BPM_FUSED_GAUSS_V3 5 /* as DEFAULT, but the Gaussian runs fused_gauss_v3_kernel (register
+                                gathers) where DEFAULT would run v4                                 */
+int bpm_set_fused(bpm_handle h, int32_t mode);
 
+/* DreamMpi._init_cr / CR state (dream.py:109-117): host arrays of n_cr doubles. */
 int bpm_set_cr_state(bpm_handle h, const double* p_cr, const double* delta_m,
                      const double* n_cr_updates);
 int bpm_get_cr_state(bpm_handle h, double* p_cr, double* delta_m, double* n_cr_updates);
@@ -294,8 +306,7 @@ int bpm_host_entry_restart(bpm_handle h);
  * bpm_set_sync).  X_host [n_local][ld] / lnl_host [n_local] are THIS rank's chains in pinned
  * (device-mapped) host memory; st is the rank's device state (st->X = its full replica).  One kernel reads
  * the shard over PCIe (zero-copy) and stores every piece into the rank's own and all peer replicas
- * (host->device copy and the reference's Allgather, demc.py:93, fused; BIPYMC_B200_SHARD_DMA=1 selects the
- * copy-engine form: chunked host copies, each chunk forwarded by peer copies), a peer barrier follows,
+ * (host->device copy and the reference's Allgather, demc.py:93, fused), a peer barrier follows,
  * n_gen generations run with the host array registered as one more replica -- so accepted rows are
  * written back by the phase kernels themselves -- and the cached likelihoods come back with one copy.
  * Collective: every rank calls it with the same k_gen0 / n_gen.  Synchronous. */

@@ -26,6 +26,15 @@ def test_reference_assertions_and_messages():
         c.chain = np.zeros((4, 2))
 
 
+@pytest.mark.parametrize("fused", [2, 6])
+def test_unknown_fused_mode_is_refused(fused):
+    """bpm_set_fused accepts 0, 1, 3 and 5 only (include/bipymc_b200.h: BPM_FUSED_*); any other value raises
+    instead of silently running the default kernels."""
+    from bipymc_b200 import DreamMpi, targets, _lib
+    with pytest.raises(_lib.BpmError, match="bpm_set_fused"):
+        DreamMpi(targets.Banana_2D().ln_like, [0.0, 0.0], n_chains=8, seed=1, fused=fused)
+
+
 def test_nan_alpha_raises_numpy_value_error():
     """lnL(cur) = lnL(prop) = -inf gives alpha = NaN; numpy's choice raises
     ValueError("probabilities contain NaN") at samplers.py:336 -- so does the device path."""

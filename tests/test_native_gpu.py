@@ -91,7 +91,7 @@ def test_native_demc_bimodal_matches_oracle_replay(fused):
     _native_vs_oracle(s, otargets.BimodeGauss2D().ln_like, gens=12, run_kwargs=dict(epsilon=1e-6))
 
 
-@pytest.mark.parametrize("fused", [1, 0, 2, 5], ids=["fused", "split", "fused-halves", "fused-v3"])
+@pytest.mark.parametrize("fused", [1, 0, 3, 5], ids=["fused", "split", "fused-ws12", "fused-v3"])
 @pytest.mark.parametrize("dim,n", [(7, 9), (100, 40), (33, 17), (100, 200)])
 def test_native_dream_gauss_matches_oracle_replay(dim, n, fused):
     from bipymc_b200 import DreamMpi, targets
@@ -275,13 +275,13 @@ def test_full_size_properties_1e5_chains_100d():
     tgt = targets.Gauss_100D()
     N, d, G = 100000, 100, 6
     runs = []
-    for fused in (1, 0, 2, 3, 5):     # 1 = TMA-staged gathers (v4, default), 5 = register gathers (v3)
+    for fused in (1, 0, 3, 5):     # 1 = TMA-staged gathers (v4, default), 3 = 12 producers, 5 = register gathers (v3)
         np.random.seed(0)
         s = DreamMpi(tgt.ln_like, np.zeros(d), n_chains=N, seed=77, burnin_gen=1000, n_cr_gen=2,
                      fused=fused, varepsilon=1.0)
         s.run_mcmc(N * (G + 1))
         runs.append(s)
-    a, b, c2, c3, c5 = runs
+    a, b, c3, c5 = runs
     ha, hb = a._hist.tensor(), b._hist.tensor()
     assert ha.shape == (G + 1, N, d)
     # v3 and v4 differ only in HOW the partner rows reach the proposal stage: identical bits everywhere
@@ -292,10 +292,10 @@ def test_full_size_properties_1e5_chains_100d():
     # default variant sums the quadratic form in DMMA fragment order, so its cached
     # likelihoods agree with the scalar variants to rounding, theirs among themselves exactly
     assert torch.equal(ha, hb), "fused and split paths must produce the same chains"
-    assert torch.equal(hb, c2._hist.tensor()) and torch.equal(hb, c3._hist.tensor())
-    assert torch.equal(b._lnl, c2._lnl) and torch.equal(b._lnl, c3._lnl)
+    assert torch.equal(hb, c3._hist.tensor())
+    assert torch.equal(b._lnl, c3._lnl)
     assert torch.allclose(a._lnl, b._lnl, rtol=1e-13, atol=0.0)
-    del c2, c3
+    del c3
     np.testing.assert_allclose(a.p_cr, b.p_cr, rtol=1e-12)
     # history row G == live population; every chain moved at most once per generation
     assert torch.equal(ha[G], a._X)

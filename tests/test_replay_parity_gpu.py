@@ -139,7 +139,7 @@ def replay_and_check(name, fused):
     check_against_reference(name, s, sink, traces, osampler)
 
 
-@pytest.mark.parametrize("fused", [1, 0, 2, 3, 5], ids=["fused", "split", "fused-halves", "fused-ws12", "fused-v3"])
+@pytest.mark.parametrize("fused", [1, 0, 3, 5], ids=["fused", "split", "fused-ws12", "fused-v3"])
 @pytest.mark.parametrize("name", sorted(CASES))
 def test_replay_device_target(name, fused):
     replay_and_check(name, fused)

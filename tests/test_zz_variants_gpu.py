@@ -3,8 +3,6 @@ default fused Gaussian kernel that the golden / headline configurations do not r
   * the run-time-general proposal stage (DREAM with del_pairs != 3, DE-MC) at d = 100, several tiles;
   * a target with a non-zero mean (the CENTER instantiation of the tile product).
 Runs last (file name) so that a regression here does not mask the main parity suite under `pytest -x`."""
-import os
-
 import numpy as np
 import pytest
 from scipy.stats import multivariate_normal
@@ -49,7 +47,7 @@ def test_native_dream_gauss_with_nonzero_mean(dim):
 
 
 # ---- RNG-replay parity against the second batch of golden vectors (oracle/cases.py: EXTRA_CASES) --------
-@pytest.mark.parametrize("fused", [1, 0, 2, 3, 5], ids=["fused", "split", "fused-halves", "fused-ws12", "fused-v3"])
+@pytest.mark.parametrize("fused", [1, 0, 3, 5], ids=["fused", "split", "fused-ws12", "fused-v3"])
 @pytest.mark.parametrize("name", sorted(__import__("oracle.cases", fromlist=["EXTRA_CASES"]).EXTRA_CASES))
 def test_replay_extra_golden_cases(name, fused):
     """Includes gauss100_dream_tiles: 136 chains at d = 100, i.e. one full 64-chain tile plus a partial tile per
@@ -58,16 +56,18 @@ def test_replay_extra_golden_cases(name, fused):
     replay_and_check(name, fused)
 
 
-# ---- d <= 4: the shuffle-free ("fly") fused kernel and the persistent cooperative kernel against the split path ---
-@pytest.mark.parametrize("fused", [1, 6, "fly"], ids=["default", "persistent", "fly"])
+# ---- d <= 4: the fused one-thread-per-chain kernel against the split path ----------------------------------------
 @pytest.mark.parametrize("target,n_chains,algo", [("banana", 1000, "dream"), ("dblgauss", 4099, "dream"),
-                                                   ("linefit", 2500, "dream"), ("banana", 777, "demc")])
-def test_small_d_shuffle_free_kernels_equal_split_path(target, n_chains, algo, fused):
-    """fused=1 (default): two launches per generation whose threads walk the chains in order and evaluate the
-    Feistel shuffle on the fly (no split / list-packing kernels); fused=6: every generation of a run_mcmc call in
-    ONE cooperative launch.  fused=0 launches split / propose / likelihood / accept / CR reduction per generation
-    over the materialised shuffle.  Same seed: identical histories, cached likelihoods, counters, running moments
-    and -- the CR block partials are summed in the same order -- bit-identical p_cr."""
+                                                   ("linefit", 2500, "dream"), ("banana", 777, "demc"),
+                                                   ("linefit", 33, "dream"), ("banana", 310000, "dream"),
+                                                   ("dblgauss", 2049, "demc"), ("linefit", 1500, "demc")])
+def test_small_d_fused_kernel_equals_split_path(target, n_chains, algo):
+    """fused=1 (default): one fused_small_kernel launch per half-phase over the chain-ordered packed lists, after
+    the split and list-packing kernels.  fused=0 launches split / propose / likelihood / accept / CR reduction per
+    generation.  Same seed: identical histories, cached likelihoods, counters, running moments and -- the CR block
+    partials are summed in the same order -- bit-identical p_cr.  The populations cover a partly filled single
+    warp (33), one chain past a list-packing block (2049), the CR reduction at its cap of 148 blocks (310000) and
+    DE-MC on every d <= 4 target."""
     import ctypes as C
     import torch
     from bipymc_b200 import DreamMpi, DeMcMpi, targets, _lib
@@ -75,31 +75,21 @@ def test_small_d_shuffle_free_kernels_equal_split_path(target, n_chains, algo, f
     th0 = [-0.8, 4.5, 0.2] if target == "linefit" else [0.0, 0.0]
     G = 37
     runs = []
-    if fused == "fly":
-        # the shuffle-free mode is read from the environment once per process (BIPYMC_B200_FLY=1): it is covered
-        # by the suite's second pass (tools/gpu_job: BIPYMC_B200_FLY=1 pytest -k "native or variants or replay")
-        if os.environ.get("BIPYMC_B200_FLY", "") != "1":
-            pytest.skip("run with BIPYMC_B200_FLY=1")
-        fused = 1
-    fly = os.environ.get("BIPYMC_B200_FLY", "") == "1"
-    for f in (fused, 0):
+    eps = 1e-2 if target == "linefit" else 0.3
+    for f in (1, 0):
         np.random.seed(21)
         if algo == "dream":
-            s = DreamMpi(tgt.ln_like, th0, n_chains=n_chains, seed=9, varepsilon=1e-2 if target == "linefit" else 0.3,
-                         n_cr_gen=3, burnin_gen=30, fused=f)
+            s = DreamMpi(tgt.ln_like, th0, n_chains=n_chains, seed=9, varepsilon=eps, n_cr_gen=3, burnin_gen=30,
+                         fused=f)
         else:
-            s = DeMcMpi(tgt.ln_like, th0, n_chains=n_chains, seed=9, varepsilon=0.3, fused=f)
+            s = DeMcMpi(tgt.ln_like, th0, n_chains=n_chains, seed=9, varepsilon=eps, fused=f)
         _lib.check(s._libh.bpm_profile(s._handle, 1))
         s.run_mcmc(n_chains * (G + 1), flip=0.3)
         ms, n = (C.c_double * 8)(), (C.c_int64 * 8)()
         _lib.check(s._libh.bpm_profile_read(s._handle, ms, n))
         runs.append((s, [int(v) for v in n]))
     (a, ka), (b, kb) = runs
-    if fused == 6:
-        assert ka[4] == 1 and ka[1] == 0 and ka[0] == 0, ka          # one launch for the whole run
-    else:
-        assert ka[4] == 2 * G and ka[1] == 0, ka
-        assert ka[0] == (0 if fly else G), ka                        # fly mode: no split / packing launches at all
+    assert ka[4] == 2 * G and ka[1] == 0 and ka[0] == G, ka
     assert kb[4] == 0 and kb[1] == 2 * G and kb[0] == G, kb
     assert torch.equal(a._hist.tensor(), b._hist.tensor())
     assert torch.equal(a._lnl, b._lnl) and torch.equal(a._X, b._X)

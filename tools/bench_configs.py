@@ -364,9 +364,9 @@ def c5full():
 def c4multi():
     """BASELINE configs[3] (launch under torchrun, 1 / 2 / 4 ranks): DREAM on the examples/ex_para_fit.py line
     fit (3 parameters, 50 data points, likelihood evaluated in-kernel), 10^5 chains in TOTAL sharded over the
-    GPUs (the config as stated: strong scaling) and 10^5 chains PER GPU (weak scaling).  One rank: every
-    generation of the call runs inside one persistent cooperative kernel; several ranks: per-phase kernels with
-    accepted rows stored into the peer replicas and the peer-memory barrier / CR exchange between them."""
+    GPUs (the config as stated: strong scaling) and 10^5 chains PER GPU (weak scaling).  Per-phase fused d <= 4
+    kernels; several ranks store accepted rows into the peer replicas and put the peer-memory barrier / CR exchange
+    between the half-phases."""
     import torch.distributed as dist
     from bipymc_b200 import DreamMpi, targets
     rank, local = int(os.environ.get("RANK", 0)), int(os.environ.get("LOCAL_RANK", 0))
@@ -397,7 +397,7 @@ def c4multi():
                               "n_chains": N, "chain_steps_per_s": N * gens / (float(ms.item()) * 1e-3),
                               "us_per_generation": 1e3 * float(ms.item()) / gens,
                               "acceptance_fraction": s.acceptance_fraction,
-                              "path": "persistent cooperative kernel" if world == 1 else
+                              "path": "per-phase kernels" if world == 1 else
                                       "per-phase kernels + peer-memory barrier (%s)" % ("on" if s._sync_on else "off")}),
                   flush=True)
         s.close()

@@ -39,6 +39,6 @@ print("%-64s %7s " % ("kernel", "instr") + " ".join("%6s" % k for k in keys))
 tot = collections.Counter()
 for name, c in per.items():
     tot.update(c)
-    if any(c[k] for k in keys[:8]) or "fused" in name or "small_gen" in name:
+    if any(c[k] for k in keys[:8]) or "fused" in name:
         print("%-64s %7d " % (name[-64:], c["_total"]) + " ".join("%6d" % c[k] for k in keys))
 print("%-64s %7d " % ("ALL KERNELS (%d)" % len(per), tot["_total"]) + " ".join("%6d" % tot[k] for k in keys))
