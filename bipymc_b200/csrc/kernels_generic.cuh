@@ -161,22 +161,35 @@ __global__ void __launch_bounds__(kCompactThreads) compact_write_kernel(const in
 }
 
 // ---- proposal ---------------------------------------------------------------------
-template <bool REPLAY, int LPC>
+// PROB (multi-problem handles, pb used): the chain of slot gid comes from problem_slot, and its draws are
+// addressed by the problem's key, the chain's index within the problem and the problem's p_cr row.
+__device__ __forceinline__ PhaseLists slot_lists(const ProblemSlot& ps) {
+  PhaseLists L;
+  L.self = nullptr; L.n_self = 0; L.skip_self = 0;
+  L.pool = ps.pool; L.n_pool = ps.n_pool;
+  return L;
+}
+template <bool REPLAY, int LPC, bool PROB = false>
 // (LPC = 32: two 256-thread blocks per SM, i.e. at most 128 registers -- without the bound the block-wise pass 2
 // takes 174 and one block per SM)
-__global__ void __launch_bounds__(kThreads, LPC == 32 ? 2 : 1) propose_kernel(const PhaseArgs a) {
+__global__ void __launch_bounds__(kThreads, LPC == 32 ? 2 : 1) propose_kernel(const PhaseArgs a, const ProblemArgs prob) {
   const int gid = (blockIdx.x * kThreads + threadIdx.x) / LPC;
   const int sub = threadIdx.x % LPC;
-  const PhaseLists L = phase_lists(a);
-  bool valid = gid < L.n_self;
-  const int c = valid ? L.self[gid] : 0;
-  valid = valid && c >= a.chain_lo && c < a.chain_hi;
+  ProblemSlot ps;
+  if constexpr (PROB) ps = problem_slot(a, prob, gid);
+  const PhaseLists L = PROB ? slot_lists(ps) : phase_lists(a);
+  bool valid = PROB ? ps.valid : gid < L.n_self;
+  const int c = PROB ? ps.c : (valid ? L.self[gid] : 0);
+  if constexpr (!PROB) valid = valid && c >= a.chain_lo && c < a.chain_hi;
   const bool dream = a.algo == BPM_ALGO_DREAM;
   const int nblk = (a.d + 3) >> 2;
 
   ChainDraws D;
   D.cr_idx = 0; D.fallback = -1; D.gamma_u = 0.0;
-  if (valid) chain_scalar_draws<REPLAY>(a, c, L.n_pool, D);
+  if (valid) {
+    if constexpr (PROB) chain_scalar_draws<REPLAY>(a, ps.rng, ps.p_cr, c, ps.j, L.n_pool, D);
+    else chain_scalar_draws<REPLAY>(a, c, L.n_pool, D);
+  }
 
   // pass 1 (DREAM): crossover mask of this lane's dimensions, d' (dream.py:51-58)
   uint32_t mbits = 0xFFFFFFFFu;
@@ -196,12 +209,14 @@ __global__ void __launch_bounds__(kThreads, LPC == 32 ? 2 : 1) propose_kernel(co
         if (b < nblk) {
           double z[4];
           if constexpr (kKeepDraws) {          // z4's native branch, keeping the call's words for zen_en4
-            const Philox4 q = draw4(a.rng, (uint32_t)c, RNG_ZEN, (uint32_t)b);
+            const Philox4 q = PROB ? draw4(ps.rng, (uint32_t)ps.j, RNG_ZEN, (uint32_t)b)
+                                   : draw4(a.rng, (uint32_t)c, RNG_ZEN, (uint32_t)b);
             qs[t] = q;
             z[0] = ((double)(q.x & 0xFFFu) + 0.5) * (1.0 / 4096.0); z[1] = ((double)(q.y & 0xFFFu) + 0.5) * (1.0 / 4096.0);
             z[2] = ((double)(q.z & 0xFFFu) + 0.5) * (1.0 / 4096.0); z[3] = ((double)(q.w & 0xFFFu) + 0.5) * (1.0 / 4096.0);
           } else {
-            z4<REPLAY>(a, c, b, z);
+            if constexpr (PROB) z4<REPLAY>(a, ps.rng, c, ps.j, b, z);
+            else z4<REPLAY>(a, c, b, z);
           }
 #pragma unroll
           for (int q = 0; q < 4; ++q)
@@ -282,7 +297,8 @@ __global__ void __launch_bounds__(kThreads, LPC == 32 ? 2 : 1) propose_kernel(co
           n[0] = n[1] = n[2] = n[3] = 0.0;
           if (a.u_eps > 0.0 || a.eps > 0.0) zen_en4(a, qs[kKeepDraws ? t : 0], e, n);
         } else {
-          en4<REPLAY>(a, c, b, e, n);
+          if constexpr (PROB) en4<REPLAY>(a, ps.rng, c, ps.j, b, e, n);
+          else en4<REPLAY>(a, c, b, e, n);
         }
         const double cur[4] = {c0.x, c0.y, c1.x, c1.y};
         const double m2v[4] = {w0.x, w0.y, w1.x, w1.y};
@@ -331,7 +347,8 @@ __global__ void __launch_bounds__(kThreads, LPC == 32 ? 2 : 1) propose_kernel(co
       const int b = sub + t * LPC;
       if (b < nblk) {
         double e[4], n[4];
-        en4<REPLAY>(a, c, b, e, n);
+        if constexpr (PROB) en4<REPLAY>(a, ps.rng, c, ps.j, b, e, n);
+        else en4<REPLAY>(a, c, b, e, n);
 #pragma unroll
         for (int q = 0; q < 4; ++q) {
           const int i = 4 * b + q;
@@ -366,19 +383,23 @@ __global__ void __launch_bounds__(kThreads, LPC == 32 ? 2 : 1) propose_kernel(co
 }
 
 // ---- accept / reject + state, moments, history ---------------------------------
-template <bool REPLAY, int LPC>
-__global__ void __launch_bounds__(kThreads) accept_kernel(const PhaseArgs a) {
+template <bool REPLAY, int LPC, bool PROB = false>
+__global__ void __launch_bounds__(kThreads) accept_kernel(const PhaseArgs a, const ProblemArgs prob) {
   const int gid = (blockIdx.x * kThreads + threadIdx.x) / LPC;
   const int sub = threadIdx.x % LPC;
-  const PhaseLists L = phase_lists(a);
-  bool valid = gid < L.n_self;
-  const int c = valid ? L.self[gid] : 0;
-  valid = valid && c >= a.chain_lo && c < a.chain_hi;
+  ProblemSlot ps;
+  if constexpr (PROB) ps = problem_slot(a, prob, gid);
+  const PhaseLists L = PROB ? slot_lists(ps) : phase_lists(a);
+  bool valid = PROB ? ps.valid : gid < L.n_self;
+  const int c = PROB ? ps.c : (valid ? L.self[gid] : 0);
+  if constexpr (!PROB) valid = valid && c >= a.chain_lo && c < a.chain_hi;
   int acc = 0;
   double lp = 0.0;
   if (valid) {
     lp = a.lnl_prop[gid];
-    const double u = accept_uniform<REPLAY>(a, c);
+    double u;
+    if constexpr (PROB) u = accept_uniform<REPLAY>(a, ps.rng, c, ps.j);
+    else u = accept_uniform<REPLAY>(a, c);
     acc = metropolis(a.lnl[c], lp, u);
     if (acc < 0) {
       *a.nan_flag = 1;
@@ -450,6 +471,10 @@ __global__ void __launch_bounds__(kThreads) accept_kernel(const PhaseArgs a) {
       if (a.tr.accept) a.tr.accept[c] = acc;
       if (a.tr.lnl_prop) a.tr.lnl_prop[c] = lp;
     }
+  }
+  if constexpr (PROB) {
+    problem_count(prob, ps.g, valid && sub == 0, acc);
+    return;
   }
   const unsigned am = __ballot_sync(0xFFFFFFFFu, valid && sub == 0 && acc);
   const unsigned rm = __ballot_sync(0xFFFFFFFFu, valid && sub == 0 && !acc);
@@ -556,129 +581,9 @@ __global__ void __launch_bounds__(256) lnl_gauss_tiled_kernel(const double* __re
 }
 
 // ---- CR adaptation: deterministic reduction + p_cr update (dream.py:119-140) -----
-// Stage 1: block b sums the chains of its contiguous segment (fixed order inside the
-// block); stage 2: one warp adds the block partials in block order.
-constexpr int kCrBlocks = 148;
-// Second half of the reduction, run by whichever block finishes last (ticket counter): adds
-// the block partials in block order -- so the sums do not depend on scheduling -- and, on an
-// unsharded handle, applies the p_cr update (dream.py:132-140).  One launch per generation
-// instead of three.
-__device__ __forceinline__ void cr_apply(const double* __restrict__ part, int n_cr, double* __restrict__ dm,
-                                         double* __restrict__ cnt, double* __restrict__ p_cr) {
-  double got = 0.0;
-  for (int m = 0; m < n_cr; ++m) {
-    dm[m] += part[m];
-    cnt[m] += part[n_cr + m];
-    got += part[n_cr + m];
-  }
-  if (got == 0.0) return;  // no chain ran _update_cr_ratios this generation
-  int nz = 0;
-  for (int m = 0; m < n_cr; ++m) nz += cnt[m] > 0.0;
-  if (nz == n_cr)
-    for (int m = 0; m < n_cr; ++m) p_cr[m] = dm[m] / cnt[m];
-  double tot = 0.0;
-  for (int m = 0; m < n_cr; ++m) tot += p_cr[m];
-  for (int m = 0; m < n_cr; ++m) p_cr[m] /= tot;
-}
-
-// first half: block `bid` of `nb` sums the chains of its contiguous segment (256 threads)
-__device__ __forceinline__ void cr_block_partials(const double* __restrict__ cr_delta,
-                                                  const int32_t* __restrict__ cr_pick, int lo, int hi, int n_cr,
-                                                  int bid, int nb, double* __restrict__ block_part) {
-  __shared__ double sm[8][2 * 4];
-  const int n = hi - lo;
-  const int per = (n + nb - 1) / nb;
-  const int c0 = lo + bid * per;
-  const int c1 = min(hi, c0 + per);
-  if (n_cr <= 4) {
-    // one pass over the block's chains, the (at most four) CR classes in registers
-    double s[4] = {0.0, 0.0, 0.0, 0.0}, k[4] = {0.0, 0.0, 0.0, 0.0};
-    // eight independent (pick, statistic) loads in flight per thread, folded in chain order
-    for (int base = c0; base < c1; base += 8 * 256) {
-      int mm[8];
-      double vv[8];
-#pragma unroll
-      for (int u = 0; u < 8; ++u) {
-        const int c = base + u * 256 + (int)threadIdx.x;
-        const bool ok = c < c1;
-        mm[u] = ok ? cr_pick[c] : -1;
-        vv[u] = ok ? cr_delta[c] : 0.0;
-      }
-#pragma unroll
-      for (int u = 0; u < 8; ++u)
-#pragma unroll
-        for (int q = 0; q < 4; ++q)
-          if (mm[u] == q) { s[q] += vv[u]; k[q] += 1.0; }
-    }
-#pragma unroll
-    for (int q = 0; q < 4; ++q) {
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) {
-        s[q] += __shfl_xor_sync(0xFFFFFFFFu, s[q], o);
-        k[q] += __shfl_xor_sync(0xFFFFFFFFu, k[q], o);
-      }
-    }
-    if ((threadIdx.x & 31) == 0) {
-#pragma unroll
-      for (int q = 0; q < 4; ++q) { sm[threadIdx.x >> 5][q] = s[q]; sm[threadIdx.x >> 5][4 + q] = k[q]; }
-    }
-    __syncthreads();
-    if (threadIdx.x < 8) {
-      const int q = threadIdx.x & 3, pass = threadIdx.x >> 2;
-      double w = 0.0;
-      for (int i = 0; i < 8; ++i) w += sm[i][threadIdx.x];
-      if (q < n_cr) block_part[(size_t)bid * 2 * BPM_MAX_CR + pass * n_cr + q] = w;
-    }
-    __syncthreads();
-  } else {
-    for (int m = 0; m < n_cr; ++m) {
-      double s = 0.0, k = 0.0;
-      for (int c = c0 + threadIdx.x; c < c1; c += blockDim.x)
-        if (cr_pick[c] == m) { s += cr_delta[c]; k += 1.0; }
-      for (int pass = 0; pass < 2; ++pass) {
-        double v = pass == 0 ? s : k;
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xFFFFFFFFu, v, o);
-        if ((threadIdx.x & 31) == 0) sm[threadIdx.x >> 5][0] = v;
-        __syncthreads();
-        if (threadIdx.x == 0) {
-          double w = 0.0;
-          for (int i = 0; i < 8; ++i) w += sm[i][0];
-          block_part[(size_t)bid * 2 * BPM_MAX_CR + pass * n_cr + m] = w;
-        }
-        __syncthreads();
-      }
-    }
-  }
-}
-// second half, one block: all block partials land in shared memory with independent loads, then each of
-// the 2 n_cr outputs is added up in block order
-__device__ __forceinline__ void cr_finish(const double* __restrict__ block_part, int nb, int n_cr,
-                                          double* __restrict__ part, int apply, double* __restrict__ dm,
-                                          double* __restrict__ cnt, double* __restrict__ p_cr) {
-  __shared__ double stage[kCrBlocks * 2 * BPM_MAX_CR / 4];    // nb <= 148 blocks x 2 n_cr <= 8 values (n_cr <= 4) or fewer blocks
-  const int nv = 2 * n_cr;
-  const int fit = (int)(sizeof(stage) / sizeof(double)) / nv;      // blocks that fit in the stage
-  double w = 0.0;
-  for (int b0 = 0; b0 < nb; b0 += fit) {
-    const int nb_here = min(nb - b0, fit);
-    for (int idx = threadIdx.x; idx < nb_here * nv; idx += blockDim.x) {
-      const int b = idx / nv, i = idx - b * nv;
-      stage[idx] = __ldcg(&block_part[(size_t)(b0 + b) * 2 * BPM_MAX_CR + i]);
-    }
-    __syncthreads();
-    if ((int)threadIdx.x < nv)
-      for (int b = 0; b < nb_here; ++b) w += stage[b * nv + threadIdx.x];
-    __syncthreads();
-  }
-  __shared__ double part_s[2 * BPM_MAX_CR];        // cr_apply reads the sums from here, not back from global memory
-  if ((int)threadIdx.x < nv) {
-    part[threadIdx.x] = w;
-    part_s[threadIdx.x] = w;
-  }
-  __syncthreads();
-  if (threadIdx.x == 0 && apply) cr_apply(part_s, n_cr, dm, cnt, p_cr);
-}
+}  // namespace bpm
+#include "cr_reduce.cuh"   // the reduction helpers, shared with the multi-problem CR kernel
+namespace bpm {
 
 __global__ void __launch_bounds__(256) cr_update_kernel(const double* __restrict__ cr_delta,
                                                         const int32_t* __restrict__ cr_pick, int lo, int hi,

@@ -35,15 +35,18 @@ constexpr int64_t kJitSmemDoubles = 4096;
 // ---- d <= 4 analytic targets: one thread per chain ------------------------------------
 // One chain-step of a d <= 4 target, start to finish (draws, proposal, likelihood, Metropolis decision,
 // state / moments / history update).  pool[r] is the global chain id of pool position r (the other half of the
-// materialised shuffle).  Returns 1 when the proposal was accepted.
-template <bool REPLAY, int TARGET>
+// materialised shuffle).  Returns 1 when the proposal was accepted.  rng, j and p_cr address the chain's
+// draws (step.cuh: chain_scalar_draws).  PROB (multi-problem handles, BPM_TARGET_JIT only): sdata is the
+// problem's data row in global memory.
+template <bool REPLAY, int TARGET, bool PROB = false>
 __device__ __forceinline__ int small_chain_step(const PhaseArgs& a, const TargetView& tv, const double* sdata,
-                                                int c, int n_pool, const int32_t* pool) {
+                                                int c, int n_pool, const int32_t* pool, const RngCtx& rng, int j,
+                                                const double* p_cr) {
   const int d = a.d;
   const bool dream = a.algo == BPM_ALGO_DREAM;
   const int npair = dream ? a.del_pairs : 1;
   ChainDraws D;
-  chain_scalar_draws<REPLAY>(a, c, n_pool, D);
+  chain_scalar_draws<REPLAY>(a, rng, p_cr, c, j, n_pool, D);
   BPM_CHECK(c >= a.chain_lo && c < a.chain_hi, "own chain id", c);
   for (int p = 0; p < npair; ++p) {
     BPM_CHECK(D.r1[p] >= 0 && D.r1[p] < n_pool && D.r2[p] >= 0 && D.r2[p] < n_pool && D.r1[p] != D.r2[p],
@@ -57,7 +60,7 @@ __device__ __forceinline__ int small_chain_step(const PhaseArgs& a, const Target
     mbits = 0u;
     const double cr = __ddiv_rn((double)(D.cr_idx + 1), (double)a.n_cr);
     double z[4];
-    z4<REPLAY>(a, c, 0, z);
+    z4<REPLAY>(a, rng, c, j, 0, z);
 #pragma unroll
     for (int q = 0; q < 4; ++q)
       if (q < d && z[q] <= cr) mbits |= 1u << q;
@@ -112,7 +115,7 @@ __device__ __forceinline__ int small_chain_step(const PhaseArgs& a, const Target
         }
     }
   double e[4], nn[4];
-  en4<REPLAY>(a, c, 0, e, nn);
+  en4<REPLAY>(a, rng, c, j, 0, e, nn);
   double delta = 0.0;
 #pragma unroll
   for (int q = 0; q < 4; ++q)
@@ -149,13 +152,14 @@ __device__ __forceinline__ int small_chain_step(const PhaseArgs& a, const Target
   if (TARGET == BPM_TARGET_BANANA) lp = banana_lnl(tv.banana, pr[0], pr[1]);
   else if (TARGET == BPM_TARGET_BIMODAL) lp = bimodal_lnl(tv.bimodal, pr[0], pr[1]);
 #ifdef BPM_JIT_LIKELIHOOD
+  else if constexpr (TARGET == BPM_TARGET_JIT && PROB) lp = ln_like(pr, sdata);
   else if constexpr (TARGET == BPM_TARGET_JIT) lp = ln_like(pr, tv.n_data <= kJitSmemDoubles ? sdata : tv.data);
 #endif
   else lp = linefit_lnl(sdata, sdata + tv.linefit_M, sdata + 2 * tv.linefit_M, tv.linefit_M, pr[0],
                         pr[1], pr[2]);
   int acc;
-  if constexpr (kPreload) acc = metropolis(lnl_c, lp, accept_uniform<REPLAY>(a, c));
-  else acc = metropolis(a.lnl[c], lp, accept_uniform<REPLAY>(a, c));
+  if constexpr (kPreload) acc = metropolis(lnl_c, lp, accept_uniform<REPLAY>(a, rng, c, j));
+  else acc = metropolis(a.lnl[c], lp, accept_uniform<REPLAY>(a, rng, c, j));
   if (acc < 0) {
     *a.nan_flag = 1;
     acc = 0;
@@ -206,7 +210,7 @@ __global__ void __launch_bounds__(128) fused_small_kernel(const PhaseArgs a, con
   const int c = valid ? L.self[gid] : 0;
   valid = valid && c >= a.chain_lo && c < a.chain_hi;
   int acc = 0;
-  if (valid) acc = small_chain_step<REPLAY, TARGET>(a, tv, sdata, c, L.n_pool, L.pool);
+  if (valid) acc = small_chain_step<REPLAY, TARGET>(a, tv, sdata, c, L.n_pool, L.pool, a.rng, c, a.p_cr);
   const unsigned am = __ballot_sync(0xFFFFFFFFu, valid && acc);
   const unsigned rm = __ballot_sync(0xFFFFFFFFu, valid && !acc);
   if ((threadIdx.x & 31) == 0) {
@@ -215,7 +219,30 @@ __global__ void __launch_bounds__(128) fused_small_kernel(const PhaseArgs a, con
   }
 }
 
-#ifdef BPM_JIT_LIKELIHOOD
+#ifdef BPM_JIT_PROBLEMS
+}  // namespace bpm
+#include "cr_reduce.cuh"     // cr_update_problems_kernel
+namespace bpm {
+// Multi-problem handles (step.cuh: ProblemArgs), d <= 4: thread t steps slot t % nA of problem t / nA with
+// the problem's key, pool, p_cr row and data row (read through L1 from global memory).
+__global__ void __launch_bounds__(128) fused_small_problems_kernel(const PhaseArgs a, const TargetView tv,
+                                                                   const ProblemArgs pb) {
+  const ProblemSlot s = problem_slot(a, pb, blockIdx.x * blockDim.x + threadIdx.x);
+  int acc = 0;
+  if (s.valid)
+    acc = small_chain_step<false, BPM_TARGET_JIT, true>(a, tv, tv.data + (size_t)s.g * tv.n_data, s.c, s.n_pool,
+                                                        s.pool, s.rng, s.j, s.p_cr);
+  problem_count(pb, s.g, s.valid, acc);
+}
+
+// ln_like over n rows; rows [g rpp, (g + 1) rpp) see problem g's data row (split path, bpm_eval_lnl)
+__global__ void __launch_bounds__(128) lnl_jit_problems_kernel(const double* __restrict__ P, int n, int ld, int rpp,
+                                                               const double* __restrict__ data, int64_t n_data,
+                                                               double* __restrict__ out) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j < n) out[j] = ln_like(P + (size_t)j * ld, data + (size_t)(j / rpp) * n_data);
+}
+#elif defined(BPM_JIT_LIKELIHOOD)
 // ln_like over a dense [n][ld] block of rows, one thread per row (split path, serial DE-MC, bpm_eval_lnl).
 __global__ void __launch_bounds__(128) lnl_jit_kernel(const double* __restrict__ P, int n, int ld,
                                                       const double* __restrict__ data, int64_t n_data,

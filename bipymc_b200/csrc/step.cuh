@@ -146,6 +146,57 @@ __device__ __forceinline__ PhaseLists phase_lists(const PhaseArgs& a) {
   return L;
 }
 
+// ---- multi-problem handles (bpm_set_problems) --------------------------------------
+// P independent populations of n chains each, problem-major: problem g owns chains [g n, (g + 1) n).  Each
+// has its own Philox key, flip, a/b split, CR state and counters, so problem g steps exactly as a handle of
+// n chains with key keys[g] would.  The split kernel (kernels_problems.cuh) writes, per problem, the halves
+// in permutation order to perm[g n, g n + nA) / [g n + nA, (g + 1) n) (global chain ids) and the same halves
+// in chain order to loc_list.  Thread t of a phase kernel steps slot t % nA of problem t / nA's half.
+struct ProblemArgs {
+  const uint64_t* keys;            // [P] Philox key of each problem
+  const int32_t* flips;            // [P] this generation's flip of each problem
+  const double* p_cr;              // [P][BPM_MAX_CR]
+  unsigned long long* counters;    // [P][2] accepted, rejected
+  int32_t P, n, nA;                // problems, chains per problem, ceil(n / 2)
+};
+// What a phase kernel needs of the chain at slot t: its global id c, its index j within the problem (the
+// RNG counter a single-problem handle uses for it), the pool of the opposite half and the problem's key.
+struct ProblemSlot {
+  int g, c, j, n_pool;
+  bool valid;
+  const int32_t* pool;
+  RngCtx rng;
+  const double* p_cr;
+};
+__device__ __forceinline__ ProblemSlot problem_slot(const PhaseArgs& a, const ProblemArgs& pb, int t) {
+  ProblemSlot s;
+  s.g = t / pb.nA;
+  const int i = t - s.g * pb.nA;
+  s.valid = s.g < pb.P;
+  if (!s.valid) s.g = 0;
+  const int base = s.g * pb.n;
+  const bool first = (a.phase ^ (pb.flips[s.g] != 0)) == 0;   // true: this phase steps half a
+  const int n_self = first ? pb.nA : pb.n - pb.nA;
+  s.valid = s.valid && i < n_self;
+  s.c = s.valid ? a.loc_list[base + (first ? 0 : pb.nA) + i] : base;
+  s.j = s.c - base;
+  s.pool = a.perm + base + (first ? pb.nA : 0);
+  s.n_pool = first ? pb.n - pb.nA : pb.nA;
+  s.rng = make_rng(pb.keys[s.g], (uint64_t)a.hist_len);
+  s.p_cr = pb.p_cr + (size_t)s.g * BPM_MAX_CR;
+  return s;
+}
+// Per-problem accepted / rejected counts of a warp: one atomic per problem the warp touches.
+__device__ __forceinline__ void problem_count(const ProblemArgs& pb, int g, bool valid, int acc) {
+  const unsigned same = __match_any_sync(0xFFFFFFFFu, g);
+  const unsigned am = __ballot_sync(0xFFFFFFFFu, valid && acc) & same;
+  const unsigned rm = __ballot_sync(0xFFFFFFFFu, valid && !acc) & same;
+  if ((threadIdx.x & 31) == __ffs(same) - 1) {
+    if (am) atomicAdd(pb.counters + 2 * g, (unsigned long long)__popc(am));
+    if (rm) atomicAdd(pb.counters + 2 * g + 1, (unsigned long long)__popc(rm));
+  }
+}
+
 // Reduce over the LPC lanes that share one chain (LPC is a power of two <= 32).
 template <int LPC>
 __device__ __forceinline__ int group_sum_i(int v) {
@@ -213,9 +264,11 @@ __device__ __forceinline__ void slot_pair(const Philox4& q, int n_pool, int& r1,
   r2 = (int)j;
 }
 
+// The draws of chain c are addressed by (rng, j): j = c on a single-problem handle; on a multi-problem
+// handle rng carries the problem's key and j is the chain's index within its problem (ProblemArgs).
 template <bool REPLAY>
-__device__ __forceinline__ void chain_scalar_draws(const PhaseArgs& a, int c, int n_pool,
-                                                   ChainDraws& D) {
+__device__ __forceinline__ void chain_scalar_draws(const PhaseArgs& a, const RngCtx& rng, const double* p_cr, int c,
+                                                   int j, int n_pool, ChainDraws& D) {
   const int npair = a.algo == BPM_ALGO_DREAM ? a.del_pairs : 1;
   if (REPLAY) {
     D.cr_idx = a.algo == BPM_ALGO_DREAM ? a.rp.cr_idx[c] : 0;
@@ -228,21 +281,29 @@ __device__ __forceinline__ void chain_scalar_draws(const PhaseArgs& a, int c, in
         D.r2[p] = a.rp.pairs[((size_t)c * npair + p) * 2 + 1];
       }
   } else {
-    const Philox4 s0 = draw4(a.rng, (uint32_t)c, RNG_SCALAR, 0);
-    const Philox4 s1 = draw4(a.rng, (uint32_t)c, RNG_SCALAR, 1);
-    D.cr_idx = a.algo == BPM_ALGO_DREAM ? pick_cr(a.p_cr, a.n_cr, slot0_cr_u(s0)) : 0;
+    const Philox4 s0 = draw4(rng, (uint32_t)j, RNG_SCALAR, 0);
+    const Philox4 s1 = draw4(rng, (uint32_t)j, RNG_SCALAR, 1);
+    D.cr_idx = a.algo == BPM_ALGO_DREAM ? pick_cr(p_cr, a.n_cr, slot0_cr_u(s0)) : 0;
     D.gamma_u = slot1_gamma_u(s1);
     D.fallback = slot1_fallback(s1, a.d);
 #pragma unroll
     for (int p = 0; p < BPM_MAX_PAIRS; ++p)
-      if (p < npair) slot_pair(draw4(a.rng, (uint32_t)c, RNG_SCALAR, 2 + p), n_pool, D.r1[p], D.r2[p]);
+      if (p < npair) slot_pair(draw4(rng, (uint32_t)j, RNG_SCALAR, 2 + p), n_pool, D.r1[p], D.r2[p]);
   }
+}
+template <bool REPLAY>
+__device__ __forceinline__ void chain_scalar_draws(const PhaseArgs& a, int c, int n_pool, ChainDraws& D) {
+  chain_scalar_draws<REPLAY>(a, a.rng, a.p_cr, c, c, n_pool, D);
 }
 
 template <bool REPLAY>
-__device__ __forceinline__ double accept_uniform(const PhaseArgs& a, int c) {
+__device__ __forceinline__ double accept_uniform(const PhaseArgs& a, const RngCtx& rng, int c, int j) {
   if (REPLAY) return a.rp.accept_u[c];
-  return slot0_accept_u(draw4(a.rng, (uint32_t)c, RNG_SCALAR, 0));
+  return slot0_accept_u(draw4(rng, (uint32_t)j, RNG_SCALAR, 0));
+}
+template <bool REPLAY>
+__device__ __forceinline__ double accept_uniform(const PhaseArgs& a, int c) {
+  return accept_uniform<REPLAY>(a, a.rng, c, c);
 }
 
 // BPM_ZEN_ONE = 1: the three per-dimension draws of a 4-dim block -- crossover-mask uniform z (dream.py:52),
@@ -290,7 +351,7 @@ __device__ __forceinline__ void zen_en4(const PhaseArgs& a, const Philox4& q, do
 
 // Four per-dimension draws for dims 4b .. 4b+3 of chain c.
 template <bool REPLAY>
-__device__ __forceinline__ void z4(const PhaseArgs& a, int c, int b, double z[4]) {
+__device__ __forceinline__ void z4(const PhaseArgs& a, const RngCtx& rng, int c, int j, int b, double z[4]) {
   if (REPLAY) {
 #pragma unroll
     for (int t = 0; t < 4; ++t) {
@@ -299,21 +360,26 @@ __device__ __forceinline__ void z4(const PhaseArgs& a, int c, int b, double z[4]
     }
   } else {
 #if BPM_ZEN_ONE
-    Philox4 q = draw4(a.rng, (uint32_t)c, RNG_ZEN, (uint32_t)b);
+    Philox4 q = draw4(rng, (uint32_t)j, RNG_ZEN, (uint32_t)b);
     z[0] = ((double)(q.x & 0xFFFu) + 0.5) * (1.0 / 4096.0); z[1] = ((double)(q.y & 0xFFFu) + 0.5) * (1.0 / 4096.0);
     z[2] = ((double)(q.z & 0xFFFu) + 0.5) * (1.0 / 4096.0); z[3] = ((double)(q.w & 0xFFFu) + 0.5) * (1.0 / 4096.0);
 #else
-    Philox4 q = draw4(a.rng, (uint32_t)c, RNG_Z, (uint32_t)b);
+    Philox4 q = draw4(rng, (uint32_t)j, RNG_Z, (uint32_t)b);
     z[0] = u32d(q.x); z[1] = u32d(q.y); z[2] = u32d(q.z); z[3] = u32d(q.w);
 #endif
   }
+}
+template <bool REPLAY>
+__device__ __forceinline__ void z4(const PhaseArgs& a, int c, int b, double z[4]) {
+  z4<REPLAY>(a, a.rng, c, c, b, z);
 }
 // Box jitter e (dream.py:83, var_box) and Gaussian jitter n (demc.py:182 / dream.py:84,
 // var_ball) for dims 4b .. 4b+3 from ONE Philox call: words x,y give four 16-bit
 // uniforms for e (a +-u_eps box on a 65536-point grid), words z,w two Box-Muller pairs for
 // n (sd epsilon ~ 1e-12: its shape only has to be Gaussian to fp32 accuracy).
 template <bool REPLAY>
-__device__ __forceinline__ void en4(const PhaseArgs& a, int c, int b, double e[4], double n[4]) {
+__device__ __forceinline__ void en4(const PhaseArgs& a, const RngCtx& rng, int c, int j, int b, double e[4],
+                                    double n[4]) {
   if (REPLAY) {
 #pragma unroll
     for (int t = 0; t < 4; ++t) {
@@ -325,11 +391,11 @@ __device__ __forceinline__ void en4(const PhaseArgs& a, int c, int b, double e[4
     e[0] = e[1] = e[2] = e[3] = 0.0;  // var_box returns 0. and draws nothing (util.py:24-28)
     n[0] = n[1] = n[2] = n[3] = 0.0;  // var_ball returns 0. and draws nothing (util.py:11-16)
 #if BPM_ZEN_ONE
-    if (a.u_eps > 0.0 || a.eps > 0.0) zen_en4(a, draw4(a.rng, (uint32_t)c, RNG_ZEN, (uint32_t)b), e, n);
+    if (a.u_eps > 0.0 || a.eps > 0.0) zen_en4(a, draw4(rng, (uint32_t)j, RNG_ZEN, (uint32_t)b), e, n);
     return;
 #endif
     if (a.u_eps > 0.0 || a.eps > 0.0) {
-      const Philox4 q = draw4(a.rng, (uint32_t)c, RNG_EN, (uint32_t)b);
+      const Philox4 q = draw4(rng, (uint32_t)j, RNG_EN, (uint32_t)b);
       if (a.u_eps > 0.0) {
         const double lo = -a.u_eps, w = __dsub_rn(a.u_eps, lo);  // numpy: low + (high-low)*u
         // u = (h + 0.5) / 65536 for a 16-bit h; (2h + 1) * (w * 2^-17) is the same product
@@ -351,6 +417,11 @@ __device__ __forceinline__ void en4(const PhaseArgs& a, int c, int b, double e[4
       }
     }
   }
+}
+
+template <bool REPLAY>
+__device__ __forceinline__ void en4(const PhaseArgs& a, int c, int b, double e[4], double n[4]) {
+  en4<REPLAY>(a, a.rng, c, c, b, e, n);
 }
 
 // dream.py:85-89:  ((1 + e) * gamma * S + n) * mask + cur, evaluated left to right.

@@ -28,6 +28,11 @@ Likelihood plug-ins, fastest first:
      of ``__device__ double ln_like_term(const double* theta, const double* row)`` over the rows of
      ``data[M][k]`` (plus an optional ``ln_prior``), each chain's sum split over the whole GPU between
      the proposal and accept kernels, in an order fixed by M alone;
+  1d. ``ln_like_cuda=targets.CudaLikelihoodSet(source, dim, data[P, n_data])``: the same model fitted to P
+     datasets in ONE sampler.  ``n_chains`` is then the number of chains of one problem; problem g runs
+     exactly as a single-problem sampler with data row g and Philox key ``problem_seeds[g]`` would, and
+     every pooled result (``acceptance_fraction``, ``param_est``, ``p_cr``, ``rhat`` ...) gets a leading
+     axis P.  One rank only; ``subpop_k``, ``outlier_gen``, ``track_covariance`` and ``_replay`` are refused;
   2. ``ln_like_batched=f``: ``f(theta)`` takes a CUDA float64 tensor ``[n, dim]`` and
      returns ``[n]`` log-likelihoods (torch ops on the current stream);
   3. any scalar ``ln_like_fn(theta, **ln_kwargs) -> float`` exactly as in the reference
@@ -328,13 +333,16 @@ class DeMcMpi(object):
     """Parallel DE-MC (emcee-style a/b pools) on B200; mirrors bipymc/demc.py:10."""
     _algo = _lib.BPM_ALGO_DEMC
     _n_phases = 2
+    n_problems = 1           # > 1: a CudaLikelihoodSet of that many problems (n_chains chains each)
+    _seed_keys = None        # Philox keys of the problems, once fixed
 
     def __init__(self, ln_like_fn, theta_0=None, varepsilon=1e-6, n_chains=8,
                  mpi_comm=None, ln_kwargs={}, **kwargs):
         varepsilon = np.asarray(varepsilon)
-        assert n_chains >= 4                                   # samplers.py:249
+        assert n_chains >= 4                                   # samplers.py:249 (per problem)
         self.n_chains = n_chains
         self.comm = _resolve_comm(mpi_comm)
+        self._check_problems(kwargs)
         if n_chains % self.comm.size != 0:
             # the reference counts j per rank (demc.py:79,103-109): ranks with fewer chains run more
             # generations and its fixed-count Allgather (demc.py:93) mismatches -- it hangs.  Say so.
@@ -342,7 +350,9 @@ class DeMcMpi(object):
                              % (n_chains, self.comm.size))
         self.local_n_accepted = 0
         self.local_n_rejected = 1                               # demc.py:19-20
-        if theta_0 is not None:
+        if self._multi:
+            self.dim = self._ln_like_cuda_set.dim
+        elif theta_0 is not None:
             self.dim = len(np.asarray(theta_0))
         else:
             self.dim = kwargs.get("dim", 1)
@@ -392,6 +402,50 @@ class DeMcMpi(object):
         else:
             self.init_warmstart_chain(self.h5_file)
 
+    # ------------------------------------------------------------------ several problems
+    @property
+    def _multi(self):
+        return self.n_problems > 1 or getattr(self, "_ln_like_cuda_set", None) is not None
+
+    @property
+    def _n_all(self):
+        """Chains of the whole population: n_chains per problem times n_problems."""
+        return self.n_chains * self.n_problems
+
+    def _check_problems(self, kwargs):
+        """A CudaLikelihoodSet makes this a multi-problem sampler; refuse what that mode does not offer."""
+        from .targets import CudaLikelihoodSet
+        cuda = kwargs.get("ln_like_cuda", None)
+        seed = kwargs.get("seed", None)
+        if not isinstance(cuda, CudaLikelihoodSet):
+            if seed is not None and np.ndim(seed) != 0:
+                raise ValueError("a sequence of seeds (one per problem) needs ln_like_cuda=targets.CudaLikelihoodSet")
+            return
+        self._ln_like_cuda_set = cuda
+        self.n_problems = cuda.n_problems
+        why = None
+        if self.comm.size > 1:
+            why = "runs on one rank (the problems already fill the GPU)"
+        elif int(kwargs.get("subpop_k", 0)):
+            why = "has no subpop_k"
+        elif int(kwargs.get("outlier_gen", 0)):
+            why = "has no outlier_gen"
+        elif kwargs.get("ln_like_batched", None) is not None:
+            why = "takes its likelihood from the CudaLikelihoodSet only (no ln_like_batched)"
+        elif kwargs.get("device_init", False):
+            why = "draws its initial states on the host (no device_init)"
+        if why:
+            raise ValueError("a multi-problem sampler (ln_like_cuda=CudaLikelihoodSet) " + why)
+        if seed is not None:
+            from .targets import problem_seeds
+            self._seed_keys = problem_seeds(seed, self.n_problems)
+
+    @property
+    def problem_seeds(self):
+        """Philox key of every problem (problem 0's is ``seed``)."""
+        from .targets import problem_seeds
+        return list(self._seed_keys) if self._seed_keys is not None else problem_seeds(self._seed, self.n_problems)
+
     # ------------------------------------------------------------------ plumbing
     def _freeze_ln_like_fn(self, **kwargs):
         self._frozen_ln_like_fn = lambda theta: self.log_like_fn(theta, **kwargs)
@@ -440,8 +494,10 @@ class DeMcMpi(object):
             if self._ln_like_cuda.dim != d:
                 raise ValueError("ln_like_cuda dimension %d != theta_0 dimension %d" % (self._ln_like_cuda.dim, d))
         self._ld = d if d <= 4 else ((d + 3) // 4) * 4
-        ids = np.array_split(np.arange(self.n_chains), self.comm.size)[self.comm.rank]
+        ids = np.array_split(np.arange(self._n_all), self.comm.size)[self.comm.rank]
         self.rank_chain_ids = ids                                   # demc.py:39-40
+        if self._seed_keys is not None:
+            self._seed = int(self._seed_keys[0])
         if self._seed is None:
             # keep np.random.seed(...) meaningful for the native stream as well
             self._seed = int(np.random.randint(0, 2 ** 31 - 1))
@@ -453,7 +509,7 @@ class DeMcMpi(object):
             n_eng, c_lo, c_hi = len(ids), 0, len(ids)
             seed = (self._seed + 0x9E3779B97F4A7C15 * (self.comm.rank + 1)) % (1 << 64)
         else:
-            n_eng, c_lo, c_hi, seed = self.n_chains, int(ids[0]), int(ids[-1]) + 1, self._seed
+            n_eng, c_lo, c_hi, seed = self._n_all, int(ids[0]), int(ids[-1]) + 1, self._seed
         self._n_engine = n_eng
         cfg = _lib.Config(algo=self._algo, n_chains=n_eng, dim=d, ld=self._ld,
                           del_pairs=dc["del_pairs"], n_cr=dc["n_cr"], burnin_gen=dc["burnin_gen"],
@@ -464,6 +520,10 @@ class DeMcMpi(object):
         h = C.c_void_p()
         _lib.check(self._libh.bpm_create(C.byref(cfg), C.byref(h)))
         self._handle = h
+        if self._multi:
+            self._seed_keys = self.problem_seeds
+            keys = np.array(self._seed_keys, dtype=np.uint64)
+            _lib.check(self._libh.bpm_set_problems(h, self.n_problems, keys.ctypes.data_as(C.POINTER(C.c_uint64))))
         # 0 split path, 1 fused (default), 3 / 5 the Gaussian's 12-producer / v3 kernel (include/bipymc_b200.h)
         _lib.check(self._libh.bpm_set_fused(h, int(self._fused)))
         if self._ln_like_cuda is not None:
@@ -686,10 +746,17 @@ class DeMcMpi(object):
         a seeded run starts from the reference's initial states.  (``inflate`` is accepted
         and ignored, as in the reference.)"""
         torch = _torch()
-        theta_0 = np.asarray(theta_0, dtype=float).flatten()
-        self.dim = len(theta_0)
+        if self._multi:
+            # theta_0: [d] shared by every problem, or [P, d]; chain g n + i starts at theta_0[g] + jitter
+            theta_0 = np.asarray(theta_0, dtype=float)
+            if theta_0.shape not in ((self.dim,), (self.n_problems, self.dim)):
+                raise ValueError("theta_0 must have shape (%d,) or (%d, %d)" % (self.dim, self.n_problems, self.dim))
+            theta_0 = np.repeat(np.broadcast_to(theta_0, (self.n_problems, self.dim)), self.n_chains, axis=0)
+        else:
+            theta_0 = np.asarray(theta_0, dtype=float).flatten()
+            self.dim = len(theta_0)
         assert np.all(np.asarray(varepsilon) >= 0.0)
-        N, d = self.n_chains, self.dim
+        N, d = self._n_all, self.dim
         if kwargs.get("device_init", False):
             # populations too large to draw on the host (BASELINE config 5: 10^7 x 1000 doubles = 80 GB):
             # theta_0 + sqrt(varepsilon) * randn on the device, seeded from the sampler's seed.  NOT numpy's
@@ -707,7 +774,7 @@ class DeMcMpi(object):
         # every rank draws the jitter of ALL chains so the replicas agree (demc.py seeds
         # every rank identically as well, tests/test_banana.py:17).  This is the FIRST use
         # of numpy's global stream, exactly as in the reference's constructor.
-        x0 = theta_0[None, :] + var_ball_batch(varepsilon, d, N)
+        x0 = (theta_0 if self._multi else theta_0[None, :]) + var_ball_batch(varepsilon, d, N)
         if self._handle is None:
             self._create_handle()          # draws the Philox seed AFTER the jitter
         if self.comm.size > 1:
@@ -858,6 +925,13 @@ class DeMcMpi(object):
         T = float(self._mom_len)
         if T < 2:
             raise RuntimeError("rhat() needs at least two rows in the running moments")
+        if self._multi:       # [P, d]: the formula of bpm_rhat, per problem
+            P, n, d = self.n_problems, self.n_chains, self.dim
+            mean = self._mean[:, :d].reshape(P, n, d)
+            m2 = self._m2[:, :d].reshape(P, n, d)
+            W = m2.sum(dim=1) / n / (T - 1.0)
+            B_over_T = mean.var(dim=1, unbiased=True)
+            return torch.sqrt(((T - 1.0) / T * W + B_over_T) / W).cpu().numpy()
         if self.comm.size == 1:
             out = np.zeros(self.dim)
             self._flush()
@@ -882,6 +956,8 @@ class DeMcMpi(object):
     def rhat_history(self, t0=None):
         """Gelman-Rubin R-hat per dimension over stored history rows [t0, T) of this rank's
         chains (default: the second half of every chain, Vrugt et al. 2009)."""
+        if self._multi:
+            raise NotImplementedError("rhat_history() is not offered on a multi-problem sampler; use rhat()")
         if self._hist.policy != "full" or self._hist.stored != self._hist.length:
             raise RuntimeError("rhat_history() needs the full stored history; use rhat()")
         if t0 is None:
@@ -942,6 +1018,12 @@ class DeMcMpi(object):
         torch = _torch()
         T = float(self._mom_len)
         mean, m2 = self._gathered_moments()
+        if self._multi:       # [P, d] each
+            mean = mean.reshape(self.n_problems, self.n_chains, self.dim)
+            m2 = m2.reshape(self.n_problems, self.n_chains, self.dim)
+            gm = mean.mean(dim=1)
+            var = (m2.sum(dim=1) + T * ((mean - gm[:, None]) ** 2).sum(dim=1)) / (T * self.n_chains)
+            return gm.cpu().numpy(), torch.sqrt(var).cpu().numpy()
         gm = mean.mean(dim=0)
         var = (m2.sum(dim=0) + T * ((mean - gm[None]) ** 2).sum(dim=0)) / (T * mean.shape[0])
         return gm.cpu().numpy(), torch.sqrt(var).cpu().numpy()
@@ -949,6 +1031,8 @@ class DeMcMpi(object):
     def track_covariance(self, on=True):
         """Start (and zero) / stop the device-side accumulation of the population's cross moments
         (bpm_cov_track): the posterior covariance without a stored history."""
+        if self._multi and on:
+            raise NotImplementedError("track_covariance() is not offered on a multi-problem sampler")
         _lib.check(self._libh.bpm_cov_track(self._handle, 1 if on else 0))
 
     def covariance_estimate(self):
@@ -1014,7 +1098,7 @@ class DeMcMpi(object):
         """Generations the reference's `while j < int((n - N) / size)` loop performs
         (demc.py:78-79, j advances by n_local per generation)."""
         limit = int((n - self.n_chains) / self.comm.size)
-        n_local = len(self.rank_chain_ids)
+        n_local = self.n_chains if self.comm.size == 1 else len(self.rank_chain_ids)   # (per problem)
         if limit <= 0:
             return 0
         return -(-limit // n_local)
@@ -1032,6 +1116,8 @@ class DeMcMpi(object):
         G = self._n_generations(n)
         replay = kwargs.get("_replay", None)
         trace = kwargs.get("_trace", None)
+        if replay is not None and self._multi:
+            raise ValueError("_replay is not offered on a multi-problem sampler")
         if replay is not None:
             G = min(G, len(replay))
         k_gen = 0
@@ -1092,6 +1178,13 @@ class DeMcMpi(object):
         _lib.check(self._libh.bpm_get_counters(self._handle, C.byref(acc), C.byref(rej), C.byref(nan)))
         if nan.value:
             raise ValueError("probabilities contain NaN")       # numpy's message at samplers.py:336
+        if self._multi:       # [P] each, every problem starting its rejections at 1 as the reference does
+            a, r = np.zeros(self.n_problems, np.uint64), np.zeros(self.n_problems, np.uint64)
+            _lib.check(self._libh.bpm_get_problem_counters(self._handle, a.ctypes.data_as(C.POINTER(C.c_uint64)),
+                                                           r.ctypes.data_as(C.POINTER(C.c_uint64))))
+            self.local_n_accepted = self.n_accepted = a.astype(np.int64)
+            self.local_n_rejected = self.n_rejected = 1 + r.astype(np.int64)
+            return
         self.local_n_accepted = int(acc.value)
         self.local_n_rejected = 1 + int(rej.value)
         if self.comm.size > 1:
@@ -1292,6 +1385,9 @@ class DeMcMpi(object):
     def param_est(self, n_burn, collection_rank=0):
         """demc.py:235-248: mean / std over super-chain rows [n_burn:]."""
         self.comm.Barrier()
+        if self._multi:       # ([P, d], [P, d], [P, rows, d]): row g from problem g's own super chain
+            sl = self.super_chain[:, n_burn:, :]
+            return (np.stack([np.mean(x, axis=0) for x in sl]), np.stack([np.std(x, axis=0) for x in sl]), sl)
         chain_slice = self.super_chain_mpi(collection_rank)
         if self.comm.rank == collection_rank:
             chain_slice = chain_slice[n_burn:, :]
@@ -1302,6 +1398,10 @@ class DeMcMpi(object):
         """Same estimate computed on the GPU without moving the history to the host;
         returns (mean, std) as numpy arrays of length dim (rank-local chains when sharded)."""
         h = self._hist.tensor()
+        if self._multi:       # [P, d] each
+            P, n, d = self.n_problems, self.n_chains, self.dim
+            flat = h[:, :, :d].reshape(-1, P, n, d).transpose(0, 1).reshape(P, -1, d)[:, n_burn:]
+            return flat.mean(dim=1).cpu().numpy(), flat.std(dim=1, unbiased=False).cpu().numpy()
         flat = h[:, :, :self.dim].reshape(-1, self.dim)[n_burn:]
         return flat.mean(dim=0).cpu().numpy(), flat.std(dim=0, unbiased=False).cpu().numpy()
 
@@ -1310,7 +1410,12 @@ class DeMcMpi(object):
 
     @property
     def super_chain(self):
-        return self._super_chain()
+        """demc.py:260-270; a multi-problem sampler: [P, T n, d], row t n + i of problem g = its chain i at time t."""
+        sc = self._super_chain()
+        if self._multi:
+            P, n, d = self.n_problems, self.n_chains, self.dim
+            return np.ascontiguousarray(sc.reshape(-1, P, n, d).transpose(1, 0, 2, 3).reshape(P, -1, d))
+        return sc
 
     def _super_chain(self, collection_rank=0):
         """demc.py:260-270: row t*N + i = chain i at time t."""
@@ -1337,13 +1442,13 @@ class DeMcMpi(object):
         if verbose:
             print("Iter all chains on rank: ", self.comm.rank)
         sys.stdout.flush()
-        for c_id in range(self.n_chains):
+        for c_id in range(self._n_all):
             yield self.get_chain(c_id, collection_rank)
 
     def get_chain(self, c_id, collection_rank=0, verbose=0):
         """demc.py:296-325.  Single rank: the local view.  Multi rank: a free-standing
         host McmcChain on the collection rank, None elsewhere."""
-        assert 0 <= c_id < self.n_chains
+        assert 0 <= c_id < self._n_all
         if self.comm.size == 1:
             return self.am_chains[c_id]
         sc = self._super_chain(collection_rank)
@@ -1375,22 +1480,32 @@ class DeMcMpi(object):
             h5py = None if h5_file.endswith(".npz") else _try_h5py()
             if h5py is not None:
                 with h5py.File(h5_file, "w") as h5f:
-                    for c_id in range(self.n_chains):
-                        h5f.create_dataset("/chains/chain_id_" + str(c_id), data=sc[c_id::self.n_chains, :],
+                    for c_id in range(self._n_all):
+                        h5f.create_dataset("/chains/chain_id_" + str(c_id), data=sc[c_id::self._n_all, :],
                                            compression="gzip")
                     for k, v in extra.items():
                         h5f["/chains"].attrs[k] = v
             else:
-                T = sc.shape[0] // self.n_chains
-                np.savez_compressed(_npz_name(h5_file), history=sc.reshape(T, self.n_chains, self.dim), **extra)
+                T = sc.shape[0] // self._n_all
+                np.savez_compressed(_npz_name(h5_file), history=sc.reshape(T, self._n_all, self.dim), **extra)
         self.comm.Barrier()
 
     def _checkpoint_extra(self):
-        return dict(b200_seed=np.uint64(self._seed))
+        e = dict(b200_seed=np.uint64(self._seed))
+        if self._multi:
+            e.update(b200_problem_seeds=np.array(self.problem_seeds, dtype=np.uint64),
+                     b200_n_problems=np.int64(self.n_problems), b200_problem_chains=np.int64(self.n_chains))
+        return e
 
     def _restore_extra(self, extra):
         if "b200_seed" in extra:
             self._seed = int(extra["b200_seed"])
+        if self._multi:
+            if "b200_problem_seeds" not in extra or int(extra["b200_n_problems"]) != self.n_problems or \
+                    int(extra["b200_problem_chains"]) != self.n_chains:
+                raise RuntimeError("the checkpoint is not one of %d problems of %d chains" % (self.n_problems,
+                                                                                              self.n_chains))
+            self._seed_keys = [int(k) for k in np.asarray(extra["b200_problem_seeds"], dtype=np.uint64).ravel()]
 
     def load_state(self, h5_file=""):
         """demc.py:217-233."""
@@ -1400,9 +1515,9 @@ class DeMcMpi(object):
         if h5py is not None:
             with h5py.File(h5_file, "r") as h5f:
                 names = set(h5f["/chains"].keys())
-                if names != set("chain_id_" + str(int(c)) for c in range(self.n_chains)):
+                if names != set("chain_id_" + str(int(c)) for c in range(self._n_all)):
                     raise RuntimeError        # another population's file (the .npz branch below rejects it too)
-                chains = [h5f["/chains/chain_id_" + str(int(c))][:] for c in range(self.n_chains)]
+                chains = [h5f["/chains/chain_id_" + str(int(c))][:] for c in range(self._n_all)]
                 extra = dict((k, np.asarray(v)) for k, v in h5f["/chains"].attrs.items())
             k_gen = len(chains[0])
             for ch in chains:
@@ -1413,11 +1528,11 @@ class DeMcMpi(object):
             with np.load(_npz_name(h5_file)) as z:
                 hist = z["history"]
                 extra = dict((k, z[k]) for k in z.files if k != "history")
-            if hist.shape[1] != self.n_chains:
+            if hist.shape[1] != self._n_all:
                 raise RuntimeError
-        seed_before = self._seed
+        seed_before = (self._seed, self._seed_keys)
         self._restore_extra(extra)
-        if self._seed != seed_before:
+        if (self._seed, self._seed_keys) != seed_before:
             # the Philox key is part of the engine configuration: rebuild the handle
             self._release_peer_memory()
             self._libh.bpm_destroy(self._handle)
@@ -1433,7 +1548,7 @@ class DeMcMpi(object):
     def load_history(self, hist):
         """hist: (T, N, dim) array of every chain's history (what load_state reads)."""
         hist = np.asarray(hist, dtype=float)
-        assert hist.shape[1] == self.n_chains and hist.shape[2] == self.dim
+        assert hist.shape[1] == self._n_all and hist.shape[2] == self.dim
         if self._subpop:      # an island's rows inside the job-wide history are its GLOBAL chain ids
             lo, hi = int(self.rank_chain_ids[0]), int(self.rank_chain_ids[-1]) + 1
         else:

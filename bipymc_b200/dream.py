@@ -59,18 +59,23 @@ class DreamMpi(DeMcMpi):
     def _init_cr(self):
         """dream.py:109-117."""
         self.CR = (np.array(range(self.n_cr)) + 1) / self.n_cr
-        n = self.n_cr
-        self._set_cr(np.ones(n) / n, np.zeros(n), np.zeros(n))
+        shape = self._cr_shape()
+        self._set_cr(np.ones(shape) / self.n_cr, np.zeros(shape), np.zeros(shape))
+
+    def _cr_shape(self):
+        """[n_cr], or [P, n_cr] on a multi-problem sampler (one row per problem)."""
+        return (self.n_problems, self.n_cr) if self._multi else (self.n_cr,)
 
     def _set_cr(self, p_cr, delta_m, n_cr_updates):
-        a = [np.ascontiguousarray(np.asarray(v, dtype=np.float64)) for v in (p_cr, delta_m, n_cr_updates)]
-        _lib.check(self._libh.bpm_set_cr_state(self._handle, _lib.dptr(a[0]), _lib.dptr(a[1]),
-                                               _lib.dptr(a[2])))
+        a = [np.ascontiguousarray(np.asarray(v, dtype=np.float64).reshape(self._cr_shape()))
+             for v in (p_cr, delta_m, n_cr_updates)]
+        fn = self._libh.bpm_set_problem_cr_state if self._multi else self._libh.bpm_set_cr_state
+        _lib.check(fn(self._handle, _lib.dptr(a[0]), _lib.dptr(a[1]), _lib.dptr(a[2])))
 
     def _get_cr(self):
-        out = [np.zeros(self.n_cr) for _ in range(3)]
-        _lib.check(self._libh.bpm_get_cr_state(self._handle, _lib.dptr(out[0]), _lib.dptr(out[1]),
-                                               _lib.dptr(out[2])))
+        out = [np.zeros(self._cr_shape()) for _ in range(3)]
+        fn = self._libh.bpm_get_problem_cr_state if self._multi else self._libh.bpm_get_cr_state
+        _lib.check(fn(self._handle, _lib.dptr(out[0]), _lib.dptr(out[1]), _lib.dptr(out[2])))
         return out
 
     @property
@@ -96,8 +101,8 @@ class DreamMpi(DeMcMpi):
 
     def _checkpoint_extra(self):
         e = super(DreamMpi, self)._checkpoint_extra()
-        p_cr, dm, cnt = self._get_cr()
-        e.update(b200_p_cr=p_cr, b200_delta_m=dm, b200_n_cr_updates=cnt)
+        p_cr, dm, cnt = self._get_cr()       # (flat: [P n_cr] on a multi-problem sampler)
+        e.update(b200_p_cr=p_cr.ravel(), b200_delta_m=dm.ravel(), b200_n_cr_updates=cnt.ravel())
         return e
 
     def _restore_extra_late(self, extra):

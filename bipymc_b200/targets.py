@@ -11,7 +11,8 @@ Mirrors the reference's test-target classes (same constructor arguments, same ``
 
 and ``CudaLikelihood``: any other model as CUDA C++ source, compiled at run time into the same
 kernels (``ln_like_cuda=`` of the samplers); ``CudaSumLikelihood``: a model that is a sum over
-observations, one CUDA C++ term per observation, summed across the whole GPU.
+observations, one CUDA C++ term per observation, summed across the whole GPU; ``CudaLikelihoodSet``: one
+``ln_like`` source fitted to many datasets at once, each an independent problem of the same sampler.
 
 ``ln_like`` stays a scalar host function, so the objects remain valid ``ln_like_fn``
 arguments everywhere; when a sampler of this package receives ``obj.ln_like`` it
@@ -352,6 +353,68 @@ class CudaLikelihood(object):
         """Compile (or take the cached cubin), load it on the handle's device and copy the data."""
         return self._call(lib.bpm_set_jit_target, handle, self.source.encode(), _lib.dptr(self.data),
                           self.data.size, self._flags)
+
+
+class CudaLikelihoodSet(CudaLikelihood):
+    """One CUDA likelihood fitted to P datasets at once: P independent problems in one sampler.
+
+    ``source`` is the ``ln_like`` of ``CudaLikelihood``; ``data`` is a finite float64 array of shape
+    ``(P, n_data)`` with P >= 1 and n_data >= 1, and problem g's ``ln_like`` sees row g (``BPM_NDATA`` is
+    n_data, ``BPM_NPROBLEMS`` is P).  Pass it as ``ln_like_cuda=`` to ``DreamMpi`` / ``DeMcMpi``: their
+    ``n_chains`` then counts the chains of ONE problem, and problem g steps exactly -- bit for bit -- as a
+    single-problem sampler with ``n_chains`` chains, data row g and Philox key ``sampler.problem_seeds[g]``
+    would, while all P problems run in the same kernel launches.  Validation, ``fmad``, the NaN rule,
+    ``CudaCompileError`` and the compile cache are those of ``CudaLikelihood``; P and n_data are part of the
+    cache key, and the kernels are compiled in a translation unit of their own."""
+
+    def __init__(self, source, dim, data, fmad=True):
+        if not isinstance(source, str):
+            raise ValueError("source must be a str of CUDA C++")
+        if isinstance(dim, bool) or int(dim) != dim or int(dim) < 1:
+            raise ValueError("dim must be an integer >= 1")
+        data = np.asarray(data, dtype=np.float64)
+        if data.ndim != 2 or data.shape[0] < 1 or data.shape[1] < 1:
+            raise ValueError("data must have shape (P, n_data) with P >= 1 and n_data >= 1: one row per problem")
+        if data.shape[0] >= 2 ** 31:
+            raise ValueError("data must have fewer than 2^31 rows")
+        if not np.all(np.isfinite(data)):
+            raise ValueError("data must be finite")
+        self.source = source
+        self.dim = int(dim)
+        self.data = np.ascontiguousarray(data)
+        self.fmad = bool(fmad)
+
+    @property
+    def n_problems(self):
+        return int(self.data.shape[0])
+
+    def compile(self):
+        """Compile for sm_100a (no device needed).  Returns True when the cubin came from the
+        process cache; raises CudaCompileError with the NVRTC log."""
+        lib = _lib.load()
+        P, nd = self.data.shape
+        return self._call(lib.bpm_jit_compile_problems, self.source.encode(), self.dim, nd, P, self._flags)
+
+    def _attach(self, lib, handle):
+        """Compile (or take the cached cubin), load it on the handle's device and copy the data (the handle
+        must be a multi-problem handle with P problems: bpm_set_problems)."""
+        return self._call(lib.bpm_set_jit_problems_target, handle, self.source.encode(), _lib.dptr(self.data),
+                          self.data.shape[1], self._flags)
+
+
+def problem_seeds(seed, n_problems):
+    """Philox keys of P problems: ``(seed + 0x9E3779B97F4A7C15 g) mod 2^64`` for an int seed (problem 0
+    keeps ``seed``), or a sequence of P ints taken as they are."""
+    P = int(n_problems)
+    if np.ndim(seed) == 0:
+        s = int(seed)
+        return [(s + 0x9E3779B97F4A7C15 * g) % (1 << 64) for g in range(P)]
+    keys = [int(k) for k in seed]
+    if len(keys) != P:
+        raise ValueError("seed: %d keys for %d problems" % (len(keys), P))
+    if any(not 0 <= k < (1 << 64) for k in keys):
+        raise ValueError("seed: every key must be in [0, 2^64)")
+    return keys
 
 
 class CudaSumLikelihood(CudaLikelihood):

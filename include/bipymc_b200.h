@@ -182,6 +182,31 @@ int bpm_jit_compile_sum(const char* source, int32_t dim, int64_t n_rows, int32_t
 int bpm_set_jit_sum_target(bpm_handle h, const char* source, const double* data, int64_t n_rows, int32_t row_len,
                            int32_t flags, int32_t* from_cache, char* log, int64_t log_cap);
 
+/* Multi-problem handles: P independent problems of n chains each in one handle (population P n, problem-major:
+ * problem g owns chains [g n, (g + 1) n)).  Problem g steps exactly as a handle of n chains with seed keys[g]
+ * would -- same flip, halves, partners, draws, CR adaptation and counters, bit for bit -- and every problem
+ * sees its own data row.  All P problems run in the same launches: per generation one split kernel, two
+ * phase launches (fused at dim <= 4, else propose + likelihood + accept each) and, for DREAM, one CR launch,
+ * whatever P is.
+ * bpm_set_problems is called right after bpm_create, on an unsharded DE-MC or DREAM handle with
+ * n_chains % n_problems == 0 and n = n_chains / n_problems >= 4; keys[n_problems] (HOST) are the problems'
+ * Philox keys.  The likelihood is then set with bpm_set_jit_problems_target: the ln_like source of
+ * bpm_jit_compile, with data the row-major [P][n_data] HOST array (n_data >= 1): problem g's ln_like gets
+ * data + g n_data, and BPM_NDATA is n_data (BPM_NPROBLEMS is P).  P and n_data are part of the cache key.
+ * A multi-problem handle offers bpm_step_generations, bpm_flush, bpm_moments_from_history, bpm_eval_lnl
+ * (n a multiple of P; rows problem-major, n / P per problem), bpm_get_counters (totals over the problems),
+ * bpm_reset_counters, bpm_set_run_params, bpm_set_fused, bpm_profile / bpm_profile_read and the problem
+ * entry points below; every other entry point that takes the handle fails naming the multi-problem mode.
+ * CR state and counters per problem: [P][n_cr] arrays, and acc[P] / rej[P] (HOST). */
+int bpm_set_problems(bpm_handle h, int32_t n_problems, const uint64_t* keys);
+int bpm_jit_compile_problems(const char* source, int32_t dim, int64_t n_data, int32_t n_problems, int32_t flags,
+                             int32_t* from_cache, char* log, int64_t log_cap);
+int bpm_set_jit_problems_target(bpm_handle h, const char* source, const double* data, int64_t n_data, int32_t flags,
+                                int32_t* from_cache, char* log, int64_t log_cap);
+int bpm_get_problem_cr_state(bpm_handle h, double* p_cr, double* dm, double* cnt);
+int bpm_set_problem_cr_state(bpm_handle h, const double* p_cr, const double* dm, const double* cnt);
+int bpm_get_problem_counters(bpm_handle h, uint64_t* acc, uint64_t* rej);
+
 /* ln_like for n rows (device in, device out) with the current target. */
 int bpm_eval_lnl(bpm_handle h, const double* X, int32_t n, double* lnl, bpm_stream stream);
 
