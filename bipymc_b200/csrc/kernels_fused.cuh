@@ -180,7 +180,7 @@ struct GaussTables {
   double* gam;   // gamma_base[d'] for d' = 0..d (dream.py:61)
   double* cdf;   // normalised CR cdf (dream.py:51)
   double* crv;   // CR values (dream.py:113)
-  uint32_t* thr; // native mode: mask_i = (philox word <= thr[m])  <=>  u32d(word) <= CR[m]
+  uint32_t* thr; // native mode: mask_i = (12-bit z word <= thr[m])  <=>  z_i <= CR[m]   (zen_threshold)
 };
 __host__ __device__ inline size_t gauss_table_doubles(int d) {
   return (size_t)d * kWld + ((d + 1) & ~1) + ((d + 2) & ~1) + 2 * BPM_MAX_CR + BPM_MAX_CR / 2;
@@ -202,9 +202,10 @@ __device__ __forceinline__ GaussTables carve_tables(double* smem, int d) {
   return t;
 }
 
-__device__ __forceinline__ void fill_tables(const PhaseArgs& a, const GaussArgs& g, const GaussTables& t,
-                                            int tid, int nthreads) {
-  load_W_shared(t.Ws, t.mus, g.W, g.mu, a.d, g.r, tid, nthreads);
+// the small proposal-stage tables; the v3 / v4 kernels call this alone: their consumers load W (83 KB), in the
+// shadow of the producers' first tile
+__device__ __forceinline__ void fill_tables_v3(const PhaseArgs& a, const GaussArgs& g, const GaussTables& t,
+                                               int tid, int nthreads) {
   for (int dp = tid; dp <= a.d; dp += nthreads)
     t.gam[dp] = dp == 0 ? 0.0
                         : __ddiv_rn(a.gamma_num, __dsqrt_rn(__dmul_rn(__dmul_rn(2.0, (double)a.del_pairs),
@@ -217,15 +218,14 @@ __device__ __forceinline__ void fill_tables(const PhaseArgs& a, const GaussArgs&
       acc = __dadd_rn(acc, a.p_cr[m]);
       t.cdf[m] = __ddiv_rn(acc, tot);
       t.crv[m] = __ddiv_rn((double)(m + 1), (double)a.n_cr);
-      // u32d(w) = (w + 0.5) 2^-32 <= cr  <=>  w <= floor(cr 2^32 - 0.5)   (all steps exact)
-#if BPM_ZEN_ONE
       t.thr[m] = zen_threshold(t.crv[m]);
-#else
-      const double lim = floor(t.crv[m] * 4294967296.0 - 0.5);
-      t.thr[m] = lim >= 4294967295.0 ? 0xFFFFFFFFu : (uint32_t)lim;
-#endif
     }
   }
+}
+__device__ __forceinline__ void fill_tables(const PhaseArgs& a, const GaussArgs& g, const GaussTables& t,
+                                            int tid, int nthreads) {
+  load_W_shared(t.Ws, t.mus, g.W, g.mu, a.d, g.r, tid, nthreads);
+  fill_tables_v3(a, g, t, tid, nthreads);
 }
 
 // One instruction pulls a whole row into L2 (no registers, no shared memory): issued for
@@ -776,35 +776,24 @@ constexpr int kV3Threads = 32 * (kV3ConsWarps + kV3ProdWarps);   // 640
 constexpr int kV3ProdThreads = 32 * kV3ProdWarps;
 constexpr int kV3ConsThreads = 32 * kV3ConsWarps;
 
-#ifdef BPM_GATHER_CG
-__device__ __forceinline__ double2 ldg2(const double* p) { return __ldcg(reinterpret_cast<const double2*>(p)); }
-#else
 __device__ __forceinline__ double2 ldg2(const double* p) { return *reinterpret_cast<const double2*>(p); }
-#endif
 
 // ---- lane -> dimension map of the write-back ----------------------------------------------
-// A lane owns two 16-byte chunks of a chain row.  "Sector" map (BPM_V3_WB_SECTOR = 1, default):
-// dims {2l, 2l+1} and {64+2l, 65+2l}, so a 128-bit warp access covers 512 contiguous bytes = whole
-// 32-byte sectors.  The plain map (dims 4l .. 4l+3) makes every access touch half of each sector,
-// and every sector twice.  Every array the write-back touches is per-dimension independent, so the
-// map is free there: 148.8 -> 141.8 us per launch (profiles/r1_consumer_experiments.txt).  The
-// proposal stage keeps the plain map: in the sector map the Philox words of a 4-dim slot and the
-// jump statistic have to be passed between lanes by ~20 shuffles, which cost more than the halved
-// sector count saved (153.2 against 143.6 us, branch exp/split-writeback).
-#ifndef BPM_V3_WB_SECTOR
-#define BPM_V3_WB_SECTOR 1
-#endif
+// A lane owns two 16-byte chunks of a chain row: dims {2l, 2l+1} and {64+2l, 65+2l}, so a 128-bit
+// warp access covers 512 contiguous bytes = whole 32-byte sectors.  The plain map (dims 4l .. 4l+3)
+// makes every access touch half of each sector, and every sector twice.  Every array the write-back
+// touches is per-dimension independent, so the map is free there: 148.8 -> 141.8 us per launch
+// against the plain map (profiles/r1_consumer_experiments.txt).  The proposal stage keeps the plain
+// map: in the sector map the Philox words of a 4-dim slot and the jump statistic have to be passed
+// between lanes by ~20 shuffles, which cost more than the halved sector count saved (153.2 against
+// 143.6 us, branch exp/split-writeback).
 struct WbMap {
   int o0, o1;      // element offsets of the lane's two 16-byte chunks inside a row
   bool h0, h1;     // chunk inside the row
 };
 __device__ __forceinline__ WbMap wb_map(int d, int lane) {
   WbMap m;
-#if BPM_V3_WB_SECTOR
   m.o0 = 2 * lane; m.o1 = 64 + 2 * lane;
-#else
-  m.o0 = 4 * lane; m.o1 = 4 * lane + 2;
-#endif
   m.h0 = m.o0 < d; m.h1 = m.o1 < d;     // d is even
   return m;
 }
@@ -909,12 +898,7 @@ __device__ __forceinline__ void tile_stage_propose_v3(const PhaseArgs& a, const 
             if (z[q] <= cr) mbits |= 1u << q;
         } else {
           const uint32_t th = tb.thr[m];
-#if BPM_ZEN_ONE
           mbits = zen_mask4(draw4(a.rng, (uint32_t)c, RNG_ZEN, (uint32_t)lane), th);
-#else
-          const Philox4 q = draw4(a.rng, (uint32_t)c, RNG_Z, (uint32_t)lane);
-          mbits = (q.x <= th ? 1u : 0u) | (q.y <= th ? 2u : 0u) | (q.z <= th ? 4u : 0u) | (q.w <= th ? 8u : 0u);
-#endif
         }
       }
       int d_prime = __reduce_add_sync(0xFFFFFFFFu, __popc(mbits));
@@ -998,22 +982,12 @@ __device__ __forceinline__ void mbar_wait(uint64_t* b, uint32_t parity) {
   }
 }
 
-// Measured (profiles/r1_ab_prefetch.txt): with 16 independent producer warps the L2 bulk
-// prefetch one tile ahead no longer pays -- the kernel is 9 % faster without it.
-#ifndef BPM_PF_MODE
-#define BPM_PF_MODE 0     // 0 none, 1 population + moments rows, 2 moments rows only, 3 population rows only
-#endif
-__device__ __forceinline__ void v3_prefetch_x(const double* p, int bytes) {
-  if (BPM_PF_MODE == 1 || BPM_PF_MODE == 3) l2_prefetch_row(p, bytes);
-}
-__device__ __forceinline__ void v3_prefetch_mom(const double* p, int bytes) {
-  if (BPM_PF_MODE == 1 || BPM_PF_MODE == 2) l2_prefetch_row(p, bytes);
-}
-
 // Per-warp scalar draws: producer warp pw owns tile rows pw, pw + 16, pw + 32, pw + 48 from the
 // draws to the write-back, so the scratch of a row is written and read by one warp only (plus
 // the consumers, ordered by the FULL mbarrier).  gid0 = population-list index of tile row 0,
-// gid_end = end of this CTA's row range.
+// gid_end = end of this CTA's row range.  No L2 prefetch of the rows a tile will touch: with 16
+// independent producer warps it no longer pays -- the kernel is 9 % faster without it
+// (profiles/r1_ab_prefetch.txt).
 template <bool REPLAY>
 __device__ __forceinline__ void warp_stage_draws(const PhaseArgs& a, const PhaseLists& L,
                                                  const GaussTables& tb, TileScratch& T, int gid0,
@@ -1031,13 +1005,6 @@ __device__ __forceinline__ void warp_stage_draws(const PhaseArgs& a, const Phase
     valid = valid && c >= a.chain_lo && c < a.chain_hi;
     if (slot == 0) T.cid[row] = valid ? c : -1;
     if (!valid) continue;
-    const int row_bytes = a.ld * 8;
-    if (slot == 0) {
-      v3_prefetch_x(a.X + (size_t)c * a.ld, row_bytes);
-      if (a.mean) v3_prefetch_mom(a.mean + (size_t)(c - a.chain_lo) * a.ld, row_bytes);
-    } else if (slot == 1) {
-      if (a.m2) v3_prefetch_mom(a.m2 + (size_t)(c - a.chain_lo) * a.ld, row_bytes);
-    }
     if (REPLAY) {
       if (slot == 0) {
         T.cr_idx[row] = dream ? a.rp.cr_idx[c] : 0;
@@ -1049,8 +1016,6 @@ __device__ __forceinline__ void warp_stage_draws(const PhaseArgs& a, const Phase
         const int p = slot - 2;
         T.pa[row][p] = L.pool[a.rp.pairs[((size_t)c * npair + p) * 2 + 0]];
         T.pb[row][p] = L.pool[a.rp.pairs[((size_t)c * npair + p) * 2 + 1]];
-        v3_prefetch_x(a.X + (size_t)T.pa[row][p] * a.ld, row_bytes);
-        v3_prefetch_x(a.X + (size_t)T.pb[row][p] * a.ld, row_bytes);
       }
     } else {
       const Philox4 q = draw4(a.rng, (uint32_t)c, RNG_SCALAR, (uint32_t)slot);
@@ -1075,8 +1040,6 @@ __device__ __forceinline__ void warp_stage_draws(const PhaseArgs& a, const Phase
         BPM_CHECK(ga >= 0 && ga < a.N && gb >= 0 && gb < a.N, "partner chain id", ga);
         T.pa[row][slot - 2] = ga;
         T.pb[row][slot - 2] = gb;
-        v3_prefetch_x(a.X + (size_t)ga * a.ld, row_bytes);
-        v3_prefetch_x(a.X + (size_t)gb * a.ld, row_bytes);
       }
     }
   }
@@ -1106,32 +1069,6 @@ __host__ __device__ inline size_t v3_ptile_doubles(int d) { return (size_t)kTile
 inline size_t fused_v3_smem(int d) {
   return sizeof(double) * (gauss_table_doubles(d) + 2 * v3_ptile_doubles(d) + 3 * gauss_scratch_doubles() + 4);
 }
-// the small proposal-stage tables; W (83 KB) is loaded by the consumers alone, in the shadow of
-// the producers' first tile
-__device__ __forceinline__ void fill_tables_v3(const PhaseArgs& a, const GaussArgs& g, const GaussTables& t,
-                                               int tid, int nthreads) {
-  for (int dp = tid; dp <= a.d; dp += nthreads)
-    t.gam[dp] = dp == 0 ? 0.0
-                        : __ddiv_rn(a.gamma_num, __dsqrt_rn(__dmul_rn(__dmul_rn(2.0, (double)a.del_pairs),
-                                                                      (double)dp)));
-  if (tid == 0) {
-    double tot = 0.0;
-    for (int m = 0; m < a.n_cr; ++m) tot = __dadd_rn(tot, a.p_cr[m]);
-    double acc = 0.0;
-    for (int m = 0; m < a.n_cr; ++m) {
-      acc = __dadd_rn(acc, a.p_cr[m]);
-      t.cdf[m] = __ddiv_rn(acc, tot);
-      t.crv[m] = __ddiv_rn((double)(m + 1), (double)a.n_cr);
-#if BPM_ZEN_ONE
-      t.thr[m] = zen_threshold(t.crv[m]);
-#else
-      const double lim = floor(t.crv[m] * 4294967296.0 - 0.5);
-      t.thr[m] = lim >= 4294967295.0 ? 0xFFFFFFFFu : (uint32_t)lim;
-#endif
-    }
-  }
-}
-
 template <bool REPLAY, bool CENTER, int NPAIR>
 __global__ void __launch_bounds__(kV3Threads, 1)
 fused_gauss_v3_kernel(const PhaseArgs a, const GaussArgs g) {

@@ -330,9 +330,7 @@ fused_gauss_v4_kernel(const PhaseArgs a, const GaussArgs g) {
     uint32_t mbits = 0xFu;
     double gamma;
     const double gu = T.gamma_u[row];
-#if BPM_ZEN_ONE
     Philox4 qzen = {0u, 0u, 0u, 0u};       // the block's single Philox call, shared by the mask and the jitters
-#endif
     if (dream) {
       const int m = T.cr_idx[row];
       if (REPLAY) {
@@ -342,13 +340,8 @@ fused_gauss_v4_kernel(const PhaseArgs a, const GaussArgs g) {
         mbits = (z[0] <= cr ? 1u : 0u) | (z[1] <= cr ? 2u : 0u) | (z[2] <= cr ? 4u : 0u) | (z[3] <= cr ? 8u : 0u);
       } else {
         const uint32_t th = tb.thr[m];
-#if BPM_ZEN_ONE
         qzen = draw4(a.rng, (uint32_t)c, RNG_ZEN, (uint32_t)lc);
         mbits = zen_mask4(qzen, th);
-#else
-        const Philox4 q = draw4(a.rng, (uint32_t)c, RNG_Z, (uint32_t)lc);
-        mbits = (q.x <= th ? 1u : 0u) | (q.y <= th ? 2u : 0u) | (q.z <= th ? 4u : 0u) | (q.w <= th ? 8u : 0u);
-#endif
       }
       int d_prime = __reduce_add_sync(0xFFFFFFFFu, act ? __popc(mbits) : 0);
       if (d_prime == 0) {
@@ -364,12 +357,8 @@ fused_gauss_v4_kernel(const PhaseArgs a, const GaussArgs g) {
     double delta = 0.0, prv[4];
     {
       double e[4], nn[4];
-#if BPM_ZEN_ONE
       if (!REPLAY && dream) zen_en4(a, qzen, e, nn);
       else en4<REPLAY>(a, c, lc, e, nn);
-#else
-      en4<REPLAY>(a, c, lc, e, nn);
-#endif
       if (fold) {
         welford_update(cur[0], a.inv_mom, mn0.x, var[0]);
         welford_update(cur[1], a.inv_mom, mn0.y, var[1]);

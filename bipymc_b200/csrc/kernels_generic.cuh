@@ -196,7 +196,7 @@ __global__ void __launch_bounds__(kThreads, LPC == 32 ? 2 : 1) propose_kernel(co
   double gamma;
   // large d (one warp per chain, rows of whole 32-byte sectors): pass 2 below works block-wise with 16-byte
   // accesses and reuses pass 1's Philox words
-  constexpr bool kKeepDraws = LPC == 32 && !REPLAY && BPM_ZEN_ONE;
+  constexpr bool kKeepDraws = LPC == 32 && !REPLAY;
   const bool vec = LPC == 32 && (a.ld & 3) == 0;
   Philox4 qs[kKeepDraws ? kMaxBlocksPerLane : 1];
   if (dream) {
@@ -212,8 +212,7 @@ __global__ void __launch_bounds__(kThreads, LPC == 32 ? 2 : 1) propose_kernel(co
             const Philox4 q = PROB ? draw4(ps.rng, (uint32_t)ps.j, RNG_ZEN, (uint32_t)b)
                                    : draw4(a.rng, (uint32_t)c, RNG_ZEN, (uint32_t)b);
             qs[t] = q;
-            z[0] = ((double)(q.x & 0xFFFu) + 0.5) * (1.0 / 4096.0); z[1] = ((double)(q.y & 0xFFFu) + 0.5) * (1.0 / 4096.0);
-            z[2] = ((double)(q.z & 0xFFFu) + 0.5) * (1.0 / 4096.0); z[3] = ((double)(q.w & 0xFFFu) + 0.5) * (1.0 / 4096.0);
+            zen_z4(q, z);
           } else {
             if constexpr (PROB) z4<REPLAY>(a, ps.rng, c, ps.j, b, z);
             else z4<REPLAY>(a, c, b, z);
@@ -611,32 +610,6 @@ __global__ void cr_apply_kernel(const double* __restrict__ part, int n_cr, doubl
                                 double* __restrict__ cnt, double* __restrict__ p_cr) {
   if (threadIdx.x != 0 || blockIdx.x != 0) return;
   cr_apply(part, n_cr, dm, cnt, p_cr);
-}
-
-// ---- host-buffer entry: write back only what changed ------------------------------
-// changed[c] |= accept[c] after every generation; then one warp per chain stores the rows of the
-// chains that moved (and their cached lnL) straight into the caller's pinned host buffers
-// (mapped memory, PCIe posted writes).  With ~15-25 % acceptance the device->host traffic of a
-// generation drops from the whole population to the accepted rows.
-__global__ void or_flags_kernel(int32_t* __restrict__ changed, const int32_t* __restrict__ accept, int N) {
-  const int c = blockIdx.x * blockDim.x + threadIdx.x;
-  if (c < N && accept[c]) changed[c] = 1;
-}
-__global__ void __launch_bounds__(256) scatter_changed_rows_kernel(const double* __restrict__ X,
-                                                                   const double* __restrict__ lnl,
-                                                                   const int32_t* __restrict__ changed,
-                                                                   double* __restrict__ X_host,
-                                                                   double* __restrict__ lnl_host, int N, int ld,
-                                                                   unsigned long long* __restrict__ n_rows) {
-  const int c = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
-  if (c >= N || !changed[c]) return;
-  const double* src = X + (size_t)c * ld;
-  double* dst = X_host + (size_t)c * ld;
-  for (int i = lane; i < ld; i += 32) dst[i] = src[i];
-  if (lane == 0) {
-    lnl_host[c] = lnl[c];
-    atomicAdd(n_rows, 1ull);
-  }
 }
 
 // ---- lazy protocol: materialise the pending row (bpm_flush) ---------------------------

@@ -39,12 +39,11 @@ __host__ __device__ __forceinline__ Philox4 philox4x32_10(uint32_t c0, uint32_t 
   return o;
 }
 
-// Purposes (high byte of counter word 3).
+// Purposes (high byte of counter word 3).  The values are part of the counter: renumbering one
+// changes the draws of every run that uses it.
 enum : uint32_t {
   RNG_SCALAR = 0,  // slot 0: cr_u | accept_u ; slot 1: gamma_u | fallback ; slot 2+p: pair p
-  RNG_Z = 1,       // slot = dim/4: four mask uniforms
-  RNG_EN = 2,      // slot = dim/4: four box-jitter uniforms (16 bit) + four jitter normals
-  RNG_ZEN = 3,     // (BPM_ZEN_ONE) slot = dim/4: mask uniform, box jitter and jitter normal of four dims in ONE call
+  RNG_ZEN = 3,     // slot = dim/4: mask uniform, box jitter and jitter normal of four dims in ONE call
   RNG_GEN = 4,     // chain = 0xFFFFFFFF: slot 0 flip_u + Feistel keys, slot 1 more keys
   RNG_INIT = 5     // device-side chain initialisation jitter
 };
@@ -74,10 +73,6 @@ __host__ __device__ __forceinline__ double u53(uint32_t hi, uint32_t lo) {
   uint64_t v = (((uint64_t)hi << 32) | (uint64_t)lo) >> 11;
   return (double)v * (1.0 / 9007199254740992.0);
 }
-// (0,1) with 32 random bits (exact in double).
-__host__ __device__ __forceinline__ double u32d(uint32_t w) {
-  return ((double)w + 0.5) * (1.0 / 4294967296.0);
-}
 // Unbiased-to-2^-64 integer in [0, n).
 __host__ __device__ __forceinline__ uint32_t below64(uint32_t hi, uint32_t lo, uint32_t n) {
   uint64_t v = ((uint64_t)hi << 32) | (uint64_t)lo;
@@ -89,28 +84,8 @@ __host__ __device__ __forceinline__ uint32_t below64(uint32_t hi, uint32_t lo, u
 }
 
 #ifdef __CUDACC__
-// Two standard normals from two 32-bit words (Box-Muller in fp32: the jitter they feed
+// Two standard normals from 12 + 12 random bits (Box-Muller in fp32: the jitter they feed
 // is scaled by epsilon ~ 1e-12, so fp32 shape accuracy is ample).
-__device__ __forceinline__ void normal2(uint32_t a, uint32_t b, float& n0, float& n1) {
-  float u1 = ((float)(a >> 8) + 1.0f) * (1.0f / 16777216.0f);  // (0,1]
-  float u2 = (float)(b >> 8) * (1.0f / 16777216.0f);           // [0,1)
-  float r = sqrtf(-2.0f * __logf(u1));
-  float s, c;
-  __sincosf(6.283185307179586f * u2, &s, &c);
-  n0 = r * c;
-  n1 = r * s;
-}
-// Same from one word (16 + 16 bits).
-__device__ __forceinline__ void normal2_16(uint32_t w, float& n0, float& n1) {
-  float u1 = ((float)(w & 0xFFFFu) + 1.0f) * (1.0f / 65536.0f);  // (0,1]
-  float u2 = (float)(w >> 16) * (1.0f / 65536.0f);               // [0,1)
-  float r = sqrtf(-2.0f * __logf(u1));
-  float s, c;
-  __sincosf(6.283185307179586f * u2, &s, &c);
-  n0 = r * c;
-  n1 = r * s;
-}
-// Same from 12 + 12 bits.
 __device__ __forceinline__ void normal2_12(uint32_t b1, uint32_t b2, float& n0, float& n1) {
   float u1 = ((float)b1 + 1.0f) * (1.0f / 4096.0f);   // (0,1]
   float u2 = (float)b2 * (1.0f / 4096.0f);            // [0,1)

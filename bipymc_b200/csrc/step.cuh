@@ -306,18 +306,19 @@ __device__ __forceinline__ double accept_uniform(const PhaseArgs& a, int c) {
   return accept_uniform<REPLAY>(a, a.rng, c, c);
 }
 
-// BPM_ZEN_ONE = 1: the three per-dimension draws of a 4-dim block -- crossover-mask uniform z (dream.py:52),
-// box jitter e (dream.py:83) and jitter normal n (dream.py:84) -- come from ONE Philox call instead of two.
+// The three per-dimension draws of a 4-dim block -- crossover-mask uniform z (dream.py:52), box jitter e
+// (dream.py:83) and jitter normal n (dream.py:84) -- come from ONE Philox call (purpose RNG_ZEN, slot b).
 // Word k of the call belongs to dim 4b + k:  bits 0-11 z on a 4096-point grid, bits 12-19 e on a 256-point
 // grid, bits 20-31 twelve bits towards a Box-Muller pair (words 0,1 -> n0,n1; words 2,3 -> n2,n3).
 // The mask compares z with CR in {1/n_cr ..}: a 2^-12 grid moves each crossover probability by < 2.5e-4;
 // e only randomises gamma by +-1 %; n has sd epsilon ~ 1e-12.  A chain-step of the fused kernel is bound by
 // its instruction count, and a Philox call is ~70 of ~850 (profiles/r2c_*).
-// Measured (profiles/r2d_*): 125.7 -> 118.0 us per launch of the fused 100-D kernel; default on.  BPM_ZEN_ONE = 0
-// restores round 1's two calls (32-bit z, 16-bit e, 16 + 16-bit Box-Muller).
-#ifndef BPM_ZEN_ONE
-#define BPM_ZEN_ONE 1
-#endif
+// Measured (profiles/r2d_*): 125.7 -> 118.0 us per launch of the fused 100-D kernel against two calls per
+// block (32-bit z, 16-bit e, 16 + 16-bit Box-Muller).
+__device__ __forceinline__ void zen_z4(const Philox4& q, double z[4]) {
+  z[0] = ((double)(q.x & 0xFFFu) + 0.5) * (1.0 / 4096.0); z[1] = ((double)(q.y & 0xFFFu) + 0.5) * (1.0 / 4096.0);
+  z[2] = ((double)(q.z & 0xFFFu) + 0.5) * (1.0 / 4096.0); z[3] = ((double)(q.w & 0xFFFu) + 0.5) * (1.0 / 4096.0);
+}
 __device__ __forceinline__ uint32_t zen_mask4(const Philox4& q, uint32_t th12) {
   return ((q.x & 0xFFFu) <= th12 ? 1u : 0u) | ((q.y & 0xFFFu) <= th12 ? 2u : 0u) |
          ((q.z & 0xFFFu) <= th12 ? 4u : 0u) | ((q.w & 0xFFFu) <= th12 ? 8u : 0u);
@@ -359,14 +360,7 @@ __device__ __forceinline__ void z4(const PhaseArgs& a, const RngCtx& rng, int c,
       z[t] = i < a.d ? a.rp.z[(size_t)c * a.d + i] : 2.0;
     }
   } else {
-#if BPM_ZEN_ONE
-    Philox4 q = draw4(rng, (uint32_t)j, RNG_ZEN, (uint32_t)b);
-    z[0] = ((double)(q.x & 0xFFFu) + 0.5) * (1.0 / 4096.0); z[1] = ((double)(q.y & 0xFFFu) + 0.5) * (1.0 / 4096.0);
-    z[2] = ((double)(q.z & 0xFFFu) + 0.5) * (1.0 / 4096.0); z[3] = ((double)(q.w & 0xFFFu) + 0.5) * (1.0 / 4096.0);
-#else
-    Philox4 q = draw4(rng, (uint32_t)j, RNG_Z, (uint32_t)b);
-    z[0] = u32d(q.x); z[1] = u32d(q.y); z[2] = u32d(q.z); z[3] = u32d(q.w);
-#endif
+    zen_z4(draw4(rng, (uint32_t)j, RNG_ZEN, (uint32_t)b), z);
   }
 }
 template <bool REPLAY>
@@ -374,9 +368,7 @@ __device__ __forceinline__ void z4(const PhaseArgs& a, int c, int b, double z[4]
   z4<REPLAY>(a, a.rng, c, c, b, z);
 }
 // Box jitter e (dream.py:83, var_box) and Gaussian jitter n (demc.py:182 / dream.py:84,
-// var_ball) for dims 4b .. 4b+3 from ONE Philox call: words x,y give four 16-bit
-// uniforms for e (a +-u_eps box on a 65536-point grid), words z,w two Box-Muller pairs for
-// n (sd epsilon ~ 1e-12: its shape only has to be Gaussian to fp32 accuracy).
+// var_ball) for dims 4b .. 4b+3, from the block's RNG_ZEN call (zen_en4).
 template <bool REPLAY>
 __device__ __forceinline__ void en4(const PhaseArgs& a, const RngCtx& rng, int c, int j, int b, double e[4],
                                     double n[4]) {
@@ -390,32 +382,7 @@ __device__ __forceinline__ void en4(const PhaseArgs& a, const RngCtx& rng, int c
   } else {
     e[0] = e[1] = e[2] = e[3] = 0.0;  // var_box returns 0. and draws nothing (util.py:24-28)
     n[0] = n[1] = n[2] = n[3] = 0.0;  // var_ball returns 0. and draws nothing (util.py:11-16)
-#if BPM_ZEN_ONE
     if (a.u_eps > 0.0 || a.eps > 0.0) zen_en4(a, draw4(rng, (uint32_t)j, RNG_ZEN, (uint32_t)b), e, n);
-    return;
-#endif
-    if (a.u_eps > 0.0 || a.eps > 0.0) {
-      const Philox4 q = draw4(rng, (uint32_t)j, RNG_EN, (uint32_t)b);
-      if (a.u_eps > 0.0) {
-        const double lo = -a.u_eps, w = __dsub_rn(a.u_eps, lo);  // numpy: low + (high-low)*u
-        // u = (h + 0.5) / 65536 for a 16-bit h; (2h + 1) * (w * 2^-17) is the same product
-        // (power-of-two scaling commutes with rounding) in one conversion + one multiply
-        const double w17 = w * (1.0 / 131072.0);
-        e[0] = __dadd_rn(lo, __dmul_rn(w17, (double)(int)(2u * (q.x & 0xFFFFu) + 1u)));
-        e[1] = __dadd_rn(lo, __dmul_rn(w17, (double)(int)(2u * (q.x >> 16) + 1u)));
-        e[2] = __dadd_rn(lo, __dmul_rn(w17, (double)(int)(2u * (q.y & 0xFFFFu) + 1u)));
-        e[3] = __dadd_rn(lo, __dmul_rn(w17, (double)(int)(2u * (q.y >> 16) + 1u)));
-      }
-      if (a.eps > 0.0) {
-        float f0, f1, f2, f3;
-        normal2_16(q.z, f0, f1);
-        normal2_16(q.w, f2, f3);
-        n[0] = __dmul_rn(a.eps, (double)f0);
-        n[1] = __dmul_rn(a.eps, (double)f1);
-        n[2] = __dmul_rn(a.eps, (double)f2);
-        n[3] = __dmul_rn(a.eps, (double)f3);
-      }
-    }
   }
 }
 

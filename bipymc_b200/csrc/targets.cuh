@@ -65,18 +65,10 @@ __device__ __forceinline__ double gauss_finish(double c0, double maha, int log_o
 //   lnL = -0.5 * sum_i [ r_i^2 * inv_i - log(inv_i) ],  inv_i = 1 / (yerr_i^2 + model_i^2 e^{2 lnf}),  r_i = y_i - model_i
 // Reference form, one IEEE division and one logarithm per data point (~120 instructions per term, 6 000 of the
 // 7 300 instructions of a whole line-fit chain-step: profiles/r2/r2x_fused_small_linefit_ncu_summary.txt).
-// Kept as the exact fallback and for the A/B (-DBPM_LINEFIT_GROUPED=0).  Measured alternatives of the same form
-// (profiles/r2/r2r_secondary.txt, r2s_*): four interleaved partial sums 76 us per generation of 10^5 chains,
-// this form 73 us, four LANES per chain 86 us.
-#ifndef BPM_LINEFIT_GROUPED
-#define BPM_LINEFIT_GROUPED 1
-#endif
-#if BPM_LINEFIT_GROUPED
-#define BPM_LINEFIT_EXACT_ATTR __noinline__          // the rare fallback stays out of the hot kernels' bodies
-#else
-#define BPM_LINEFIT_EXACT_ATTR __forceinline__
-#endif
-__device__ BPM_LINEFIT_EXACT_ATTR double linefit_lnl_per_term(const double* x, const double* y, const double* yerr,
+// Kept as the exact fallback of linefit_lnl, out of line so the rare case stays out of the hot kernels' bodies.
+// Measured alternatives of the same form (profiles/r2/r2r_secondary.txt, r2s_*): four interleaved partial sums
+// 76 us per generation of 10^5 chains, this form 73 us, four LANES per chain 86 us.
+__device__ __noinline__ double linefit_lnl_per_term(const double* x, const double* y, const double* yerr,
                                                     int M, double m, double b, double e2) {
   double s = 0.0;
 #pragma unroll 5
@@ -90,7 +82,7 @@ __device__ BPM_LINEFIT_EXACT_ATTR double linefit_lnl_per_term(const double* x, c
   return 0.0 + -0.5 * s;
 }
 
-// Default: five data points share ONE reciprocal and ONE logarithm.  With P = den_1 ... den_5 (den_i and r_i
+// linefit_lnl: five data points share ONE reciprocal and ONE logarithm.  With P = den_1 ... den_5 (den_i and r_i
 // computed exactly as above): inv_i = (1 / P) * prod_{j != i} den_j from prefix / suffix products, and
 // -sum log(inv_i) = log(P).  15 multiplications + 1 reciprocal + 1 logarithm per group instead of 5 divisions +
 // 5 logarithms.  inv_i carries ~3 ulp instead of 0.5, log(P) the same absolute error as one of the five
@@ -109,7 +101,6 @@ __device__ __forceinline__ double linefit_lnl(const double* x, const double* y, 
                                               int M, double m, double b, double lnf) {
   if (!(-5.0 < m && m < 0.5 && 0.0 < b && b < 10.0 && -10.0 < lnf && lnf < 1.0)) return -INFINITY;
   const double e2 = exp(__dmul_rn(2.0, lnf));
-#if BPM_LINEFIT_GROUPED
   double s = 0.0, lg = 0.0;
   bool ok = true;
   // one group of five points: adds sum r_i^2 inv_i to s, returns P = den_1 ... den_5
@@ -153,9 +144,6 @@ __device__ __forceinline__ double linefit_lnl(const double* x, const double* y, 
     lg -= log(inv);
   }
   return 0.0 + -0.5 * (s + lg);
-#else
-  return linefit_lnl_per_term(x, y, yerr, M, m, b, e2);
-#endif
 }
 
 // Exponential-relaxation fit, examples/ex_exp_fit.py:38-121.

@@ -337,9 +337,10 @@ int bpm_host_entry_restart(bpm_handle h);
  * Collective: every rank calls it with the same k_gen0 / n_gen.  Synchronous. */
 int bpm_generations_host_sharded(bpm_handle h, bpm_state* st, double* X_host, double* lnl_host,
                                  int64_t k_gen0, int32_t n_gen, bpm_stream stream);
-/* When both host arrays are pinned (device-mapped) memory, bpm_generations_host writes back only
- * the rows of chains that moved (the device stores them straight into the host arrays; rows of
- * chains that did not move are already correct there).  Bytes the last call moved device->host. */
+/* Bytes the last host-entry call moved device->host.  When both host arrays are pinned (device-mapped)
+ * memory, bpm_generations_host writes back only the accepted rows, which the phase kernels store straight
+ * into the host array (rows of chains that did not move are already correct there), plus one copy of the
+ * cached likelihoods; with pageable arrays it copies the whole population and the likelihoods back. */
 int bpm_last_d2h_bytes(bpm_handle h, uint64_t* bytes);
 
 /* Materialise a pending row (bpm_state.pending): writes history row hist_len - 1 from X and folds it

@@ -435,7 +435,6 @@ def test_host_buffer_entry_equals_device_resident_generations(pinned, adapt):
     with crossover adaptation on, the same p_cr: the entry keeps the chains' running moments on the
     device between calls (dream.py:119-140 needs np.std of every chain's history)."""
     import ctypes as C
-    import os
     import torch
     from bipymc_b200 import DreamMpi, targets, _lib
     N, d, G = 4096, 100, 7
@@ -451,7 +450,6 @@ def test_host_buffer_entry_equals_device_resident_generations(pinned, adapt):
     if pinned:
         Xh, Lh = Xh.pin_memory(), Lh.pin_memory()
     Xh.copy_(b._X.cpu()); Lh.copy_(b._lnl.cpu())
-    host_peer = pinned and os.environ.get("BIPYMC_B200_HOST_PEER", "1") != "0"
     moved = 0
     for g in range(G):
         before = Xh.clone()
@@ -460,10 +458,8 @@ def test_host_buffer_entry_equals_device_resident_generations(pinned, adapt):
         _lib.check(b._libh.bpm_last_d2h_bytes(b._handle, C.byref(nb)))
         rows = int((before != Xh).any(dim=1).sum())
         moved += rows
-        if host_peer:       # accepted rows stored from inside the kernels + one copy of the cached likelihoods
+        if pinned:       # accepted rows stored from inside the kernels + one copy of the cached likelihoods
             assert nb.value == rows * b._ld * 8 + N * 8 + 16
-        elif pinned:
-            assert nb.value == rows * (b._ld + 1) * 8 + 8
         else:
             assert nb.value == N * (b._ld + 1) * 8
     a.run_mcmc(N * (G + 1))
