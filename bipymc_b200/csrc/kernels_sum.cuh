@@ -1,5 +1,5 @@
 // Per-observation likelihoods summed across the whole GPU (BPM_TARGET_JIT_SUM).  Device code only: the
-// run-time compiled translation unit of a sum-form source (engine.cu: jit_sum_translation_unit) is the only one
+// run-time compiled translation unit of a sum-form source (engine.cu: kJitSum) is the only one
 // that includes this header.  It places, before this header, the user's
 //   __device__ double ln_like_term(const double* theta, const double* row);   // one observation
 //   __device__ double ln_prior(const double* theta);                          // when BPM_HAS_PRIOR is 1

@@ -317,15 +317,29 @@ class CudaLikelihood(object):
             raise ValueError("source must be a str of CUDA C++")
         if isinstance(dim, bool) or int(dim) != dim or int(dim) < 1:
             raise ValueError("dim must be an integer >= 1")
-        data = np.zeros(0) if data is None else np.asarray(data, dtype=np.float64)
-        if data.ndim != 1:
-            raise ValueError("data must be 1-D (concatenate the arrays the source reads)")
+        data = self._shaped(data)
         if not np.all(np.isfinite(data)):
             raise ValueError("data must be finite")
         self.source = source
         self.dim = int(dim)
         self.data = np.ascontiguousarray(data)
         self.fmad = bool(fmad)
+
+    @staticmethod
+    def _shaped(data):
+        """``data`` as the float64 array of the shape this kind takes, or ValueError."""
+        data = np.zeros(0) if data is None else np.asarray(data, dtype=np.float64)
+        if data.ndim != 1:
+            raise ValueError("data must be 1-D (concatenate the arrays the source reads)")
+        return data
+
+    def _compile_call(self, lib):
+        """This kind's C-ABI compile function and its arguments before ``flags``."""
+        return lib.bpm_jit_compile, (self.source.encode(), self.dim, self.data.size)
+
+    def _attach_call(self, lib, handle):
+        """This kind's C-ABI attach function and its arguments before ``flags``."""
+        return lib.bpm_set_jit_target, (handle, self.source.encode(), _lib.dptr(self.data), self.data.size)
 
     @property
     def _flags(self):
@@ -334,7 +348,7 @@ class CudaLikelihood(object):
     def _call(self, fn, *head):
         log = C.create_string_buffer(self._LOG_BYTES)
         cached = C.c_int32(0)
-        rc = fn(*(head + (C.byref(cached), log, self._LOG_BYTES)))
+        rc = fn(*(head + (self._flags, C.byref(cached), log, self._LOG_BYTES)))
         if rc != 0:
             msg = _lib.load().bpm_last_error().decode()
             text = log.value.decode(errors="replace")
@@ -346,13 +360,13 @@ class CudaLikelihood(object):
     def compile(self):
         """Compile for sm_100a (no device needed).  Returns True when the cubin came from the
         process cache; raises CudaCompileError with the NVRTC log."""
-        lib = _lib.load()
-        return self._call(lib.bpm_jit_compile, self.source.encode(), self.dim, self.data.size, self._flags)
+        fn, args = self._compile_call(_lib.load())
+        return self._call(fn, *args)
 
     def _attach(self, lib, handle):
         """Compile (or take the cached cubin), load it on the handle's device and copy the data."""
-        return self._call(lib.bpm_set_jit_target, handle, self.source.encode(), _lib.dptr(self.data),
-                          self.data.size, self._flags)
+        fn, args = self._attach_call(lib, handle)
+        return self._call(fn, *args)
 
 
 class CudaLikelihoodSet(CudaLikelihood):
@@ -368,38 +382,29 @@ class CudaLikelihoodSet(CudaLikelihood):
     cache key, and the kernels are compiled in a translation unit of their own."""
 
     def __init__(self, source, dim, data, fmad=True):
-        if not isinstance(source, str):
-            raise ValueError("source must be a str of CUDA C++")
-        if isinstance(dim, bool) or int(dim) != dim or int(dim) < 1:
-            raise ValueError("dim must be an integer >= 1")
+        super(CudaLikelihoodSet, self).__init__(source, dim, data, fmad)
+
+    @staticmethod
+    def _shaped(data):
         data = np.asarray(data, dtype=np.float64)
         if data.ndim != 2 or data.shape[0] < 1 or data.shape[1] < 1:
             raise ValueError("data must have shape (P, n_data) with P >= 1 and n_data >= 1: one row per problem")
         if data.shape[0] >= 2 ** 31:
             raise ValueError("data must have fewer than 2^31 rows")
-        if not np.all(np.isfinite(data)):
-            raise ValueError("data must be finite")
-        self.source = source
-        self.dim = int(dim)
-        self.data = np.ascontiguousarray(data)
-        self.fmad = bool(fmad)
+        return data
+
+    def _compile_call(self, lib):
+        P, nd = self.data.shape
+        return lib.bpm_jit_compile_problems, (self.source.encode(), self.dim, nd, P)
+
+    def _attach_call(self, lib, handle):
+        # the handle must be a multi-problem handle with P problems (bpm_set_problems), which gives P
+        return lib.bpm_set_jit_problems_target, (handle, self.source.encode(), _lib.dptr(self.data),
+                                                 self.data.shape[1])
 
     @property
     def n_problems(self):
         return int(self.data.shape[0])
-
-    def compile(self):
-        """Compile for sm_100a (no device needed).  Returns True when the cubin came from the
-        process cache; raises CudaCompileError with the NVRTC log."""
-        lib = _lib.load()
-        P, nd = self.data.shape
-        return self._call(lib.bpm_jit_compile_problems, self.source.encode(), self.dim, nd, P, self._flags)
-
-    def _attach(self, lib, handle):
-        """Compile (or take the cached cubin), load it on the handle's device and copy the data (the handle
-        must be a multi-problem handle with P problems: bpm_set_problems)."""
-        return self._call(lib.bpm_set_jit_problems_target, handle, self.source.encode(), _lib.dptr(self.data),
-                          self.data.shape[1], self._flags)
 
 
 def problem_seeds(seed, n_problems):
@@ -452,10 +457,11 @@ class CudaSumLikelihood(CudaLikelihood):
     all SMs, between the proposal and accept kernels at every d.  Pass it as ``ln_like_cuda=``."""
 
     def __init__(self, source, dim, data, prior=False, fmad=True):
-        if not isinstance(source, str):
-            raise ValueError("source must be a str of CUDA C++")
-        if isinstance(dim, bool) or int(dim) != dim or int(dim) < 1:
-            raise ValueError("dim must be an integer >= 1")
+        super(CudaSumLikelihood, self).__init__(source, dim, data, fmad)
+        self.prior = bool(prior)
+
+    @staticmethod
+    def _shaped(data):
         data = np.asarray(data, dtype=np.float64)
         if data.ndim == 1:
             data = data.reshape(-1, 1)
@@ -463,27 +469,16 @@ class CudaSumLikelihood(CudaLikelihood):
             raise ValueError("data must have shape (M, k) with M >= 1 and k >= 1 (or be 1-D with M >= 1)")
         if data.shape[0] >= 2 ** 31:
             raise ValueError("data must have fewer than 2^31 rows")
-        if not np.all(np.isfinite(data)):
-            raise ValueError("data must be finite")
-        self.source = source
-        self.dim = int(dim)
-        self.data = np.ascontiguousarray(data)
-        self.prior = bool(prior)
-        self.fmad = bool(fmad)
+        return data
+
+    def _compile_call(self, lib):
+        M, k = self.data.shape
+        return lib.bpm_jit_compile_sum, (self.source.encode(), self.dim, M, k)
+
+    def _attach_call(self, lib, handle):
+        M, k = self.data.shape
+        return lib.bpm_set_jit_sum_target, (handle, self.source.encode(), _lib.dptr(self.data), M, k)
 
     @property
     def _flags(self):
         return (1 if self.fmad else 0) | (2 if self.prior else 0)
-
-    def compile(self):
-        """Compile for sm_100a (no device needed).  Returns True when the cubin came from the
-        process cache; raises CudaCompileError with the NVRTC log."""
-        lib = _lib.load()
-        M, k = self.data.shape
-        return self._call(lib.bpm_jit_compile_sum, self.source.encode(), self.dim, M, k, self._flags)
-
-    def _attach(self, lib, handle):
-        """Compile (or take the cached cubin), load it on the handle's device and copy the data."""
-        M, k = self.data.shape
-        return self._call(lib.bpm_set_jit_sum_target, handle, self.source.encode(), _lib.dptr(self.data), M, k,
-                          self._flags)
