@@ -1,6 +1,6 @@
 // Per-observation likelihoods summed across the whole GPU (BPM_TARGET_JIT_SUM).  Device code only: the
-// run-time compiled translation unit of a sum-form source (engine.cu: kJitSum) is the only one
-// that includes this header.  It places, before this header, the user's
+// run-time compiled translation units of a sum-form source (engine.cu: kJitSum, kJitSumProblems) are the only
+// ones that compile its kernels.  Each places, before this header, the user's
 //   __device__ double ln_like_term(const double* theta, const double* row);   // one observation
 //   __device__ double ln_prior(const double* theta);                          // when BPM_HAS_PRIOR is 1
 // and defines BPM_DIM, BPM_NROWS (M), BPM_ROWLEN (k) and BPM_HAS_PRIOR.  data is the row-major [M][k] array.
@@ -240,3 +240,68 @@ __global__ void __launch_bounds__(128) lnl_sum_finish_kernel(const double* __res
 #endif  // BPM_JIT_SUM
 
 }  // namespace bpm
+
+#if defined(BPM_JIT_SUM) && defined(BPM_JIT_PROBLEMS)
+#include "cr_reduce.cuh"     // cr_update_problems_kernel
+namespace bpm {
+// Multi-problem handles (engine.cu: kJitSumProblems): data is [BPM_NPROBLEMS][BPM_NROWS][BPM_ROWLEN], and rows
+// [g rpp, (g + 1) rpp) of P belong to problem g.  The body of lnl_sum_kernel on a tile that never straddles two
+// problems: block x holds tile x % tpp (tpp = ceil(rpp / tile)) of problem g = x / tpp and reads problem g's rows, so
+// every sum is added in the order of one problem of M rows.  A phase's idle slot (n odd: the last of the smaller
+// half) is evaluated like the others on whatever proposal row it holds; accept never reads its result.
+// grid (P tpp, n_groups), kSumThreads threads; dynamic shared memory sum_smem_bytes(tile).
+__global__ void __launch_bounds__(kSumThreads) lnl_sum_problems_kernel(const double* __restrict__ P, int n, int ld,
+                                                                       int rpp, int tpp,
+                                                                       const double* __restrict__ data, int tile,
+                                                                       int log2_group, int n_groups,
+                                                                       double* __restrict__ ws,
+                                                                       double* __restrict__ out) {
+  extern __shared__ __align__(16) double sm_sum[];
+  const int g = blockIdx.x / tpp;
+  const int t0 = (blockIdx.x - g * tpp) * tile;         // first row of the tile inside problem g
+  const int c0 = g * rpp + t0;
+  const int nt = min(tile, rpp - t0);
+  const double* __restrict__ pdata = data + (int64_t)g * kSumRows * kSumK;
+  double* stk = sm_sum;                                  // [tile][kSumMaxDepth]
+  double* prior = stk + tile * kSumMaxDepth;             // [tile]
+  double* srows = prior + tile;                          // [k][kSumStageRows] when staged
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int64_t G = (int64_t)1 << log2_group;
+  const int64_t q0 = (int64_t)blockIdx.y * G;
+  for (int ci = threadIdx.x; ci < nt; ci += kSumThreads) {
+    SumTheta th;
+    th.load(P + (size_t)(c0 + ci) * ld);
+    prior[ci] = sum_prior(th.ptr());
+  }
+  __syncthreads();
+  const int64_t m = min(G, kSumChunks - q0);
+  const int sc = G < kSumStageChunks ? (int)G : kSumStageChunks;
+  for (int64_t s0 = 0; s0 < m; s0 += sc) {
+    const int64_t r0 = (q0 + s0) * kSumChunk;
+    const int ns = (int)min((int64_t)sc, m - s0);
+    if constexpr (kSumStaged) {
+      __syncthreads();
+      const int64_t nr = min((int64_t)ns * kSumChunk, kSumRows - r0);
+      for (int64_t i = threadIdx.x; i < nr * kSumK; i += kSumThreads) {
+        const int64_t r = i / kSumK;
+        srows[(i - r * kSumK) * kSumStageRows + r] = pdata[r0 * kSumK + i];
+      }
+      __syncthreads();
+    }
+    for (int ci = warp; ci < nt; ci += kSumThreads / 32) {
+      if (prior[ci] == -INFINITY) continue;
+      double* cs = stk + ci * kSumMaxDepth;
+      SumTheta th;
+      th.load(P + (size_t)(c0 + ci) * ld);
+      for (int s = 0; s < ns; ++s) sum_push(cs, s0 + s, sum_chunk(th.ptr(), q0 + s0 + s, srows, r0, pdata, lane), lane);
+    }
+  }
+  __syncthreads();
+  for (int ci = threadIdx.x; ci < nt; ci += kSumThreads) {
+    const double S = sum_flush(stk + ci * kSumMaxDepth, m, log2_group);
+    if (n_groups == 1) out[c0 + ci] = sum_finish_value(prior[ci], S);
+    else ws[(size_t)blockIdx.y * n + c0 + ci] = S;
+  }
+}
+}  // namespace bpm
+#endif

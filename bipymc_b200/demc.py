@@ -33,6 +33,10 @@ Likelihood plug-ins, fastest first:
      exactly as a single-problem sampler with data row g and Philox key ``problem_seeds[g]`` would, and
      every pooled result (``acceptance_fraction``, ``param_est``, ``p_cr``, ``rhat`` ...) gets a leading
      axis P.  One rank only; ``subpop_k``, ``outlier_gen``, ``track_covariance`` and ``_replay`` are refused;
+  1e. ``ln_like_cuda=targets.CudaSumLikelihoodSet(source, dim, data[P, M, k], prior)``: the per-observation
+     form of 1c fitted to P datasets of M rows in ONE sampler, with the contract and refusals of 1d: problem g
+     runs exactly as a ``CudaSumLikelihood`` sampler on ``data[g]`` with key ``problem_seeds[g]`` would.
+     Each phase is propose + sum + accept at every dim; the sum kernel's tiles of chains stay inside one problem;
   2. ``ln_like_batched=f``: ``f(theta)`` takes a CUDA float64 tensor ``[n, dim]`` and
      returns ``[n]`` log-likelihoods (torch ops on the current stream);
   3. any scalar ``ln_like_fn(theta, **ln_kwargs) -> float`` exactly as in the reference
@@ -333,7 +337,7 @@ class DeMcMpi(object):
     """Parallel DE-MC (emcee-style a/b pools) on B200; mirrors bipymc/demc.py:10."""
     _algo = _lib.BPM_ALGO_DEMC
     _n_phases = 2
-    n_problems = 1           # > 1: a CudaLikelihoodSet of that many problems (n_chains chains each)
+    n_problems = 1           # > 1: a CudaLikelihoodSet / CudaSumLikelihoodSet of that many problems (n_chains each)
     _seed_keys = None        # Philox keys of the problems, once fixed
 
     def __init__(self, ln_like_fn, theta_0=None, varepsilon=1e-6, n_chains=8,
@@ -413,13 +417,15 @@ class DeMcMpi(object):
         return self.n_chains * self.n_problems
 
     def _check_problems(self, kwargs):
-        """A CudaLikelihoodSet makes this a multi-problem sampler; refuse what that mode does not offer."""
-        from .targets import CudaLikelihoodSet
+        """A CudaLikelihoodSet or CudaSumLikelihoodSet makes this a multi-problem sampler; refuse what that mode
+        does not offer."""
+        from .targets import CudaLikelihoodSet, CudaSumLikelihoodSet
         cuda = kwargs.get("ln_like_cuda", None)
         seed = kwargs.get("seed", None)
-        if not isinstance(cuda, CudaLikelihoodSet):
+        if not isinstance(cuda, (CudaLikelihoodSet, CudaSumLikelihoodSet)):
             if seed is not None and np.ndim(seed) != 0:
-                raise ValueError("a sequence of seeds (one per problem) needs ln_like_cuda=targets.CudaLikelihoodSet")
+                raise ValueError("a sequence of seeds (one per problem) needs ln_like_cuda=targets.CudaLikelihoodSet "
+                                 "or targets.CudaSumLikelihoodSet")
             return
         self._ln_like_cuda_set = cuda
         self.n_problems = cuda.n_problems
@@ -431,11 +437,11 @@ class DeMcMpi(object):
         elif int(kwargs.get("outlier_gen", 0)):
             why = "has no outlier_gen"
         elif kwargs.get("ln_like_batched", None) is not None:
-            why = "takes its likelihood from the CudaLikelihoodSet only (no ln_like_batched)"
+            why = "takes its likelihood from the %s only (no ln_like_batched)" % type(cuda).__name__
         elif kwargs.get("device_init", False):
             why = "draws its initial states on the host (no device_init)"
         if why:
-            raise ValueError("a multi-problem sampler (ln_like_cuda=CudaLikelihoodSet) " + why)
+            raise ValueError("a multi-problem sampler (ln_like_cuda=%s) " % type(cuda).__name__ + why)
         if seed is not None:
             from .targets import problem_seeds
             self._seed_keys = problem_seeds(seed, self.n_problems)

@@ -43,10 +43,10 @@ class DeMc(DeMcMpi):
         self._history_policy = proposal_kwargs.get("history", "full")
         self._ln_like_batched = proposal_kwargs.get("ln_like_batched", None)
         self._ln_like_cuda = proposal_kwargs.get("ln_like_cuda", None)
-        from .targets import CudaLikelihoodSet
-        if isinstance(self._ln_like_cuda, CudaLikelihoodSet):
-            raise NotImplementedError("serial DeMc does not run a CudaLikelihoodSet (several problems in one sampler): "
-                                      "use DeMcMpi or DreamMpi")
+        from .targets import CudaLikelihoodSet, CudaSumLikelihoodSet
+        if isinstance(self._ln_like_cuda, (CudaLikelihoodSet, CudaSumLikelihoodSet)):
+            raise NotImplementedError("serial DeMc does not run a %s (several problems in one sampler): "
+                                      "use DeMcMpi or DreamMpi" % type(self._ln_like_cuda).__name__)
         self._device_index = proposal_kwargs.get("device", None)
         self._fused = False                                         # the sweep uses the split launches
         self._chunk_bytes = int(proposal_kwargs.get("history_chunk_bytes", 1 << 30))

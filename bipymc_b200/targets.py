@@ -12,7 +12,8 @@ Mirrors the reference's test-target classes (same constructor arguments, same ``
 and ``CudaLikelihood``: any other model as CUDA C++ source, compiled at run time into the same
 kernels (``ln_like_cuda=`` of the samplers); ``CudaSumLikelihood``: a model that is a sum over
 observations, one CUDA C++ term per observation, summed across the whole GPU; ``CudaLikelihoodSet``: one
-``ln_like`` source fitted to many datasets at once, each an independent problem of the same sampler.
+``ln_like`` source fitted to many datasets at once, each an independent problem of the same sampler;
+``CudaSumLikelihoodSet``: the same for a per-observation source.
 
 ``ln_like`` stays a scalar host function, so the objects remain valid ``ln_like_fn``
 arguments everywhere; when a sampler of this package receives ``obj.ln_like`` it
@@ -482,3 +483,44 @@ class CudaSumLikelihood(CudaLikelihood):
     @property
     def _flags(self):
         return (1 if self.fmad else 0) | (2 if self.prior else 0)
+
+
+class CudaSumLikelihoodSet(CudaSumLikelihood):
+    """One per-observation CUDA likelihood fitted to P datasets at once: P independent problems in one sampler.
+
+    ``source`` and ``prior`` are those of ``CudaSumLikelihood``; ``data`` is a finite float64 array of shape
+    ``(P, M, k)`` (a 2-D ``(P, M)`` array is ``(P, M, 1)``): problem g's sum runs over its own M rows
+    ``data[g]``.  ``BPM_NROWS`` is M (the rows of ONE problem), ``BPM_ROWLEN`` k and ``BPM_NPROBLEMS`` P.
+    Pass it as ``ln_like_cuda=`` to ``DreamMpi`` / ``DeMcMpi``: as with ``CudaLikelihoodSet``, ``n_chains``
+    then counts the chains of one problem, and problem g steps exactly -- bit for bit -- as a single-problem
+    sampler with ``n_chains`` chains, ``CudaSumLikelihood(source, dim, data[g], prior, fmad)`` and Philox key
+    ``sampler.problem_seeds[g]`` would, while all P problems run in the same kernel launches.  Each problem's
+    sum is added in the order of ``CudaSumLikelihood`` for M rows and is split over the GPU in tiles of chains
+    that never straddle two problems: the form for many datasets of many observations and few chains each.
+    P, M, k and ``prior`` are part of the cache key, and the kernels are compiled in a translation unit of their
+    own."""
+
+    @staticmethod
+    def _shaped(data):
+        data = np.asarray(data, dtype=np.float64)
+        if data.ndim == 2:
+            data = data.reshape(data.shape + (1,))
+        if data.ndim != 3 or min(data.shape) < 1:
+            raise ValueError("data must have shape (P, M, k) with P, M, k >= 1 (or (P, M) with k = 1), not %s"
+                             % (data.shape,))
+        if data.shape[0] >= 2 ** 31 or data.shape[1] >= 2 ** 31:
+            raise ValueError("data shape %s: P and M must each be below 2^31" % (data.shape,))
+        return data
+
+    def _compile_call(self, lib):
+        P, M, k = self.data.shape
+        return lib.bpm_jit_compile_sum_problems, (self.source.encode(), self.dim, M, k, P)
+
+    def _attach_call(self, lib, handle):
+        # the handle must be a multi-problem handle with P problems (bpm_set_problems), which gives P
+        _, M, k = self.data.shape
+        return lib.bpm_set_jit_sum_problems_target, (handle, self.source.encode(), _lib.dptr(self.data), M, k)
+
+    @property
+    def n_problems(self):
+        return int(self.data.shape[0])

@@ -190,7 +190,8 @@ int bpm_set_jit_sum_target(bpm_handle h, const char* source, const double* data,
  * whatever P is.
  * bpm_set_problems is called right after bpm_create, on an unsharded DE-MC or DREAM handle with
  * n_chains % n_problems == 0 and n = n_chains / n_problems >= 4; keys[n_problems] (HOST) are the problems'
- * Philox keys.  The likelihood is then set with bpm_set_jit_problems_target: the ln_like source of
+ * Philox keys.  The likelihood is then set with bpm_set_jit_problems_target (or, per observation,
+ * bpm_set_jit_sum_problems_target below): the ln_like source of
  * bpm_jit_compile, with data the row-major [P][n_data] HOST array (n_data >= 1): problem g's ln_like gets
  * data + g n_data, and BPM_NDATA is n_data (BPM_NPROBLEMS is P).  P and n_data are part of the cache key.
  * A multi-problem handle offers bpm_step_generations, bpm_flush, bpm_moments_from_history, bpm_eval_lnl
@@ -203,6 +204,17 @@ int bpm_jit_compile_problems(const char* source, int32_t dim, int64_t n_data, in
                              int32_t* from_cache, char* log, int64_t log_cap);
 int bpm_set_jit_problems_target(bpm_handle h, const char* source, const double* data, int64_t n_data, int32_t flags,
                                 int32_t* from_cache, char* log, int64_t log_cap);
+/* The per-observation form on a multi-problem handle (target BPM_TARGET_JIT_SUM): the ln_like_term source and
+ * flags of bpm_jit_compile_sum, with data the row-major [P][n_rows][row_len] HOST array; problem g's sum runs over
+ * its own n_rows rows (data + g n_rows row_len), in the order bpm_jit_compile_sum gives for n_rows rows, so it
+ * gets the bits a single-problem handle holding problem g's rows would.  BPM_NROWS is n_rows (the rows of ONE
+ * problem), BPM_ROWLEN row_len, BPM_NPROBLEMS P; P, n_rows, row_len and the prior bit are part of the cache key.
+ * A tile of chains never straddles two problems, and the launches per generation do not depend on P: at every
+ * dim each phase is propose + likelihood + accept. */
+int bpm_jit_compile_sum_problems(const char* source, int32_t dim, int64_t n_rows, int32_t row_len, int32_t n_problems,
+                                 int32_t flags, int32_t* from_cache, char* log, int64_t log_cap);
+int bpm_set_jit_sum_problems_target(bpm_handle h, const char* source, const double* data, int64_t n_rows,
+                                    int32_t row_len, int32_t flags, int32_t* from_cache, char* log, int64_t log_cap);
 int bpm_get_problem_cr_state(bpm_handle h, double* p_cr, double* dm, double* cnt);
 int bpm_set_problem_cr_state(bpm_handle h, const double* p_cr, const double* dm, const double* cnt);
 int bpm_get_problem_counters(bpm_handle h, uint64_t* acc, uint64_t* rej);
