@@ -76,6 +76,11 @@ SIGNATURES = {
                                                C.POINTER(C.c_int32), C.c_char_p, C.c_int64]),
     "bpm_set_jit_sum_problems_target": (C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(C.c_double), C.c_int64,
                                                   C.c_int32, C.c_int32, C.POINTER(C.c_int32), C.c_char_p, C.c_int64]),
+    "bpm_jit_compile_sum_ragged": (C.c_int, [C.c_char_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                             C.POINTER(C.c_int32), C.c_char_p, C.c_int64]),
+    "bpm_set_jit_sum_ragged_target": (C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(C.c_double),
+                                                C.POINTER(C.c_int64), C.c_int32, C.c_int32, C.POINTER(C.c_int32),
+                                                C.c_char_p, C.c_int64]),
     "bpm_get_problem_cr_state": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_double),
                                            C.POINTER(C.c_double)]),
     "bpm_set_problem_cr_state": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_double),

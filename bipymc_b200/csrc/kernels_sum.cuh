@@ -1,9 +1,11 @@
 // Per-observation likelihoods summed across the whole GPU (BPM_TARGET_JIT_SUM).  Device code only: the
-// run-time compiled translation units of a sum-form source (engine.cu: kJitSum, kJitSumProblems) are the only
-// ones that compile its kernels.  Each places, before this header, the user's
+// run-time compiled translation units of a sum-form source (engine.cu: kJitSum, kJitSumProblems, kJitSumRagged)
+// are the only ones that compile its kernels.  Each places, before this header, the user's
 //   __device__ double ln_like_term(const double* theta, const double* row);   // one observation
 //   __device__ double ln_prior(const double* theta);                          // when BPM_HAS_PRIOR is 1
 // and defines BPM_DIM, BPM_NROWS (M), BPM_ROWLEN (k) and BPM_HAS_PRIOR.  data is the row-major [M][k] array.
+// The ragged kind (BPM_JIT_SUM_RAGGED instead of BPM_JIT_SUM) has no BPM_NROWS: its problems' M differ and are
+// read at run time.
 //
 // Summation order -- a function of M alone (never of the number of chains, the batch, the launch shape or the
 // number of GPUs), so a given theta always gets the same bits:
@@ -45,10 +47,8 @@ __host__ __device__ constexpr size_t sum_smem_bytes(int tile, int k) {
                            (k <= kSumSmemRowLen ? (size_t)k * sum_stage_chunks(k) * kSumChunk : 0));
 }
 
-#ifdef BPM_JIT_SUM
-constexpr int64_t kSumRows = BPM_NROWS;
+#if defined(BPM_JIT_SUM) || defined(BPM_JIT_SUM_RAGGED)
 constexpr int kSumK = BPM_ROWLEN;
-constexpr int64_t kSumChunks = (kSumRows + kSumChunk - 1) / kSumChunk;
 constexpr bool kSumStaged = kSumK <= kSumSmemRowLen;
 constexpr int kSumStageChunks = sum_stage_chunks(kSumK);
 constexpr int kSumStageRows = kSumStageChunks * kSumChunk;
@@ -88,10 +88,11 @@ __device__ __forceinline__ double sum_finish_value(double prior, double S) {
 #endif
 }
 
-// Chunk `chunk` (global index) of one chain: steps 1-2; every lane returns the same value.  srows: the stage's
-// rows, column-major [k][kSumStageRows], starting at row r0 (staged) -- or nullptr: rows from global memory.
+// Chunk `chunk` (global index) of one chain of data[n_rows][k]: steps 1-2; every lane returns the same value.
+// srows: the stage's rows, column-major [k][kSumStageRows], starting at row r0 (staged) -- or nullptr: rows from
+// global memory.
 __device__ __forceinline__ double sum_chunk(const double* theta, int64_t chunk, const double* srows, int64_t r0,
-                                            const double* __restrict__ data, int lane) {
+                                            const double* __restrict__ data, int64_t n_rows, int lane) {
   auto term = [&](int64_t row) -> double {
     if constexpr (kSumStaged) {
       double rv[kSumK];
@@ -106,7 +107,7 @@ __device__ __forceinline__ double sum_chunk(const double* theta, int64_t chunk, 
   const int64_t base = chunk * kSumChunk + lane;
   double t[8];
 #pragma unroll
-  for (int j = 0; j < 8; ++j) t[j] = base + 32 * j < kSumRows ? term(base + 32 * j) : 0.0;
+  for (int j = 0; j < 8; ++j) t[j] = base + 32 * j < n_rows ? term(base + 32 * j) : 0.0;
 #pragma unroll
   for (int j = 0; j < 4; ++j) t[j] = t[j] + t[j + 4];
 #pragma unroll
@@ -145,6 +146,37 @@ __device__ __forceinline__ void sum_push(double* stk, int64_t i, double p, int l
   if (lane == 0) stk[lvl] = p;
   __syncwarp();
 }
+// Step 3 above the groups, by the whole warp of row c: the n_groups partials ws[i n + c] are the first leaves of a
+// tree of 2^log2_groups (= P2 / G) leaves, the rest 0.0.  Lane l reduces the aligned block of leaves
+// [l B, (l + 1) B), B = max(1, 2^log2_groups / 32), by the binary-counter stack; an adjacent-pair shuffle tree
+// (lane l + off into lane l) adds the blocks.  Lane 0 returns the tree's value.
+__device__ __forceinline__ double sum_groups(const double* __restrict__ ws, int n, int c, int n_groups,
+                                             int log2_groups, int lane) {
+  const int lb = log2_groups > 5 ? log2_groups - 5 : 0;     // log2 of the leaves per lane
+  const int64_t B = (int64_t)1 << lb;
+  const int64_t first = (int64_t)lane * B;
+  const int64_t m = max((int64_t)0, min(B, (int64_t)n_groups - first));
+  double v = 0.0;                                            // an all-zero block is +0.0
+  if (m > 0) {
+    double stk[kSumMaxDepth];
+    for (int64_t i = 0; i < m; ++i) {
+      int lvl;
+      const double p = sum_merge(stk, i, ws[(size_t)(first + i) * n + c], &lvl);
+      stk[lvl] = p;
+    }
+    v = sum_flush(stk, m, lb);
+  }
+  for (int off = 1; off < (1 << (log2_groups - lb)); off <<= 1) {
+    const double o = __shfl_down_sync(0xFFFFFFFFu, v, off);
+    if ((lane & (2 * off - 1)) == 0) v = v + o;
+  }
+  return v;
+}
+#endif  // BPM_JIT_SUM || BPM_JIT_SUM_RAGGED
+
+#ifdef BPM_JIT_SUM
+constexpr int64_t kSumRows = BPM_NROWS;
+constexpr int64_t kSumChunks = (kSumRows + kSumChunk - 1) / kSumChunk;
 
 // grid (ceil(n / tile), n_groups), kSumThreads threads; dynamic shared memory sum_smem_bytes(tile) (engine.cu).
 // P: rows [n][ld]; n_dev (may be null): device-side count of valid rows, rows past it are skipped.
@@ -190,7 +222,8 @@ __global__ void __launch_bounds__(kSumThreads) lnl_sum_kernel(const double* __re
       double* cs = stk + ci * kSumMaxDepth;
       SumTheta th;
       th.load(P + (size_t)(c0 + ci) * ld);
-      for (int s = 0; s < ns; ++s) sum_push(cs, s0 + s, sum_chunk(th.ptr(), q0 + s0 + s, srows, r0, data, lane), lane);
+      for (int s = 0; s < ns; ++s)
+        sum_push(cs, s0 + s, sum_chunk(th.ptr(), q0 + s0 + s, srows, r0, data, kSumRows, lane), lane);
     }
   }
   __syncthreads();
@@ -201,10 +234,7 @@ __global__ void __launch_bounds__(kSumThreads) lnl_sum_kernel(const double* __re
   }
 }
 
-// Step 3 above the groups and step 4, one warp per row: the n_groups partials of row c are the first leaves of a
-// tree of 2^log2_groups (= P2 / G) leaves, the rest 0.0.  Lane l reduces the aligned block of leaves
-// [l B, (l + 1) B), B = max(1, 2^log2_groups / 32), by the binary-counter stack; an adjacent-pair shuffle tree
-// (lane l + off into lane l) adds the blocks.
+// Step 3 above the groups and step 4, one warp per row (sum_groups).
 __global__ void __launch_bounds__(128) lnl_sum_finish_kernel(const double* __restrict__ P, int n, int ld,
                                                              const int32_t* __restrict__ n_dev,
                                                              const double* __restrict__ ws, int n_groups,
@@ -213,24 +243,7 @@ __global__ void __launch_bounds__(128) lnl_sum_finish_kernel(const double* __res
   const int c = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   if (c >= nv) return;
-  const int lb = log2_groups > 5 ? log2_groups - 5 : 0;     // log2 of the leaves per lane
-  const int64_t B = (int64_t)1 << lb;
-  const int64_t first = (int64_t)lane * B;
-  const int64_t m = max((int64_t)0, min(B, (int64_t)n_groups - first));
-  double v = 0.0;                                            // an all-zero block is +0.0
-  if (m > 0) {
-    double stk[kSumMaxDepth];
-    for (int64_t i = 0; i < m; ++i) {
-      int lvl;
-      const double p = sum_merge(stk, i, ws[(size_t)(first + i) * n + c], &lvl);
-      stk[lvl] = p;
-    }
-    v = sum_flush(stk, m, lb);
-  }
-  for (int off = 1; off < (1 << (log2_groups - lb)); off <<= 1) {
-    const double o = __shfl_down_sync(0xFFFFFFFFu, v, off);
-    if ((lane & (2 * off - 1)) == 0) v = v + o;
-  }
+  const double v = sum_groups(ws, n, c, n_groups, log2_groups, lane);
   if (lane == 0) {
     SumTheta th;
     th.load(P + (size_t)c * ld);
@@ -293,7 +306,8 @@ __global__ void __launch_bounds__(kSumThreads) lnl_sum_problems_kernel(const dou
       double* cs = stk + ci * kSumMaxDepth;
       SumTheta th;
       th.load(P + (size_t)(c0 + ci) * ld);
-      for (int s = 0; s < ns; ++s) sum_push(cs, s0 + s, sum_chunk(th.ptr(), q0 + s0 + s, srows, r0, pdata, lane), lane);
+      for (int s = 0; s < ns; ++s)
+        sum_push(cs, s0 + s, sum_chunk(th.ptr(), q0 + s0 + s, srows, r0, pdata, kSumRows, lane), lane);
     }
   }
   __syncthreads();
@@ -305,3 +319,118 @@ __global__ void __launch_bounds__(kSumThreads) lnl_sum_problems_kernel(const dou
 }
 }  // namespace bpm
 #endif
+
+#ifdef BPM_JIT_SUM_RAGGED
+#include "cr_reduce.cuh"     // cr_update_problems_kernel (BPM_JIT_PROBLEMS is defined too)
+namespace bpm {
+// Multi-problem handles with datasets of different lengths (engine.cu: kJitSumRagged).  data is the concatenated
+// [sum_g M_g][BPM_ROWLEN] array, problem g's M_g rows start at row row_off[g] (row_off[BPM_NPROBLEMS] = sum_g M_g),
+// and rows [g rpp, (g + 1) rpp) of P belong to problem g.  Problem g's tree has C_g = ceil(M_g / 256) chunks and
+// P2_g leaves; it uses groups of G_g = min(G, P2_g) chunks, G = 2^log2_group the launch's, so a problem shorter
+// than a group ends its tree at P2_g as a single-problem handle does (one more level of + 0.0 would turn a -0.0 sum
+// into +0.0).
+struct RaggedGroups {
+  int64_t M;      // rows
+  int64_t C;      // chunks
+  int lg;         // log2(G_g)
+  int n_groups;   // ceil(C / G_g)
+  int log2_groups;// log2(P2_g / G_g)
+  __device__ __forceinline__ RaggedGroups(const int64_t* __restrict__ row_off, int g, int log2_group) {
+    M = row_off[g + 1] - row_off[g];
+    C = (M + kSumChunk - 1) / kSumChunk;
+    const int lp2 = C > 1 ? 64 - __clzll(C - 1) : 0;
+    lg = min(log2_group, lp2);
+    n_groups = (int)((C + ((int64_t)1 << lg) - 1) >> lg);
+    log2_groups = lp2 - lg;
+  }
+};
+
+// The body of lnl_sum_problems_kernel with problem g's row count taken at run time.  The grid is a flat work list:
+// problem g owns blocks [blk_off[g], blk_off[g + 1]), tpp tiles (tpp = ceil(rpp / tile)) times its groups, tiles
+// of one group adjacent.  A problem of one group writes ln L; otherwise group partials go to ws[ng_max][n] and
+// lnl_sum_ragged_finish_kernel completes them.  kSumThreads threads; dynamic shared memory sum_smem_bytes(tile).
+__global__ void __launch_bounds__(kSumThreads) lnl_sum_ragged_kernel(const double* __restrict__ P, int n, int ld,
+                                                                     int rpp, int tpp,
+                                                                     const double* __restrict__ data,
+                                                                     const int64_t* __restrict__ row_off,
+                                                                     const int32_t* __restrict__ blk_off, int tile,
+                                                                     int log2_group, double* __restrict__ ws,
+                                                                     double* __restrict__ out) {
+  extern __shared__ __align__(16) double sm_sum[];
+  const int b = blockIdx.x;
+  int g = 0, hi = BPM_NPROBLEMS;                          // blk_off[g] <= b < blk_off[g + 1]
+  while (hi - g > 1) {
+    const int mid = (g + hi) >> 1;
+    if (blk_off[mid] <= b) g = mid;
+    else hi = mid;
+  }
+  const RaggedGroups pg(row_off, g, log2_group);
+  const int local = b - blk_off[g];
+  const int grp = local / tpp;
+  const int t0 = (local - grp * tpp) * tile;             // first row of the tile inside problem g
+  const int c0 = g * rpp + t0;
+  const int nt = min(tile, rpp - t0);
+  const double* __restrict__ pdata = data + row_off[g] * kSumK;
+  double* stk = sm_sum;                                  // [tile][kSumMaxDepth]
+  double* prior = stk + tile * kSumMaxDepth;             // [tile]
+  double* srows = prior + tile;                          // [k][kSumStageRows] when staged
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int64_t G = (int64_t)1 << pg.lg;
+  const int64_t q0 = (int64_t)grp * G;
+  for (int ci = threadIdx.x; ci < nt; ci += kSumThreads) {
+    SumTheta th;
+    th.load(P + (size_t)(c0 + ci) * ld);
+    prior[ci] = sum_prior(th.ptr());
+  }
+  __syncthreads();
+  const int64_t m = min(G, pg.C - q0);
+  const int sc = G < kSumStageChunks ? (int)G : kSumStageChunks;
+  for (int64_t s0 = 0; s0 < m; s0 += sc) {
+    const int64_t r0 = (q0 + s0) * kSumChunk;
+    const int ns = (int)min((int64_t)sc, m - s0);
+    if constexpr (kSumStaged) {
+      __syncthreads();
+      const int64_t nr = min((int64_t)ns * kSumChunk, pg.M - r0);
+      for (int64_t i = threadIdx.x; i < nr * kSumK; i += kSumThreads) {
+        const int64_t r = i / kSumK;
+        srows[(i - r * kSumK) * kSumStageRows + r] = pdata[r0 * kSumK + i];
+      }
+      __syncthreads();
+    }
+    for (int ci = warp; ci < nt; ci += kSumThreads / 32) {
+      if (prior[ci] == -INFINITY) continue;
+      double* cs = stk + ci * kSumMaxDepth;
+      SumTheta th;
+      th.load(P + (size_t)(c0 + ci) * ld);
+      for (int s = 0; s < ns; ++s)
+        sum_push(cs, s0 + s, sum_chunk(th.ptr(), q0 + s0 + s, srows, r0, pdata, pg.M, lane), lane);
+    }
+  }
+  __syncthreads();
+  for (int ci = threadIdx.x; ci < nt; ci += kSumThreads) {
+    const double S = sum_flush(stk + ci * kSumMaxDepth, m, pg.lg);
+    if (pg.n_groups == 1) out[c0 + ci] = sum_finish_value(prior[ci], S);
+    else ws[(size_t)grp * n + c0 + ci] = S;
+  }
+}
+
+// Step 3 above the groups and step 4 for the rows of problems of several groups, one warp per row (sum_groups over
+// the problem's own n_groups and log2_groups); rows of one-group problems were written by the sum kernel.
+__global__ void __launch_bounds__(128) lnl_sum_ragged_finish_kernel(const double* __restrict__ P, int n, int ld,
+                                                                    int rpp, const int64_t* __restrict__ row_off,
+                                                                    const double* __restrict__ ws, int log2_group,
+                                                                    double* __restrict__ out) {
+  const int c = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int lane = threadIdx.x & 31;
+  if (c >= n) return;
+  const RaggedGroups pg(row_off, c / rpp, log2_group);
+  if (pg.n_groups == 1) return;
+  const double v = sum_groups(ws, n, c, pg.n_groups, pg.log2_groups, lane);
+  if (lane == 0) {
+    SumTheta th;
+    th.load(P + (size_t)c * ld);
+    out[c] = sum_finish_value(sum_prior(th.ptr()), v);
+  }
+}
+}  // namespace bpm
+#endif  // BPM_JIT_SUM_RAGGED

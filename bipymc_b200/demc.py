@@ -36,7 +36,10 @@ Likelihood plug-ins, fastest first:
   1e. ``ln_like_cuda=targets.CudaSumLikelihoodSet(source, dim, data[P, M, k], prior)``: the per-observation
      form of 1c fitted to P datasets of M rows in ONE sampler, with the contract and refusals of 1d: problem g
      runs exactly as a ``CudaSumLikelihood`` sampler on ``data[g]`` with key ``problem_seeds[g]`` would.
-     Each phase is propose + sum + accept at every dim; the sum kernel's tiles of chains stay inside one problem;
+     Each phase is propose + sum + accept at every dim; the sum kernel's tiles of chains stay inside one problem.
+     ``data`` may also be a list of P arrays ``(M_g, k)`` of different lengths: problem g then runs exactly as a
+     ``CudaSumLikelihood`` sampler on its own M_g rows would, and the sum kernel evaluates sum_g M_g terms per
+     chain rather than P max_g M_g;
   2. ``ln_like_batched=f``: ``f(theta)`` takes a CUDA float64 tensor ``[n, dim]`` and
      returns ``[n]`` log-likelihoods (torch ops on the current stream);
   3. any scalar ``ln_like_fn(theta, **ln_kwargs) -> float`` exactly as in the reference

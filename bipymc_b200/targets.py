@@ -498,7 +498,51 @@ class CudaSumLikelihoodSet(CudaSumLikelihood):
     sum is added in the order of ``CudaSumLikelihood`` for M rows and is split over the GPU in tiles of chains
     that never straddle two problems: the form for many datasets of many observations and few chains each.
     P, M, k and ``prior`` are part of the cache key, and the kernels are compiled in a translation unit of their
-    own."""
+    own.
+
+    Datasets of different lengths: ``data`` may also be a list or tuple of P arrays, array g of shape ``(M_g, k)``
+    (or ``(M_g,)``: k = 1), every M_g in [1, 2^31) and one k for all.  When every M_g is equal this is the
+    rectangular set above, ``data`` stacked.  Otherwise ``data`` is the concatenated ``(sum_g M_g, k)`` array and
+    ``n_rows`` the int64 ``[P]`` array of the M_g; problem g's sum runs over its own M_g rows in the order of
+    ``CudaSumLikelihood`` for M_g rows, so the contract above holds with ``CudaSumLikelihood(source, dim,
+    data_g, prior, fmad)``.  The work is that of the sum_g M_g terms, not of P max_g M_g.  ``BPM_ROWLEN`` and
+    ``BPM_NPROBLEMS`` are defined but ``BPM_NROWS`` is not: a term that needs its problem's row count reads it
+    from a data column.  P, k and ``prior`` are part of the cache key, the M_g are not, so new datasets of other
+    lengths reuse the compiled module."""
+
+    def __init__(self, source, dim, data, prior=False, fmad=True):
+        self.n_rows = None      # ragged form: the int64 [P] row counts
+        if isinstance(data, (list, tuple)):
+            data, self.n_rows = self._ragged(data)
+            if self.n_rows is not None:
+                self._shaped = lambda rows: rows      # (sum M_g, k) as _ragged shaped them
+        super(CudaSumLikelihoodSet, self).__init__(source, dim, data, prior, fmad)
+
+    @staticmethod
+    def _ragged(arrays):
+        """P arrays of shape (M_g, k) or (M_g,): ``(stacked (P, M, k), None)`` when every M_g is equal, else
+        ``(concatenated (sum M_g, k), n_rows)``; ValueError on an empty sequence, problem or row, or mixed k."""
+        if len(arrays) == 0:
+            raise ValueError("data: an empty sequence (one array per problem expected)")
+        parts = []
+        for g, a in enumerate(arrays):
+            a = np.asarray(a, dtype=np.float64)
+            if a.ndim == 1:
+                a = a.reshape(-1, 1)
+            if a.ndim != 2 or a.shape[1] < 1:
+                raise ValueError("data[%d] must have shape (M, k) or (M,), not %s" % (g, a.shape))
+            if not 1 <= a.shape[0] < 2 ** 31:
+                raise ValueError("data[%d] has %d rows: every problem needs M in [1, 2^31)" % (g, a.shape[0]))
+            if parts and a.shape[1] != parts[0].shape[1]:
+                raise ValueError("data[%d] has rows of %d values, data[0] of %d: every problem needs the same k"
+                                 % (g, a.shape[1], parts[0].shape[1]))
+            parts.append(a)
+        if len(parts) >= 2 ** 31:
+            raise ValueError("data: P must be below 2^31")
+        n_rows = np.array([a.shape[0] for a in parts], dtype=np.int64)
+        if np.all(n_rows == n_rows[0]):
+            return np.stack(parts), None
+        return np.concatenate(parts), n_rows
 
     @staticmethod
     def _shaped(data):
@@ -513,14 +557,20 @@ class CudaSumLikelihoodSet(CudaSumLikelihood):
         return data
 
     def _compile_call(self, lib):
+        if self.n_rows is not None:
+            return lib.bpm_jit_compile_sum_ragged, (self.source.encode(), self.dim, self.data.shape[1], self.n_problems)
         P, M, k = self.data.shape
         return lib.bpm_jit_compile_sum_problems, (self.source.encode(), self.dim, M, k, P)
 
     def _attach_call(self, lib, handle):
         # the handle must be a multi-problem handle with P problems (bpm_set_problems), which gives P
+        if self.n_rows is not None:
+            return lib.bpm_set_jit_sum_ragged_target, (handle, self.source.encode(), _lib.dptr(self.data),
+                                                       self.n_rows.ctypes.data_as(C.POINTER(C.c_int64)),
+                                                       self.data.shape[1])
         _, M, k = self.data.shape
         return lib.bpm_set_jit_sum_problems_target, (handle, self.source.encode(), _lib.dptr(self.data), M, k)
 
     @property
     def n_problems(self):
-        return int(self.data.shape[0])
+        return int(self.data.shape[0]) if self.n_rows is None else int(self.n_rows.size)

@@ -191,7 +191,7 @@ int bpm_set_jit_sum_target(bpm_handle h, const char* source, const double* data,
  * bpm_set_problems is called right after bpm_create, on an unsharded DE-MC or DREAM handle with
  * n_chains % n_problems == 0 and n = n_chains / n_problems >= 4; keys[n_problems] (HOST) are the problems'
  * Philox keys.  The likelihood is then set with bpm_set_jit_problems_target (or, per observation,
- * bpm_set_jit_sum_problems_target below): the ln_like source of
+ * bpm_set_jit_sum_problems_target or bpm_set_jit_sum_ragged_target below): the ln_like source of
  * bpm_jit_compile, with data the row-major [P][n_data] HOST array (n_data >= 1): problem g's ln_like gets
  * data + g n_data, and BPM_NDATA is n_data (BPM_NPROBLEMS is P).  P and n_data are part of the cache key.
  * A multi-problem handle offers bpm_step_generations, bpm_flush, bpm_moments_from_history, bpm_eval_lnl
@@ -215,6 +215,17 @@ int bpm_jit_compile_sum_problems(const char* source, int32_t dim, int64_t n_rows
                                  int32_t flags, int32_t* from_cache, char* log, int64_t log_cap);
 int bpm_set_jit_sum_problems_target(bpm_handle h, const char* source, const double* data, int64_t n_rows,
                                     int32_t row_len, int32_t flags, int32_t* from_cache, char* log, int64_t log_cap);
+/* The same on datasets of different lengths (target BPM_TARGET_JIT_SUM): data is the row-major HOST array of the
+ * P problems' rows one after another, [sum_g M_g][row_len], and row_counts[P] (HOST) the M_g, each in
+ * [1, 2^31 - 1]; their sum may exceed 2^31.  Problem g's sum runs over its own M_g rows in the order
+ * bpm_jit_compile_sum gives for M_g rows, so it gets the bits a single-problem handle holding them would.
+ * BPM_ROWLEN is row_len and BPM_NPROBLEMS P; BPM_NROWS is not defined (a term that needs its problem's row count
+ * reads it from a data column).  P, row_len and the prior bit are part of the cache key, the M_g are not: new
+ * datasets of other lengths reuse the module.  The launches per generation depend neither on P nor on the M_g. */
+int bpm_jit_compile_sum_ragged(const char* source, int32_t dim, int32_t row_len, int32_t n_problems, int32_t flags,
+                               int32_t* from_cache, char* log, int64_t log_cap);
+int bpm_set_jit_sum_ragged_target(bpm_handle h, const char* source, const double* data, const int64_t* row_counts,
+                                  int32_t row_len, int32_t flags, int32_t* from_cache, char* log, int64_t log_cap);
 int bpm_get_problem_cr_state(bpm_handle h, double* p_cr, double* dm, double* cnt);
 int bpm_set_problem_cr_state(bpm_handle h, const double* p_cr, const double* dm, const double* cnt);
 int bpm_get_problem_counters(bpm_handle h, uint64_t* acc, uint64_t* rej);
