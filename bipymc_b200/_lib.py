@@ -14,7 +14,7 @@ LIB_PATH = os.environ.get("BIPYMC_B200_LIB") or os.path.join(_HERE, "lib", "libb
 
 BPM_ALGO_DEMC, BPM_ALGO_DREAM, BPM_ALGO_DEMC_SERIAL = 0, 1, 2
 TARGET_EXTERNAL, TARGET_BANANA, TARGET_BIMODAL, TARGET_GAUSS, TARGET_LINEFIT, TARGET_EXPFIT, TARGET_JIT, \
-    TARGET_JIT_SUM = 0, 1, 2, 3, 4, 5, 6, 7
+    TARGET_JIT_SUM, TARGET_JIT_GAUSS = 0, 1, 2, 3, 4, 5, 6, 7, 8
 BPM_MAX_PAIRS, BPM_MAX_CR, BPM_MAX_PEERS = 8, 16, 15
 
 
@@ -67,6 +67,11 @@ SIGNATURES = {
                                       C.c_char_p, C.c_int64]),
     "bpm_set_jit_sum_target": (C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(C.c_double), C.c_int64, C.c_int32,
                                          C.c_int32, C.POINTER(C.c_int32), C.c_char_p, C.c_int64]),
+    "bpm_jit_compile_gauss": (C.c_int, [C.c_char_p, C.c_int32, C.c_int64, C.c_int32, C.c_int32,
+                                        C.POINTER(C.c_int32), C.c_char_p, C.c_int64]),
+    "bpm_set_jit_gauss_target": (C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(C.c_double), C.c_int64, C.c_int32,
+                                           C.POINTER(C.c_double), C.POINTER(C.c_double), C.c_double, C.c_int32,
+                                           C.POINTER(C.c_int32), C.c_char_p, C.c_int64]),
     "bpm_set_problems": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(C.c_uint64)]),
     "bpm_jit_compile_problems": (C.c_int, [C.c_char_p, C.c_int32, C.c_int64, C.c_int32, C.c_int32,
                                            C.POINTER(C.c_int32), C.c_char_p, C.c_int64]),

@@ -47,7 +47,8 @@ __host__ __device__ constexpr size_t sum_smem_bytes(int tile, int k) {
                            (k <= kSumSmemRowLen ? (size_t)k * sum_stage_chunks(k) * kSumChunk : 0));
 }
 
-#if defined(BPM_JIT_SUM) || defined(BPM_JIT_SUM_RAGGED)
+// The Gaussian kind (BPM_JIT_GAUSS, kernels_gauss.cuh) shares the row staging, SumTheta and the prior helpers.
+#if defined(BPM_JIT_SUM) || defined(BPM_JIT_SUM_RAGGED) || defined(BPM_JIT_GAUSS)
 constexpr int kSumK = BPM_ROWLEN;
 constexpr bool kSumStaged = kSumK <= kSumSmemRowLen;
 constexpr int kSumStageChunks = sum_stage_chunks(kSumK);
@@ -88,6 +89,16 @@ __device__ __forceinline__ double sum_finish_value(double prior, double S) {
 #endif
 }
 
+// Stage rows [r0, r0 + nr) of data[][k] into srows, column-major [k][kSumStageRows], by a CTA of kSumThreads threads
+__device__ __forceinline__ void sum_stage(double* srows, const double* __restrict__ data, int64_t r0, int64_t nr) {
+  for (int64_t i = threadIdx.x; i < nr * kSumK; i += kSumThreads) {
+    const int64_t r = i / kSumK;
+    srows[(i - r * kSumK) * kSumStageRows + r] = data[r0 * kSumK + i];
+  }
+}
+#endif  // BPM_JIT_SUM || BPM_JIT_SUM_RAGGED || BPM_JIT_GAUSS
+
+#if defined(BPM_JIT_SUM) || defined(BPM_JIT_SUM_RAGGED)
 // Chunk `chunk` (global index) of one chain of data[n_rows][k]: steps 1-2; every lane returns the same value.
 // srows: the stage's rows, column-major [k][kSumStageRows], starting at row r0 (staged) -- or nullptr: rows from
 // global memory.
@@ -210,11 +221,7 @@ __global__ void __launch_bounds__(kSumThreads) lnl_sum_kernel(const double* __re
     const int ns = (int)min((int64_t)sc, m - s0);
     if constexpr (kSumStaged) {
       __syncthreads();                                   // the previous stage's rows are no longer read
-      const int64_t nr = min((int64_t)ns * kSumChunk, kSumRows - r0);
-      for (int64_t i = threadIdx.x; i < nr * kSumK; i += kSumThreads) {
-        const int64_t r = i / kSumK;
-        srows[(i - r * kSumK) * kSumStageRows + r] = data[r0 * kSumK + i];
-      }
+      sum_stage(srows, data, r0, min((int64_t)ns * kSumChunk, kSumRows - r0));
       __syncthreads();
     }
     for (int ci = warp; ci < nt; ci += kSumThreads / 32) {
@@ -294,11 +301,7 @@ __global__ void __launch_bounds__(kSumThreads) lnl_sum_problems_kernel(const dou
     const int ns = (int)min((int64_t)sc, m - s0);
     if constexpr (kSumStaged) {
       __syncthreads();
-      const int64_t nr = min((int64_t)ns * kSumChunk, kSumRows - r0);
-      for (int64_t i = threadIdx.x; i < nr * kSumK; i += kSumThreads) {
-        const int64_t r = i / kSumK;
-        srows[(i - r * kSumK) * kSumStageRows + r] = pdata[r0 * kSumK + i];
-      }
+      sum_stage(srows, pdata, r0, min((int64_t)ns * kSumChunk, kSumRows - r0));
       __syncthreads();
     }
     for (int ci = warp; ci < nt; ci += kSumThreads / 32) {
@@ -390,11 +393,7 @@ __global__ void __launch_bounds__(kSumThreads) lnl_sum_ragged_kernel(const doubl
     const int ns = (int)min((int64_t)sc, m - s0);
     if constexpr (kSumStaged) {
       __syncthreads();
-      const int64_t nr = min((int64_t)ns * kSumChunk, pg.M - r0);
-      for (int64_t i = threadIdx.x; i < nr * kSumK; i += kSumThreads) {
-        const int64_t r = i / kSumK;
-        srows[(i - r * kSumK) * kSumStageRows + r] = pdata[r0 * kSumK + i];
-      }
+      sum_stage(srows, pdata, r0, min((int64_t)ns * kSumChunk, pg.M - r0));
       __syncthreads();
     }
     for (int ci = warp; ci < nt; ci += kSumThreads / 32) {

@@ -40,6 +40,10 @@ Likelihood plug-ins, fastest first:
      ``data`` may also be a list of P arrays ``(M_g, k)`` of different lengths: problem g then runs exactly as a
      ``CudaSumLikelihood`` sampler on its own M_g rows would, and the sum kernel evaluates sum_g M_g terms per
      chain rather than P max_g M_g;
+  1f. ``ln_like_cuda=targets.CudaGaussLikelihood(source, dim, x, y, cov, prior)``: a Gaussian likelihood with a
+     dense data covariance around ``__device__ double model_mean(const double* theta, const double* row)``.
+     Each phase is propose + model means + quadratic form on the FP64 tensor pipe + finish + accept at every
+     dim, in an order fixed by M alone.  One problem and one rank;
   2. ``ln_like_batched=f``: ``f(theta)`` takes a CUDA float64 tensor ``[n, dim]`` and
      returns ``[n]`` log-likelihoods (torch ops on the current stream);
   3. any scalar ``ln_like_fn(theta, **ln_kwargs) -> float`` exactly as in the reference
@@ -422,9 +426,11 @@ class DeMcMpi(object):
     def _check_problems(self, kwargs):
         """A CudaLikelihoodSet or CudaSumLikelihoodSet makes this a multi-problem sampler; refuse what that mode
         does not offer."""
-        from .targets import CudaLikelihoodSet, CudaSumLikelihoodSet
+        from .targets import CudaGaussLikelihood, CudaLikelihoodSet, CudaSumLikelihoodSet
         cuda = kwargs.get("ln_like_cuda", None)
         seed = kwargs.get("seed", None)
+        if isinstance(cuda, CudaGaussLikelihood) and self.comm.size > 1:
+            raise ValueError("ln_like_cuda=CudaGaussLikelihood runs on one rank (%d ranks given)" % self.comm.size)
         if not isinstance(cuda, (CudaLikelihoodSet, CudaSumLikelihoodSet)):
             if seed is not None and np.ndim(seed) != 0:
                 raise ValueError("a sequence of seeds (one per problem) needs ln_like_cuda=targets.CudaLikelihoodSet "

@@ -43,10 +43,12 @@ class DeMc(DeMcMpi):
         self._history_policy = proposal_kwargs.get("history", "full")
         self._ln_like_batched = proposal_kwargs.get("ln_like_batched", None)
         self._ln_like_cuda = proposal_kwargs.get("ln_like_cuda", None)
-        from .targets import CudaLikelihoodSet, CudaSumLikelihoodSet
+        from .targets import CudaGaussLikelihood, CudaLikelihoodSet, CudaSumLikelihoodSet
         if isinstance(self._ln_like_cuda, (CudaLikelihoodSet, CudaSumLikelihoodSet)):
             raise NotImplementedError("serial DeMc does not run a %s (several problems in one sampler): "
                                       "use DeMcMpi or DreamMpi" % type(self._ln_like_cuda).__name__)
+        if isinstance(self._ln_like_cuda, CudaGaussLikelihood) and self.comm.size > 1:
+            raise ValueError("ln_like_cuda=CudaGaussLikelihood runs on one rank (%d ranks given)" % self.comm.size)
         self._device_index = proposal_kwargs.get("device", None)
         self._fused = False                                         # the sweep uses the split launches
         self._chunk_bytes = int(proposal_kwargs.get("history_chunk_bytes", 1 << 30))

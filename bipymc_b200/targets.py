@@ -574,3 +574,101 @@ class CudaSumLikelihoodSet(CudaSumLikelihood):
     @property
     def n_problems(self):
         return int(self.data.shape[0]) if self.n_rows is None else int(self.n_rows.size)
+
+
+class CudaGaussLikelihood(CudaLikelihood):
+    """A Gaussian likelihood with correlated noise: a model mean in CUDA C++ and a dense data covariance.
+    ``source`` defines::
+
+        __device__ double model_mean(const double* theta, const double* row);   // E[y_i | theta] at row x_i
+        __device__ double ln_prior(const double* theta);                        // only when prior=True
+
+    ``x`` is a finite float64 array of shape ``(M, k)`` (a 1-D array is ``(M, 1)``), 1 <= M <= 32768, and ``row``
+    points at the k values of x_i; ``y`` is finite of shape ``(M,)``; ``cov`` is finite, ``(M, M)``, symmetric
+    (max |C - C^T| <= 1e-12 max |C|; its lower triangle is used) and positive definite, as scipy's
+    ``multivariate_normal`` requires by default.  ``BPM_DIM``, ``BPM_NROWS`` (M), ``BPM_ROWLEN`` (k) and
+    ``BPM_HAS_PRIOR`` are macros; the scope, ``fmad``, the NaN rule and ``CudaCompileError`` are those of
+    ``CudaLikelihood``.  The value is::
+
+        ln L(theta) = ln_prior(theta) + (-0.5 (c0 + |(m(theta) - y) . B|^2))
+
+    with C = L L^T the Cholesky factor (numpy, on the host), B = L^-T and c0 = M ln(2 pi) + 2 sum_i ln L_ii: it
+    equals ``scipy.stats.multivariate_normal(m(theta), cov).logpdf(y) + ln_prior(theta)`` to rounding.  It is
+    exactly ``-inf`` when ``ln_prior`` is ``-inf``, whatever ``model_mean`` returns there.  The order of every
+    addition is fixed by M alone, so a given theta gets the same bits whatever the batch or the number of chains.
+    Each generation runs the proposal kernel, then the model means of every chain, the quadratic form on the FP64
+    tensor pipe (half of it: B is triangular) and a finish kernel, then the accept kernel, at every d.  The source,
+    dim, M, k, ``prior`` and ``fmad`` are the cache key: new ``y`` or ``cov`` of the same shape reuse the module.
+
+    Which form to use: ``CudaSumLikelihood`` when the noise is independent (a diagonal covariance) -- it costs O(M)
+    per chain against this form's O(M^2).  This form when the errors are correlated: a calibration shared by all
+    points, drift, overlapping bins, a covariance shipped with the data.  One problem and one rank only.  Pass it
+    as ``ln_like_cuda=``."""
+
+    MAX_ROWS = 32768
+
+    def __init__(self, source, dim, x, y, cov, prior=False, fmad=True):
+        super(CudaGaussLikelihood, self).__init__(source, dim, x, fmad)
+        M = self.data.shape[0]
+        y = np.asarray(y, dtype=np.float64)
+        if y.shape != (M,):
+            raise ValueError("y must have shape (%d,) (one value per row of x), not %s" % (M, y.shape))
+        if not np.all(np.isfinite(y)):
+            raise ValueError("y must be finite")
+        cov = np.asarray(cov, dtype=np.float64)
+        if cov.shape != (M, M):
+            raise ValueError("cov must have shape (%d, %d), not %s" % (M, M, cov.shape))
+        if not np.all(np.isfinite(cov)):
+            raise ValueError("cov must be finite")
+        if np.max(np.abs(cov - cov.T)) > 1e-12 * np.max(np.abs(cov)):
+            raise ValueError("cov must be symmetric: max |C - C^T| > 1e-12 max |C|")
+        self.prior = bool(prior)
+        self.y = np.ascontiguousarray(y)
+        self.cov = cov
+        self.B, self.c0 = self.factor(cov)
+
+    @staticmethod
+    def factor(cov):
+        """``(B, c0)`` of a symmetric covariance (its lower triangle is used): B = L^-T, upper triangular, and
+        c0 = M ln(2 pi) + ln det C.  ValueError unless C is positive definite by scipy's test (``_PSD``: every
+        eigenvalue above 1e6 eps max |eigenvalue|)."""
+        import scipy.linalg
+        M = cov.shape[0]
+        low = np.tril(cov) + np.tril(cov, -1).T
+        s = np.linalg.eigvalsh(low)
+        eps = 1e6 * np.finfo(np.float64).eps * np.max(np.abs(s))
+        if np.min(s) <= eps:
+            raise ValueError("cov must be positive definite (smallest eigenvalue %.3g, scipy's threshold %.3g)"
+                             % (np.min(s), eps))
+        try:
+            L = np.linalg.cholesky(low)
+        except np.linalg.LinAlgError:
+            raise ValueError("cov must be positive definite (its Cholesky factorisation failed)")
+        Linv = scipy.linalg.solve_triangular(L, np.eye(M), lower=True)
+        B = np.ascontiguousarray(np.triu(Linv.T))
+        c0 = M * np.log(2.0 * np.pi) + 2.0 * np.sum(np.log(np.diag(L)))
+        return B, float(c0)
+
+    @staticmethod
+    def _shaped(data):
+        data = CudaSumLikelihood._shaped(data)
+        if data.shape[0] > CudaGaussLikelihood.MAX_ROWS:
+            raise ValueError("x has %d rows: M must be in [1, %d]" % (data.shape[0], CudaGaussLikelihood.MAX_ROWS))
+        return data
+
+    @property
+    def x(self):
+        return self.data
+
+    def _compile_call(self, lib):
+        M, k = self.data.shape
+        return lib.bpm_jit_compile_gauss, (self.source.encode(), self.dim, M, k)
+
+    def _attach_call(self, lib, handle):
+        M, k = self.data.shape
+        return lib.bpm_set_jit_gauss_target, (handle, self.source.encode(), _lib.dptr(self.data), M, k,
+                                              _lib.dptr(self.y), _lib.dptr(self.B), self.c0)
+
+    @property
+    def _flags(self):
+        return (1 if self.fmad else 0) | (2 if self.prior else 0)

@@ -44,6 +44,7 @@ extern "C" {
 #define BPM_TARGET_EXPFIT 5   /* examples/ex_exp_fit.py:38-121     params: t[M], y[M]; dim = 5     */
 #define BPM_TARGET_JIT 6      /* user CUDA source compiled at run time: bpm_set_jit_target only   */
 #define BPM_TARGET_JIT_SUM 7  /* per-observation CUDA source, summed: bpm_set_jit_sum_target only */
+#define BPM_TARGET_JIT_GAUSS 8 /* CUDA model mean, dense data covariance: bpm_set_jit_gauss_target only */
 
 typedef struct bpm_engine* bpm_handle;
 typedef void* bpm_stream; /* cudaStream_t */
@@ -181,6 +182,29 @@ int bpm_jit_compile_sum(const char* source, int32_t dim, int64_t n_rows, int32_t
                         int32_t* from_cache, char* log, int64_t log_cap);
 int bpm_set_jit_sum_target(bpm_handle h, const char* source, const double* data, int64_t n_rows, int32_t row_len,
                            int32_t flags, int32_t* from_cache, char* log, int64_t log_cap);
+
+/* Run-time compiled Gaussian likelihood with a dense data covariance (BPM_TARGET_JIT_GAUSS).  `source` is CUDA
+ * C++ defining
+ *   __device__ double model_mean(const double* theta, const double* row)   -- E[y_i | theta] at row x_i
+ *   __device__ double ln_prior(const double* theta)                        -- only with flags bit 1
+ * with theta[BPM_DIM] and row[BPM_ROWLEN]; BPM_NROWS (M) is defined too, and the scope is that of
+ * bpm_jit_compile.  x is the row-major [n_rows][row_len] HOST array, 1 <= n_rows <= 32768; y [n_rows] (HOST)
+ * the observations; B [n_rows][n_rows] (HOST, row-major) the upper triangular L^-T of the covariance's Cholesky
+ * factor C = L L^T (an entry below the diagonal that is not 0 is refused); c0 = M ln(2 pi) + ln det C.
+ *   ln L = ln_prior(theta) + (-0.5 (c0 + |(m(theta) - y) . B|^2)),  m_i(theta) = model_mean(theta, x_i)
+ * (-inf when ln_prior is -inf, whatever model_mean returns).  Per evaluation three launches: the predictions
+ * [n][Mp] (Mp = M rounded up to 16) into a workspace, the quadratic form on the FP64 tensor pipe in column blocks
+ * of 128 (bipymc_b200/csrc/gauss_data.cuh), and the finish.  Every addition's order is fixed by M alone, so a
+ * given theta gets the same bits whatever the batch, the number of chains or the launch shape.  The likelihood
+ * runs between the propose and accept kernels at every dim (never in the fused d <= 4 kernel), in serial DE-MC
+ * and in bpm_eval_lnl.  One problem per handle, one rank.  flags, cache, log and from_cache as for
+ * bpm_jit_compile_sum; M, row_len and the prior bit are part of the cache key, x, y, B and c0 are not.  A refused
+ * or failed bpm_set_jit_gauss_target leaves the handle's previous target as it was. */
+int bpm_jit_compile_gauss(const char* source, int32_t dim, int64_t n_rows, int32_t row_len, int32_t flags,
+                          int32_t* from_cache, char* log, int64_t log_cap);
+int bpm_set_jit_gauss_target(bpm_handle h, const char* source, const double* x, int64_t n_rows, int32_t row_len,
+                             const double* y, const double* B, double c0, int32_t flags, int32_t* from_cache,
+                             char* log, int64_t log_cap);
 
 /* Multi-problem handles: P independent problems of n chains each in one handle (population P n, problem-major:
  * problem g owns chains [g n, (g + 1) n)).  Problem g steps exactly as a handle of n chains with seed keys[g]
